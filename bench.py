@@ -6,7 +6,7 @@ normal-equation assembly, damped Schur reduction onto the camera system, sparse 
 reduced system (FP64 DMMA), back-substitution, |Jp| statistics and the trial-point residual.  Accepted
 trial points are taken, so successive steps walk the real LM path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N = 1: BASELINE config 4 (1000 cameras x 200k points x 2M observations, shared Brown IO, depend datum).
 N > 1 (torchrun, one rank per GPU): BASELINE config 5 cut to N/8 of its cameras and points - 1250 cameras, 500k
@@ -53,7 +53,33 @@ def parse():
                     help='object points per rank (default: 200k at N = 1, 500k at N > 1)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--ref-budget', type=float, default=420.0, help='wall seconds for the reference arm')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step returned as DIR/<name>.npy: the step p (float64; at N > 1 '
+                         'p_rank<r>.npy per rank) and its statistics f, jp2, rjp, f_new, singular')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU path; the reference arm has none')
+    return args
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(d, p, st, rank, world):
+    """The outputs of the last timed step, for comparing two builds on the same seeded scene.  A step vector larger
+    than this rank's share of DUMP_BYTES (less 4 kB for file headers and the statistics) is cut to a fixed, seeded
+    sample of its entries (same sample every run)."""
+    os.makedirs(d, exist_ok=True)
+    p = np.asarray(p, dtype=np.float64)
+    keep = (DUMP_BYTES // world - 4096) // 8
+    if len(p) > keep:
+        p = p[np.sort(np.random.default_rng(rank).choice(len(p), keep, replace=False))]
+    np.save(os.path.join(d, 'p.npy' if world == 1 else 'p_rank%d.npy' % rank), p)
+    if rank == 0:
+        for k in ('f', 'jp2', 'rjp', 'f_new', 'singular'):
+            np.save(os.path.join(d, k + '.npy'), np.array([st[k]], dtype=np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -326,6 +352,13 @@ def main():
     timed(min(args.warmup, 3), False)
     wall_e2e, dev_ms_e2e, _ = timed(args.steps, False)
     sampler.stop()
+    if args.dump_outputs:
+        # The timed device-resident path once more from x0, its last step handed back to the host.  The default path is
+        # bit-reproducible, so these are the timed steps' outputs; taking them here leaves the timed steps untouched.
+        P.normal_step(x0, lam, trial=True, accept=False, want_p=False)   # restart the path at x0
+        for i in range(args.steps):
+            p, st = P.normal_step(None, lam, trial=True, accept=True, want_p=i == args.steps - 1)
+        dump_outputs(args.dump_outputs, p, st, rank, world)
 
     t = torch.tensor([wall, wall_e2e, float(np.sum(dev_ms))], dtype=torch.float64, device='cuda')
     if world > 1:
