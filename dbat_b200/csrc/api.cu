@@ -100,7 +100,6 @@ struct dbat_handle {
     double* h_G = nullptr;              // pinned: summed Gram of the last evaluation
     unsigned long long* h_piv = nullptr;   // pinned: min / max pivot and the breakdown flag of the last factorisation
     double* solve_pout = nullptr;       // step vector of a solve_step whose host-side part (finish_solve) is still due
-    bool solve_jp = false;
     double *d_x = nullptr, *d_t = nullptr, *d_p = nullptr, *d_pgn = nullptr, *d_g = nullptr, *d_pc = nullptr;
     double* d_pEO = nullptr;             // nImg x 6: EO part of the last camera-side step per image (0 = fixed element)
     double *d_camDiag = nullptr, *d_camG = nullptr, *d_diagN = nullptr, *d_dscale = nullptr;
@@ -527,25 +526,12 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     }
     AL(P.W, (size_t)std::max(1, nObs) * DBAT_W_STRIDE);
     if (P.ioGeneral) AL(P.Wfull, (size_t)std::max(1, nObs) * DBAT_WF_STRIDE);
-    {   // deterministic Schur index: inverse permutation, point of every pm observation, pair blocks
-        std::vector<int> cm2pm(nObs), pt_pm(nObs);
-        for (int o = 0; o < nObs; ++o) { cm2pm[h->h_pm2cm[o]] = o; pt_pm[o] = h->h_pt_cm[h->h_pm2cm[o]]; }
-        int *d_cm2pm, *d_pt_pm, *d_img_start;
-        UP(d_cm2pm, cm2pm); UP(d_pt_pm, pt_pm); UP(d_img_start, h->h_img_start);
-        P.cm2pm = d_cm2pm; P.pt_pm = d_pt_pm; P.img_start = d_img_start;
-        std::vector<long long> pair_off(nOP + 1, 0);
-        for (int j = 0; j < nOP; ++j) {
-            const long long k = h->h_pt_start[j + 1] - h->h_pt_start[j];
-            pair_off[j + 1] = pair_off[j] + k * (k + 1) / 2;
-        }
-        long long *dp = nullptr, *dk = nullptr, *doff = nullptr; int nBlk = 0;
-        if (build_pair_index(d_pt_start, d_img_pm, pair_off.data(), nOP, nImg, &dp, &dk, &doff, &nBlk, h->st))
-            return fail_create(h, DBAT_E_OOM, "out of memory while building the Schur pair index");
-        h->allocs.push_back(dp); h->allocs.push_back(dk); h->allocs.push_back(doff);
-        P.pairs = dp; P.blk_key = dk; P.blk_off = doff; P.nBlk = nBlk;
-        AL(P.Y, (size_t)std::max(1, nObs) * DBAT_W_STRIDE);
-        AL(P.ptaux, (size_t)std::max(1, nOP) * DBAT_PTAUX_STRIDE);
-        AL(P.shPart, (size_t)((nOP + DBAT_SHCHUNK - 1) / DBAT_SHCHUNK + 1) * DBAT_NSLOT * DBAT_SHCOLS);
+    {   // point of every point-major observation
+        std::vector<int> pt_pm(nObs);
+        for (int o = 0; o < nObs; ++o) pt_pm[o] = h->h_pt_cm[h->h_pm2cm[o]];
+        int* d_pt_pm;
+        UP(d_pt_pm, pt_pm);
+        P.pt_pm = d_pt_pm;
     }
     {   // point-side assembly blocks: runs [begin, end) of whole points with at most DBAT_PSB observations (and at most
         // DBAT_PSB / 2 points); a point with more observations than that goes to the one-thread-per-point kernel
@@ -580,7 +566,7 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
         }
         const int* ps = h->h_pt_start.data();
         // image lists in elimination-order rank (ascending inside a point): the union of a group is then
-        // ascending in S order, which the tile pairs of k_schur_group rely on
+        // ascending in S order, which the lower-triangular window blocks of k_schur_win rely on
         std::vector<int> rk(std::max(1, nObs));
         for (int j = 0; j < nOP; ++j) {
             for (int o = ps[j]; o < ps[j + 1]; ++o) rk[o] = imgRank[img_pm[o]];
@@ -597,9 +583,8 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
         // greedy groups of consecutive points: at most gcap points, union of their image lists at most
         // `mu` images (a single point always fits).  A point that lacks an image of the union simply
         // has zero rows there.
-        const int gcap = std::max(1, std::min(WIN_GP, (int)(cand.size() / (148 * 8))));   // <= WIN_GP (and GRP_CAP of schur.cu)
-        int mu = 12;
-        if (const char* e = getenv("DBAT_GRP_MU")) mu = std::max(1, std::min(DBAT_GRP_MAXM, atoi(e)));
+        const int gcap = std::max(1, std::min(WIN_GP, (int)(cand.size() / (148 * 8))));
+        const int mu = 12;
         std::vector<int> gstart, gimg_off, gimg, uni, tmp;
         std::vector<unsigned char> slot(std::max(1, nObs), 0);
         gstart.push_back(0); gimg_off.push_back(0);
@@ -631,20 +616,14 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
         const bool noCand = cand.empty();
         if (noCand) { cand.push_back(0); gstart.assign(1, 0); gimg_off.assign(1, 0); gimg.push_back(0); }
         if (big.empty()) big.push_back(0); else P.nBig = (int)big.size();
-        P.nGrp = (int)gstart.size() - 1;
-        {
-            int *d_go, *d_gi; unsigned char* d_sl;
-            UP(d_go, gimg_off); UP(d_gi, gimg); UP(d_sl, slot);
-            P.grp_img_off = d_go; P.grp_img = d_gi; P.obs_slot = d_sl;
-        }
-        int *d_gp, *d_gs, *d_big;
-        UP(d_gp, cand); UP(d_gs, gstart); UP(d_big, big);
-        P.grp_pt = d_gp; P.grp_start = d_gs; P.big_pt = d_big;
+        const int nGrp = (int)gstart.size() - 1;
+        int *d_gp, *d_big;
+        UP(d_gp, cand); UP(d_big, big);
+        P.grp_pt = d_gp; P.big_pt = d_big;
         AL(P.vinv, (size_t)std::max(1, nOP) * 8);
         // ---- window Schur (schur_win.cu): group headers, clusters of consecutive groups whose unions span at most
         //      WIN_MAXW images, and the fixed-order reduction index of the cluster images
         P.nCand = noCand ? 0 : (int)cand.size();
-        const int nGrp = P.nGrp;
         std::vector<WinHdr> hdr((size_t)std::max(1, nGrp));
         std::vector<int> clu_grp(1, 0), clu_img_off(1, 0), clu_img;
         std::vector<long long> clu_stg(1, 0);
@@ -836,14 +815,6 @@ static int allreduce_max_u64(dbat_handle* h, unsigned long long* buf, size_t cnt
 
 // scatter device vector xdev into the parameter arrays and rebuild the per-image records
 static void set_params(dbat_handle* h, const double* xdev) {
-    static const bool split = getenv("DBAT_SETPARAMS_SPLIT") != nullptr;     // debugging: the five separate launches
-    if (split) {
-        launch_deserialize(xdev, h->d_IOsrc, h->d_IOdst, h->P.IOval, h->nIOdes, h->st);
-        launch_deserialize(xdev, h->d_EOsrc, h->d_EOdst, h->P.EOval, h->nEOdes, h->st);
-        launch_deserialize(xdev, h->d_OPsrc, h->d_OPdst, h->P.OPval, h->nOPdes, h->st);
-        launch_param_setup(h->P, h->d_rep, h->nIOrec, h->st);
-        return;
-    }
     launch_set_params(h->P, xdev, ScatterList{h->d_IOsrc, h->d_IOdst, h->P.IOval, h->nIOdes, 0},
                       ScatterList{h->d_EOsrc, h->d_EOdst, h->P.EOval, h->nEOdes, 0},
                       ScatterList{h->d_OPsrc, h->d_OPdst, h->P.OPval, h->nOPdes, 0}, h->d_rep, h->nIOrec, h->st);
@@ -876,20 +847,12 @@ static int eval_full(dbat_handle* h, bool sync = true) {
     // bandwidth-bound, so they run side by side on two streams
     // The camera-side kernel (the shorter one) is launched first: the two kernels cannot share an SM's registers, so they
     // run one after the other anyway, and this way the chunk -> image -> total sums run beside the point side.  Capping
-    // the camera-side CTAs per SM to make room for point-side CTAs was measured and is slower (DBAT_EVAL_POINT_FIRST:
-    // the earlier order).
-    static const bool camFirst = getenv("DBAT_EVAL_POINT_FIRST") == nullptr;
+    // the camera-side CTAs per SM to make room for point-side CTAs was measured and is slower.
     cudaEventRecord(h->evFork, h->st);
     cudaStreamWaitEvent(h->st2, h->evFork, 0);
-    if (camFirst) {
-        launch_cam_side(h->P, h->d_img_chunk_start, h->d_tmpG, h->st);
-        launch_point_side(h->P, h->st2);
-        cudaEventRecord(h->evJoin, h->st2);
-    } else {
-        launch_point_side(h->P, h->st2);
-        cudaEventRecord(h->evJoin, h->st2);
-        launch_cam_side(h->P, h->d_img_chunk_start, h->d_tmpG, h->st);
-    }
+    launch_cam_side(h->P, h->d_img_chunk_start, h->d_tmpG, h->st);
+    launch_point_side(h->P, h->st2);
+    cudaEventRecord(h->evJoin, h->st2);
     cudaStreamWaitEvent(h->st, h->evJoin, 0);
     const bool clearPrior = h->nranks > 1;      // the in-place allreduce below leaves the sums of all ranks in these arrays
     launch_prior_apply(h->P, h->d_x, h->d_camDiag, h->d_camG, h->d_col2pt, clearPrior, h->st);
@@ -980,12 +943,9 @@ static void finish_solve(dbat_handle* h, int* singular) {
     double mm[2];
     memcpy(mm, h->h_piv, sizeof(mm));
     const int info = (int)h->h_piv[2];
-    h->jp_vec = nullptr;
-    if (h->solve_jp) {
-        h->jp_cache[0] = h->h_scal[SC_JPP] + h->h_scal[SC_JPP + 2];
-        h->jp_cache[1] = h->h_scal[SC_JPP + 1] + h->h_scal[SC_JPP + 3];
-        h->jp_vec = h->solve_pout;
-    }
+    h->jp_cache[0] = h->h_scal[SC_JPP] + h->h_scal[SC_JPP + 2];
+    h->jp_cache[1] = h->h_scal[SC_JPP + 1] + h->h_scal[SC_JPP + 3];
+    h->jp_vec = h->solve_pout;
     const double ratio = mm[1] > 0 ? mm[0] / mm[1] : 1.0;      // no camera-side unknown at all: nothing to be singular
     *singular = (info != 0) || !(ratio * ratio > 2.220446049250313e-16);
 }
@@ -1060,19 +1020,16 @@ static int solve_step(dbat_handle* h, double lambda, bool jacobi, double* pout, 
         if (rc) return rc;
     }
     launch_unpermute(P, tc.xs, jacobi ? h->d_dscale : nullptr, h->d_pc, h->d_pEO, h->st);
-    static const bool fusedJp = !getenv("DBAT_JP_SEPARATE");
-    double* jpOut = fusedJp ? h->d_scal + SC_JPP : nullptr;
+    double* jpOut = h->d_scal + SC_JPP;
     launch_backsub(P, lambda, h->d_pc, h->d_pEO, pout, h->d_partial, h->d_camDiag, h->d_camG, jpOut, h->st, h->st2, h->evFork, h->evJoin);
-    if (jpOut) {
-        if (h->nranks > 1) { int rc = allreduce(h, jpOut, 2); if (rc) return rc; }     // point parts; the camera part is global already
-        cudaMemcpyAsync(h->h_scal + SC_JPP, jpOut, 4 * sizeof(double), cudaMemcpyDeviceToHost, h->st);
-    }
+    if (h->nranks > 1) { int rc = allreduce(h, jpOut, 2); if (rc) return rc; }     // point parts; the camera part is global already
+    cudaMemcpyAsync(h->h_scal + SC_JPP, jpOut, 4 * sizeof(double), cudaMemcpyDeviceToHost, h->st);
     // pivot statistics into pinned memory (a copy into pageable memory would block the host until it has run)
     h->h_piv[2] = 0;
     cudaMemcpyAsync(h->h_piv + 2, tc.d.info, sizeof(int), cudaMemcpyDeviceToHost, h->st);
     cudaMemcpyAsync(h->h_piv, tc.d.minmax, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->st);
     ph_end(h, PH_SOLVE, a);
-    h->solve_pout = pout; h->solve_jp = jpOut != nullptr;
+    h->solve_pout = pout;
     h->jp_vec = nullptr;
     if (!sync) return 0;
     cudaError_t e = cudaStreamSynchronize(h->st);
@@ -1192,36 +1149,33 @@ extern "C" int dbat_normal_step(dbat_handle* h, const double* x, double lambda, 
     if (x) { CK(cudaMemcpyAsync(h->d_x, x, sizeof(double) * h->P.n, cudaMemcpyHostToDevice, h->st)); h->cscWeighted = -1; mask_unowned(h, h->d_x); }
     const int64_t l0 = g_dbat_launches;
     // The whole iteration is queued without a host round trip; one synchronisation at the end, then the host-side
-    // parts of the three stages (DBAT_STEP_SYNC: synchronise after every stage, as the optimisers' first iteration does).
-    static const bool stepSync = getenv("DBAT_STEP_SYNC") != nullptr;
-    int rc = eval_full(h, stepSync);
+    // parts of the three stages.
+    int rc = eval_full(h, false);
     if (rc) return rc;
     int sing = 0;
-    rc = solve_step(h, lambda, (flags & 1) != 0, h->d_p, &sing, stepSync);
+    rc = solve_step(h, lambda, (flags & 1) != 0, h->d_p, &sing, false);
     if (rc) return rc;
     double jp2 = 0, rjp = 0, fNew = NAN, rrT = 0;
     // the step goes back to the host on the second stream, beside the trial-point residual (queued after it in host
     // order: a pageable destination makes the copy call block)
-    const bool sideCopy = p && (flags & 2) && !stepSync;
+    const bool sideCopy = p && (flags & 2);
     if (sideCopy) cudaEventRecord(h->evStep, h->st);
     else if (p) CK(cudaMemcpyAsync(p, h->d_p, sizeof(double) * h->P.n, cudaMemcpyDeviceToHost, h->st));
     if (flags & 2) {
         launch_axpy(1.0, h->d_p, h->d_x, h->d_t, h->P.n, h->st);
-        rc = eval_rr(h, h->d_t, &rrT, stepSync);
+        rc = eval_rr(h, h->d_t, &rrT, false);
         if (rc) return rc;
     }
     if (sideCopy) {
         cudaStreamWaitEvent(h->st2, h->evStep, 0);
         CK(cudaMemcpyAsync(p, h->d_p, sizeof(double) * h->P.n, cudaMemcpyDeviceToHost, h->st2));
     }
-    if (!stepSync) {
-        cudaError_t e = cudaStreamSynchronize(h->st);
-        if (e == cudaSuccess && sideCopy) e = cudaStreamSynchronize(h->st2);
-        if (e != cudaSuccess) { h->err = std::string("dbat_normal_step: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
-        if ((rc = finish_eval(h))) return rc;
-        finish_solve(h, &sing);
-        rrT = h->h_scal[SC_RRT];
-    }
+    cudaError_t e = cudaStreamSynchronize(h->st);
+    if (e == cudaSuccess && sideCopy) e = cudaStreamSynchronize(h->st2);
+    if (e != cudaSuccess) { h->err = std::string("dbat_normal_step: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
+    if ((rc = finish_eval(h))) return rc;
+    finish_solve(h, &sing);
+    rrT = h->h_scal[SC_RRT];
     const double f = 0.5 * h->h_scal[SC_RR];
     const bool jpCached = h->jp_vec == h->d_p;      // otherwise eval_jp sets the parameter arrays back to d_x
     rc = eval_jp(h, h->d_p, &jp2, &rjp);
@@ -1425,8 +1379,7 @@ static int solve_lm(dbat_handle* h, const dbat_opts* o, dbat_result* res, TraceO
             int sing = 0;
             // after the first iteration the solve and the trial-point residual are queued back to back and the host
             // waits once (LM never looks at the singular flag; the |Jp| statistics come out of the back-substitution)
-            static const bool stepSync = getenv("DBAT_STEP_SYNC") != nullptr;
-            const bool defer = n > 0 && !stepSync;
+            const bool defer = n > 0;
             if ((rc = solve_step(h, lambda, false, h->d_p, &sing, !defer))) return rc;   // :119
             if (res->nRr < cap + 1) res->rr[res->nRr++] = std::sqrt(rr);      // :122
             if (n == 0 && structurally_deficient(h)) {                // :126-135 (p = NaN)

@@ -10,7 +10,6 @@
 //   k_point_side (point-major order, one thread per object point): V_j, g_j, the IO x OP
 //                cross block and the per-observation EO x OP cross blocks W_o.
 // Both are HBM-bound streams (48-52 B read per observation, see DESIGN.md).
-#include <cstdlib>
 #include "kernels.cuh"
 #include "launch.h"
 
@@ -38,52 +37,8 @@ __device__ __forceinline__ double block_sum(double v, double* sm /* >= 32 double
     return t;
 }
 
-__global__ void k_scatter(const double* __restrict__ x, const int* __restrict__ src,
-                          const int* __restrict__ dest, double* __restrict__ arr, int cnt) {
-    int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k < cnt) arr[dest[k]] = x[src[k]];
-}
-
-// deserialize.m:28-30 on device: scatter x into the IO/EO/OP value arrays.
-void launch_deserialize(const double* x, const int* src, const int* dest, double* arr, int cnt,
-                        cudaStream_t st) {
-    if (cnt <= 0) return;
-    k_scatter<<<(cnt + 255) / 256, 256, 0, st>>>(x, src, dest, arr, cnt);
-    count_launch();
-}
-
-__global__ void k_image_setup(DevProblem P) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= P.nImg) return;
-    const double* e = P.EOval + 6 * (size_t)i;
-    ImgRec& g = P.img[i];
-    g.q0[0] = e[0]; g.q0[1] = e[1]; g.q0[2] = e[2];
-    sincos(e[3], &g.sw, &g.cw);
-    sincos(e[4], &g.sp, &g.cp);
-    sincos(e[5], &g.sk, &g.ck);
-}
-
-// IO records in slot layout from the IOval columns of the representative images.
-__global__ void k_io_setup(DevProblem P, const int* __restrict__ rep, int nIO) {
-    int u = blockIdx.x * blockDim.x + threadIdx.x;
-    if (u >= nIO) return;
-    const int NC = 5 + P.nK + P.nP;
-    const double* c = P.IOval + (size_t)NC * rep[u];
-    IORec& r = P.io[u];
-    for (int s = 0; s < DBAT_NSLOT; ++s) r.v[s] = 0.0;
-    for (int s = 0; s < 5; ++s) r.v[s] = c[s];
-    for (int k = 0; k < P.nK; ++k) r.v[DBAT_SLOT_K + k] = c[5 + k];
-    for (int k = 0; k < P.nP; ++k) r.v[DBAT_SLOT_P + k] = c[5 + P.nK + k];
-}
-
-void launch_param_setup(const DevProblem& P, const int* rep, int nIO, cudaStream_t st) {
-    k_image_setup<<<(P.nImg + 127) / 128, 128, 0, st>>>(P);
-    k_io_setup<<<(nIO + 127) / 128, 128, 0, st>>>(P, rep, nIO);
-    count_launch(2);
-}
-
-// The same in two launches instead of five (they sit on the critical path of every evaluation and every trial point):
-// one kernel runs the three deserialisation lists, one builds the image and the IO records.
+// deserialize.m:28-30 on device, in two launches (they sit on the critical path of every evaluation and every trial
+// point): one kernel scatters x into the IO / EO / OP value arrays (three lists), one builds the image and IO records.
 __global__ void __launch_bounds__(256) k_scatter3(const double* __restrict__ x, ScatterList a, ScatterList b, ScatterList c) {
     int blk = blockIdx.x;
     ScatterList l = a;
@@ -432,13 +387,13 @@ void launch_cam_side(const DevProblem& P, const int* img_chunk_start, double* tm
 }
 
 // ---------------------------------------------------------------------------------------------
-// point side: one thread per object point
+// point side: one thread per object point (the points of a list: those with more than DBAT_PSB observations)
 // ---------------------------------------------------------------------------------------------
 template <int MODEL>
 __global__ void __launch_bounds__(128, DBAT_EVAL_MINBLOCKS) k_point_side(DevProblem P, const int* __restrict__ list, int nList) {
     const int jj = blockIdx.x * blockDim.x + threadIdx.x;
-    if (jj >= (list ? nList : P.nOP)) return;
-    const int j = list ? list[jj] : jj;
+    if (jj >= nList) return;
+    const int j = list[jj];
     const double Q[3] = {P.OPval[3 * (size_t)j], P.OPval[3 * (size_t)j + 1], P.OPval[3 * (size_t)j + 2]};
     double m[3];
 #pragma unroll
@@ -610,12 +565,8 @@ __global__ void __launch_bounds__(DBAT_PSB, 3) k_point_side_obs(DevProblem P) {
     }
 }
 
-// compact point side (see k_cam_side_c): 9 IO columns, nK / nP compile-time; 11 items per point in phase 2
+// compact point side (see k_cam_side_c): 9 IO columns, nK / nP compile-time
 #define PSC_ROW 27     // A_op 6 | r 2 | A_io x-rows 9 | A_io y-rows 9 (+1: odd stride)
-#define PSC_ITEMS (CE_NA + 2)
-#ifndef PSC_DMMA
-#define PSC_DMMA 1                   // 0: the scalar phase 2 (one thread per (point, item)), kept as a cross-check
-#endif
 __device__ __constant__ unsigned char c_ceSlot[CE_NA] = {0, 1, 2, 3, 5, 6, 7, 10, 11};
 #ifndef PSC_MINB
 #define PSC_MINB 5
@@ -686,7 +637,6 @@ __global__ void __launch_bounds__(DBAT_PSB, PSC_MINB) k_point_side_obs_c(DevProb
         }
     }
     __syncthreads();
-#if PSC_DMMA
     {
         // Phase 2 on the FP64 tensor pipe: per point the 3 x 13 product  A_op' [A_op | r | A_io]  over its 2 n rows
         // (observation, x/y).  One warp per point; one k-step of m8n8k4 takes two observations; rows 3..7 of the A
@@ -732,55 +682,10 @@ __global__ void __launch_bounds__(DBAT_PSB, PSC_MINB) k_point_side_obs_c(DevProb
             }
         }
     }
-    return;
-#endif
-    const int nItems = (p1 - p0) * PSC_ITEMS;
-    for (int item = tid; item < nItems; item += DBAT_PSB) {
-        const int jj = item / PSC_ITEMS, it = item - jj * PSC_ITEMS;
-        const int j = p0 + jj;
-        const int r0 = P.pt_start[j] - ob0, r1 = P.pt_start[j + 1] - ob0;
-        double* rec = P.pt + (size_t)j * DBAT_PT_STRIDE;
-        if (it < CE_NA) {                                    // IO slot x OP cross block
-            double a0 = 0.0, a1 = 0.0, a2 = 0.0;
-            for (int r = r0; r < r1; ++r) {
-                const double* row = rows + r * PSC_ROW;
-                const double u0 = row[8 + it], u1 = row[8 + CE_NA + it];
-                a0 = fma(u1, row[3], fma(u0, row[0], a0)); a1 = fma(u1, row[4], fma(u0, row[1], a1)); a2 = fma(u1, row[5], fma(u0, row[2], a2));
-            }
-            double* d = rec + DBAT_PT_WSH + 3 * c_ceSlot[it];
-            d[0] = a0; d[1] = a1; d[2] = a2;
-        } else if (it == CE_NA) {                            // V_j (upper triangle, row-wise)
-            double V[6] = {0, 0, 0, 0, 0, 0};
-            for (int r = r0; r < r1; ++r) {
-                const double* row = rows + r * PSC_ROW;
-                V[0] += row[0] * row[0] + row[3] * row[3];
-                V[1] += row[0] * row[1] + row[3] * row[4];
-                V[2] += row[0] * row[2] + row[3] * row[5];
-                V[3] += row[1] * row[1] + row[4] * row[4];
-                V[4] += row[1] * row[2] + row[4] * row[5];
-                V[5] += row[2] * row[2] + row[5] * row[5];
-            }
-#pragma unroll
-            for (int k = 0; k < 6; ++k) rec[k] = V[k];
-        } else {                                             // g_j
-            double g0 = 0.0, g1 = 0.0, g2 = 0.0;
-            for (int r = r0; r < r1; ++r) {
-                const double* row = rows + r * PSC_ROW;
-                g0 += row[0] * row[6] + row[3] * row[7]; g1 += row[1] * row[6] + row[4] * row[7]; g2 += row[2] * row[6] + row[5] * row[7];
-            }
-            rec[6] = g0; rec[7] = g1; rec[8] = g2; rec[9] = 0.0;
-        }
-    }
 }
 
 template <int MODEL>
 static void launch_point_side_t(const DevProblem& P, cudaStream_t st) {
-    static const bool perPoint = getenv("DBAT_POINT_SIDE_PER_POINT") != nullptr;
-    if (perPoint || !P.psb_pt) {
-        if (P.nOP > 0) k_point_side<MODEL><<<(P.nOP + 127) / 128, 128, 0, st>>>(P, nullptr, 0);
-        count_launch();
-        return;
-    }
     if (P.nPsb > 0) {
         if (P.evalCompact) k_point_side_obs_c<MODEL><<<P.nPsb, DBAT_PSB, 0, st>>>(P);
         else k_point_side_obs<MODEL><<<P.nPsb, DBAT_PSB, 0, st>>>(P);

@@ -15,13 +15,9 @@
 #define DBAT_CHUNK 1024            // max observations per camera-side chunk (one CTA)
 #define DBAT_PT_STRIDE 52          // doubles per point record: V[6] g[3] pad Wsh[14][3]
 #define DBAT_PT_WSH 10
-#define DBAT_W_STRIDE 18
+#define DBAT_W_STRIDE 18           // doubles per observation cross block W_o (6 EO x 3 OP)
 #define DBAT_NCAM (DBAT_NSLOT + 6)  // camera-side parameters of one image: IO slots then EO
 #define DBAT_WF_STRIDE (3 * DBAT_NCAM)
-#define DBAT_PTAUX_STRIDE 46       // Vg[3], pad, Ysh[14][3]
-#define DBAT_PTAUX_YSH 4
-#define DBAT_SHCOLS 16              // NSLOT shared columns + rhs + pad
-#define DBAT_SHCHUNK 1024           // points per CTA in the shared x shared reduction           // doubles per observation cross block W_o (6 EO x 3 OP)
 
 static_assert(DBAT_NSLOT + 7 <= DBAT_GW, "Gram width");
 
@@ -93,34 +89,18 @@ struct DevProblem {
     double* pt;            // nOP x PT_STRIDE point records
     double* W;             // nObs x 18       cross blocks, point-major order
     double* rhs;           // ldS             reduced right-hand side (S order)
-    // deterministic Schur reduction (index built once at create, schur_index.cu)
-    double* Y;             // nObs x 18       Y_o = W_o (V_j + lambda I)^-1, point-major order
-    double* ptaux;         // nOP x PTAUX_STRIDE : Vg[3], pad, Ysh[14][3]
-    const int* img_start;  // nImg+1 camera-major observation ranges
-    const int* cm2pm;      // camera-major observation -> point-major index
     const int* pt_pm;      // point of every point-major observation
-    const long long* pairs;      // sorted (oA<<32|oB) pm-index pairs, grouped by camera-pair block
-    const long long* blk_key;    // nBlk: imgA * nImg + imgB  (imgA >= imgB)
-    const long long* blk_off;    // nBlk+1 offsets into pairs
-    int nBlk;
-    double* shPart;        // per-CTA partials of the shared x shared reduction
-    // grouped Schur update (default): points sorted by their image list; a group is a run of <= 16
-    // neighbouring points whose image lists have a small union, so the camera x camera blocks of a
-    // whole group are summed on chip and reach S with one atomic per entry
+    // Schur reduction: estimated points sorted by their image list; a group is a run of <= WIN_GP neighbouring
+    // points whose image lists have a union of at most 12 images (schur_win.cu)
     const int* grp_pt;     // point ids, grouped
-    const int* grp_start;  // nGrp+1 offsets into grp_pt
-    const int* grp_img_off;      // nGrp+1 offsets into grp_img
-    const int* grp_img;          // ascending union of the image lists of every group
-    const unsigned char* obs_slot;   // per point-major observation: position of its image in the group's union
-    int nGrp;
-    int grpMaxRays;        // largest union among the groups (sizes the kernel's shared memory)
-    const int* big_pt;     // points with more than DBAT_GRP_MAXM rays (per-point kernel)
+    int grpMaxRays;        // largest union among the groups (sizes the window kernel's operand)
+    const int* big_pt;     // points with more than DBAT_GRP_MAXM rays (k_schur_atomic)
     int nBig;
-    double* vinv;          // nOP x 8: (V_j + lambda I)^-1 (6 entries) of the current solve
-    // window Schur (default, schur_win.cu): clusters of consecutive groups accumulate their camera x camera blocks in
+    double* vinv;          // nOP x 8: (V_j + lambda I)^-1 (6 entries) for dbat_cov (launch_point_vinv)
+    // window Schur (schur_win.cu): clusters of consecutive groups accumulate their camera x camera blocks in
     // shared memory; every cluster leaves ONE image of its window in a staging buffer and a second kernel sums the
     // images per block of S in a fixed order (index built at create) - no atomics, bit-reproducible
-    const WinHdr* win_hdr; // nGrp
+    const WinHdr* win_hdr; // one per group
     const int* clu_grp;    // nClu+1: first group of every cluster
     const int* clu_order;  // nClu: cluster ids, most groups first (launch order)
     const int* clu_img_off;      // nClu+1 offsets into clu_img
@@ -137,4 +117,4 @@ struct DevProblem {
     const long long* redi_off;   // staging offset of entry (shared row 0, EO element 0) of the contribution
     double* win_ssPart;    // per 256 clusters: partial sums of the 16 x 16 shared x shared tables
 };
-#define DBAT_GRP_MAXM 20   // grouped path up to 20 rays per point (= WIN_MAXW); more rays: per-point kernel
+#define DBAT_GRP_MAXM 20   // grouped path up to 20 rays per point (= WIN_MAXW); more rays: k_schur_atomic

@@ -10,8 +10,6 @@ extern int64_t g_dbat_launches;
 static inline void count_launch(int n = 1) { __atomic_fetch_add(&g_dbat_launches, (int64_t)n, __ATOMIC_RELAXED); }
 
 // eval.cu
-void launch_deserialize(const double* x, const int* src, const int* dest, double* arr, int cnt, cudaStream_t st);
-void launch_param_setup(const DevProblem& P, const int* rep, int nIO, cudaStream_t st);
 struct ScatterList { const int* src; const int* dest; double* arr; int cnt; int nb; };
 void launch_set_params(const DevProblem& P, const double* x, ScatterList io, ScatterList eo, ScatterList op,
                        const int* rep, int nIO, cudaStream_t st);
@@ -44,7 +42,7 @@ void launch_axpy(double alpha, const double* x, const double* y, double* out, in
 void launch_inv_sqrt(const double* in, double* out, int n, cudaStream_t st);
 void launch_mul(const double* a, const double* b, double* out, int n, cudaStream_t st);
 
-// schur_win.cu (default Schur reduction: window accumulation per point cluster + fixed-order sums, no atomics)
+// schur_win.cu (Schur reduction: window accumulation per point cluster + fixed-order sums, no atomics)
 void launch_schur_win(const DevProblem& P, double lambda, const double* shAcc, cudaStream_t st);
 
 // general_io.cu (general IO block structure)
@@ -55,11 +53,6 @@ int launch_backsub_gen(const DevProblem& P, double lambda, double* p, double* st
 void launch_cop_gen(const DevProblem& P, const double* C, int ldc, const double* dsc, double s02, double* out, cudaStream_t st);
 void launch_io_diag_grad_gen(const DevProblem& P, const double* camDiag, const double* camG, double* diagN, double* grad,
                              cudaStream_t st);
-
-// schur_index.cu
-int build_pair_index(const int* d_pt_start, const int* d_img_pm, const long long* h_pair_off, int nOP,
-                     int nImg, long long** d_pairs, long long** d_blk_key, long long** d_blk_off, int* nBlk,
-                     cudaStream_t st);
 
 // chol.cu
 struct CholWork {

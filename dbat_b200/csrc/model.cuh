@@ -18,7 +18,7 @@
 #define DBAT_SLOT_K 5
 #define DBAT_SLOT_P (5 + DBAT_KMAX)
 
-// Per-image record rebuilt from x before every evaluation (k_image_setup).
+// Per-image record rebuilt from x before every evaluation (k_param_setup, eval.cu).
 struct __align__(16) ImgRec {
     double sw, cw, sp, cp, sk, ck;        // sin/cos of omega, phi, kappa
     double q0[3];                         // camera centre

@@ -4,7 +4,6 @@
 // (gauss_newton_armijo.m:166-174) with the block elimination of SURVEY.md Appendix A:
 //   S = N_cc + lambda*I - sum_j W~_j (V_j + lambda*I)^-1 W~_j',   rhs = -g_c + sum_j W~_j (..)^-1 g_j
 //   p_j = (V_j + lambda*I)^-1 (-g_j - W~_j' p_c)
-#include <cstdlib>
 #include "kernels.cuh"
 #include <algorithm>
 #include "launch.h"
@@ -146,199 +145,10 @@ void launch_build_S(const DevProblem& P, const double* camDiag, const double* ca
     count_launch();
 }
 
-// ---------------------------------------------------------------------------------------------
-// Deterministic Schur reduction.  No atomics: every entry of S is owned by exactly one warp and
-// all sums run in a fixed order (pairs inside a camera-pair block are in point order).
-//   k_point_prep   per point: Vi=(V+lambda I)^-1, Vg=Vi g, Ysh=Wsh Vi, Y_o=W_o Vi
-//   k_schur_pairs  warp per camera-pair block (a,b): S_ab -= sum Y_oA W_oB'       (index from create)
-//   k_schur_cam    CTA per image: S(eo_i, sh) -= sum_o W_o Ysh_j' ; rhs(eo_i) += sum_o W_o Vg_j
-//   k_schur_sh     shared x shared and rhs_sh: per-CTA partials, then one fixed-order final sum
-// ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) k_point_prep(DevProblem P, double lambda) {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= P.nOP) return;
-    const double* rec = P.pt + (size_t)j * DBAT_PT_STRIDE;
-    const int* opc = P.op_col + 3 * (size_t)j;
-    double* aux = P.ptaux + (size_t)j * DBAT_PTAUX_STRIDE;
-    double Vi[6];
-    point_inverse(rec, opc, lambda, Vi);         // fixed coordinates give zero rows/cols
-    const double gj[3] = {rec[6], rec[7], rec[8]};
-    double v[3];
-    symv3(Vi, gj, v);
-    aux[0] = v[0]; aux[1] = v[1]; aux[2] = v[2]; aux[3] = 0.0;
-#pragma unroll
-    for (int s = 0; s < DBAT_NSLOT; ++s) {
-        const double w[3] = {rec[DBAT_PT_WSH + 3 * s], rec[DBAT_PT_WSH + 3 * s + 1], rec[DBAT_PT_WSH + 3 * s + 2]};
-        symv3(Vi, w, v);
-        aux[DBAT_PTAUX_YSH + 3 * s] = v[0]; aux[DBAT_PTAUX_YSH + 3 * s + 1] = v[1]; aux[DBAT_PTAUX_YSH + 3 * s + 2] = v[2];
-    }
-    const int o0 = P.pt_start[j], o1 = P.pt_start[j + 1];
-    for (int ob = o0; ob < o1; ++ob) {
-        const double* Wo = P.W + (size_t)ob * DBAT_W_STRIDE;
-        double* Yo = P.Y + (size_t)ob * DBAT_W_STRIDE;
-#pragma unroll
-        for (int a = 0; a < 6; ++a) {
-            const double w[3] = {Wo[3 * a], Wo[3 * a + 1], Wo[3 * a + 2]};
-            symv3(Vi, w, v);
-            Yo[3 * a] = v[0]; Yo[3 * a + 1] = v[1]; Yo[3 * a + 2] = v[2];
-        }
-    }
-}
-
-__global__ void __launch_bounds__(256) k_schur_pairs(DevProblem P) {
-    const int lane = threadIdx.x & 31;
-    const int warpGlobal = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int nWarps = (gridDim.x * blockDim.x) >> 5;
-    for (int blk = warpGlobal; blk < P.nBlk; blk += nWarps) {
-        const long long key = P.blk_key[blk];
-        const int ia = (int)(key / P.nImg), ib = (int)(key % P.nImg);
-        const long long e0 = P.blk_off[blk], e1 = P.blk_off[blk + 1];
-        double acc[6][6];
-#pragma unroll
-        for (int a = 0; a < 6; ++a)
-#pragma unroll
-            for (int b = 0; b < 6; ++b) acc[a][b] = 0.0;
-        for (long long e = e0 + lane; e < e1; e += 32) {
-            const long long pr = P.pairs[e];
-            const double2* Ya = reinterpret_cast<const double2*>(P.Y + (size_t)(pr >> 32) * DBAT_W_STRIDE);
-            const double2* Wb = reinterpret_cast<const double2*>(P.W + (size_t)(pr & 0xffffffffll) * DBAT_W_STRIDE);
-            double ya[18], wb[18];
-#pragma unroll
-            for (int q = 0; q < 9; ++q) { const double2 t = Ya[q]; ya[2 * q] = t.x; ya[2 * q + 1] = t.y; }
-#pragma unroll
-            for (int q = 0; q < 9; ++q) { const double2 t = Wb[q]; wb[2 * q] = t.x; wb[2 * q + 1] = t.y; }
-#pragma unroll
-            for (int a = 0; a < 6; ++a)
-#pragma unroll
-                for (int b = 0; b < 6; ++b)
-                    acc[a][b] += ya[3 * a] * wb[3 * b] + ya[3 * a + 1] * wb[3 * b + 1] + ya[3 * a + 2] * wb[3 * b + 2];
-        }
-#pragma unroll
-        for (int a = 0; a < 6; ++a)
-#pragma unroll
-            for (int b = 0; b < 6; ++b)
-#pragma unroll
-                for (int o = 16; o > 0; o >>= 1) acc[a][b] += __shfl_xor_sync(0xffffffffu, acc[a][b], o);
-        const int* ra = P.eo_s + 6 * (size_t)ia;
-        const int* cb = P.eo_s + 6 * (size_t)ib;
-#pragma unroll
-        for (int a = 0; a < 6; ++a)
-#pragma unroll
-            for (int b = 0; b < 6; ++b)
-                if (lane == ((a * 6 + b) & 31)) {
-                    const int row = ra[a], col = cb[b];
-                    if (row < 0 || col < 0) continue;
-                    if (ia == ib) { if (col <= row) *tc_at(P.T, row, col) -= acc[a][b]; }
-                    else *tc_at(P.T, max(row, col), min(row, col)) -= acc[a][b];
-                }
-    }
-}
-
-__global__ void __launch_bounds__(128) k_schur_cam(DevProblem P) {
-    const int i = blockIdx.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    double acc[6][4];
-#pragma unroll
-    for (int a = 0; a < 6; ++a)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) acc[a][c] = 0.0;
-    for (int k = P.img_start[i] + lane; k < P.img_start[i + 1]; k += 32) {
-        const int o = P.cm2pm[k];
-        const double* Wo = P.W + (size_t)o * DBAT_W_STRIDE;
-        const double* aux = P.ptaux + (size_t)P.pt_pm[o] * DBAT_PTAUX_STRIDE;
-        double wo[18];
-#pragma unroll
-        for (int q = 0; q < 18; ++q) wo[q] = Wo[q];
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-            const int col = 4 * w + c;                       // 0..13 shared slots, 14 = rhs, 15 = unused
-            const double* v = (col < DBAT_NSLOT) ? aux + DBAT_PTAUX_YSH + 3 * col : aux;
-            const double m = (col <= DBAT_NSLOT) ? 1.0 : 0.0;
-            const double v0 = v[0] * m, v1 = v[1] * m, v2 = v[2] * m;
-#pragma unroll
-            for (int a = 0; a < 6; ++a) acc[a][c] += wo[3 * a] * v0 + wo[3 * a + 1] * v1 + wo[3 * a + 2] * v2;
-        }
-    }
-#pragma unroll
-    for (int a = 0; a < 6; ++a)
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) acc[a][c] += __shfl_xor_sync(0xffffffffu, acc[a][c], o);
-    const int* ec = P.eo_s + 6 * (size_t)i;
-#pragma unroll
-    for (int a = 0; a < 6; ++a)
-#pragma unroll
-        for (int c = 0; c < 4; ++c)
-            if (lane == a * 4 + c) {
-                const int row = ec[a], col = 4 * w + c;
-                if (row >= 0) {
-                    if (col < DBAT_NSLOT) { const int sc = P.sh_s[col]; if (sc >= 0) *tc_at(P.T, sc, row) -= acc[a][c]; }
-                    else if (col == DBAT_NSLOT) P.rhs[row] += acc[a][c];
-                }
-            }
-}
-
-// shared x shared: sum_j Wsh_j [Ysh_j | Vg_j]'  (NSLOT x (NSLOT+1)); warp w of a CTA owns columns 2w, 2w+1
-__global__ void __launch_bounds__(256) k_schur_sh(DevProblem P) {
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int j0 = blockIdx.x * DBAT_SHCHUNK, j1 = min(P.nOP, j0 + DBAT_SHCHUNK);
-    double acc[DBAT_NSLOT][2];
-#pragma unroll
-    for (int s = 0; s < DBAT_NSLOT; ++s) { acc[s][0] = 0.0; acc[s][1] = 0.0; }
-    for (int j = j0 + lane; j < j1; j += 32) {
-        const double* ws = P.pt + (size_t)j * DBAT_PT_STRIDE + DBAT_PT_WSH;
-        const double* aux = P.ptaux + (size_t)j * DBAT_PTAUX_STRIDE;
-        double v[2][3];
-#pragma unroll
-        for (int c = 0; c < 2; ++c) {
-            const int col = 2 * w + c;
-            const double* p = (col < DBAT_NSLOT) ? aux + DBAT_PTAUX_YSH + 3 * col : aux;
-            const double m = (col <= DBAT_NSLOT) ? 1.0 : 0.0;
-            v[c][0] = p[0] * m; v[c][1] = p[1] * m; v[c][2] = p[2] * m;
-        }
-#pragma unroll
-        for (int s = 0; s < DBAT_NSLOT; ++s) {
-            const double a0 = ws[3 * s], a1 = ws[3 * s + 1], a2 = ws[3 * s + 2];
-            acc[s][0] += a0 * v[0][0] + a1 * v[0][1] + a2 * v[0][2];
-            acc[s][1] += a0 * v[1][0] + a1 * v[1][1] + a2 * v[1][2];
-        }
-    }
-#pragma unroll
-    for (int s = 0; s < DBAT_NSLOT; ++s)
-#pragma unroll
-        for (int c = 0; c < 2; ++c)
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) acc[s][c] += __shfl_xor_sync(0xffffffffu, acc[s][c], o);
-    double* out = P.shPart + (size_t)blockIdx.x * (DBAT_NSLOT * DBAT_SHCOLS);
-#pragma unroll
-    for (int s = 0; s < DBAT_NSLOT; ++s)
-#pragma unroll
-        for (int c = 0; c < 2; ++c)
-            if (lane == ((s * 2 + c) & 31)) out[s * DBAT_SHCOLS + 2 * w + c] = acc[s][c];
-}
-__global__ void k_schur_sh_final(DevProblem P, int nPart) {
-    for (int e = threadIdx.x; e < DBAT_NSLOT * DBAT_SHCOLS; e += blockDim.x) {
-        const int s = e / DBAT_SHCOLS, c = e % DBAT_SHCOLS;
-        double t = 0.0;
-        for (int q = 0; q < nPart; ++q) t += P.shPart[(size_t)q * (DBAT_NSLOT * DBAT_SHCOLS) + e];
-        const int row = P.sh_s[s];
-        if (row < 0) continue;
-        if (c < DBAT_NSLOT) {
-            const int col = P.sh_s[c];
-            if (col >= 0 && c <= s) *tc_at(P.T, row, col) -= t;
-        } else if (c == DBAT_NSLOT) {
-            P.rhs[row] += t;
-        }
-    }
-}
-// ---------------------------------------------------------------------------------------------
-// Fast Schur update (default): one warp per object point, lane = (pair, EO row), 6x6 pair
-// blocks scattered with FP64 red.global.add (6 consecutive rows per lane group -> coalesced
-// sectors; the kernel is bound by the L2 FP64-atomic rate, ~8.5e10 sector-ops/s measured).  The sum ORDER into an
-// entry of S is not fixed (results agree with the deterministic path to ~1e-16 relative); set
-// DBAT_SCHUR=det to use the pair-index kernels above instead.
-// ---------------------------------------------------------------------------------------------
-// Schur update, one warp per object point (v1: FP64 atomics into the dense lower triangle).
+// Schur update of the points with more than DBAT_GRP_MAXM rays, which the window kernels (schur_win.cu) do not take:
+// one warp per point, lane = (pair, EO row), 6x6 pair blocks scattered with FP64 red.global.add (6 consecutive rows
+// per lane group -> coalesced sectors).  The shared x shared table and its rhs column go to shAcc.  The sum ORDER into
+// an entry of S is not fixed, so a project with such points is not bit-reproducible from run to run.
 __global__ void __launch_bounds__(256) k_schur_atomic(DevProblem P, double lambda, double* __restrict__ shAcc,
                                                       const int* __restrict__ list, int nList) {
     const int lane = threadIdx.x & 31;
@@ -351,9 +161,8 @@ __global__ void __launch_bounds__(256) k_schur_atomic(DevProblem P, double lambd
 #pragma unroll
     for (int k = 0; k < NEL; ++k) accSh[k] = 0.0;
 
-    const int nPts = list ? nList : P.nOP;
-    for (int jj = warpGlobal; jj < nPts; jj += nWarps) {
-        const int j = list ? list[jj] : jj;
+    for (int jj = warpGlobal; jj < nList; jj += nWarps) {
+        const int j = list[jj];
         const double* rec = P.pt + (size_t)j * DBAT_PT_STRIDE;
         const int* opc = P.op_col + 3 * (size_t)j;
         if (opc[0] < 0 && opc[1] < 0 && opc[2] < 0) continue;
@@ -425,22 +234,7 @@ __global__ void __launch_bounds__(256) k_schur_atomic(DevProblem P, double lambd
     }
 }
 
-// ---------------------------------------------------------------------------------------------
-// Grouped Schur update (default).  Points are sorted by their image list at create; a group is a
-// run of ng <= 16 points seen by exactly the same m images.  For one group the whole update is ONE
-// small dense contraction over k = (point, coordinate), K = 3 ng:
-//     What (6m x K)   rows: the EO x OP blocks W_o of all points side by side
-//     Wsh  (15 x K)   rows: the shared IO x OP slots and the gradient g_j
-//     Yhat = What (V + lambda I)^-1 per point,   Ysh likewise
-//     S[cams, cams] -= Yhat What'    S[shared, cams] -= Yhat Wsh'    rhs += Yhat g    shared x shared += Ysh Wsh'
-// One CTA per group stages What / Wsh with coalesced loads, forms Yhat once per row, and runs the
-// product on the FP64 tensor pipe (DMMA m8n8k4, 8x8 output tiles of the lower triangle dealt to the
-// warps).  Every C fragment goes to S with one `red.global.add` per entry (8 consecutive rows per
-// 8 lanes); the shared x shared tiles stay in registers across all groups of the CTA.
-// With the 10-nearest-camera visibility of the synthetic blocks a group holds ~5-7 points: that many
-// times fewer atomics than one flush per point (which bound the per-point kernel this replaced), and
-// ~3x fewer instructions and shared-memory bytes than the same sums with scalar FP64 FMAs.
-// ---------------------------------------------------------------------------------------------
+// (V_j + lambda I)^-1 of every point into P.vinv (the point blocks of the covariance, dbat_cov)
 __global__ void k_point_vinv(DevProblem P, double lambda) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= P.nOP) return;
@@ -450,430 +244,24 @@ __global__ void k_point_vinv(DevProblem P, double lambda) {
     o[0] = make_double2(Vi[0], Vi[1]); o[1] = make_double2(Vi[2], Vi[3]); o[2] = make_double2(Vi[4], Vi[5]);
 }
 
-#define GRP_TH 256
-#define GRP_CAP 16            // max points per group (create-time cap)
-#define GRP_LDK 52            // row stride of What / Yhat / Wsh: 3*GRP_CAP = 48 columns + 4 (= 4 mod 16: conflict-free fragments)
-struct GrpHeader {            // per-group data staged in shared memory (double-buffered)
-    int m, ng, maxobs;                           // images in the union, points, largest ray count of a point
-    int j[GRP_CAP], ob[GRP_CAP], nob[GRP_CAP];   // point id, first point-major observation, ray count
-    int eoc[DBAT_GRP_MAXM * 6];                  // S index of every EO element of the union's images (ascending)
-    double vi[GRP_CAP * 6];
-};
-// Registers of one thread's share of the next group's header (loaded early, stored late).
-struct GrpPrefetch { int j, ob, nob, eoc; double2 v01, v23, v45; int m, ng; };
-
-__device__ __forceinline__ void grp_prefetch(const DevProblem& P, int grp, int t, GrpPrefetch& f) {
-    f.m = 0; f.ng = 0; f.j = 0; f.ob = 0; f.nob = 0; f.eoc = -1;
-    if (grp >= P.nGrp) return;
-    const int g0 = P.grp_start[grp];
-    f.ng = P.grp_start[grp + 1] - g0;
-    const int i0 = P.grp_img_off[grp];
-    f.m = P.grp_img_off[grp + 1] - i0;
-    if (t < f.ng) {
-        f.j = P.grp_pt[g0 + t];
-        f.ob = P.pt_start[f.j];
-        f.nob = P.pt_start[f.j + 1] - f.ob;
-        const double2* vp = reinterpret_cast<const double2*>(P.vinv + (size_t)f.j * 8);
-        f.v01 = vp[0]; f.v23 = vp[1]; f.v45 = vp[2];
-    }
-    if (t >= 64 && t - 64 < 6 * f.m) f.eoc = P.eo_s[6 * (size_t)P.grp_img[i0 + (t - 64) / 6] + (t - 64) % 6];
-}
-__device__ __forceinline__ void grp_store(GrpHeader& h, int t, const GrpPrefetch& f) {
-    if (t == 0) { h.m = f.m; h.ng = f.ng; }
-    if (t < 32) {                                            // largest ray count of the group (warp 0)
-        int mo = t < f.ng ? f.nob : 0;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) mo = max(mo, __shfl_xor_sync(0xffffffffu, mo, o));
-        if (t == 0) h.maxobs = mo;
-    }
-    if (t < f.ng) {
-        h.j[t] = f.j; h.ob[t] = f.ob; h.nob[t] = f.nob;
-        double* sv = h.vi + 6 * t;
-        sv[0] = f.v01.x; sv[1] = f.v01.y; sv[2] = f.v23.x; sv[3] = f.v23.y; sv[4] = f.v45.x; sv[5] = f.v45.y;
-    }
-    if (t >= 64 && t - 64 < 6 * f.m) h.eoc[t - 64] = f.eoc;
-}
-
-__device__ __forceinline__ void dmma_s(double& c0, double& c1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};"
-                 : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
-// dynamic shared memory (RW = 6m rounded up to 8, for the largest m of the problem):
-//   What[RW][LDK] | Yhat[RW + 16][LDK] (rows RW.. : Ysh) | Wsh[16][LDK]
-__global__ void __launch_bounds__(GRP_TH, 3) k_schur_group(DevProblem P, double* __restrict__ shAcc) {
-    extern __shared__ __align__(16) double dsm[];
-    __shared__ GrpHeader s_hdr[2];
-    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-    const int fr = lane >> 2, fk = lane & 3;
-    const int RWmax = (6 * P.grpMaxRays + 7) & ~7;
-    double* What = dsm;
-    double* Yhat = What + RWmax * GRP_LDK;
-    double* Wsh = Yhat + (RWmax + 16) * GRP_LDK;
-    for (int i = t; i < (2 * RWmax + 32) * GRP_LDK; i += GRP_TH) dsm[i] = 0.0;     // padding rows / columns stay zero
-    double accSh[2] = {0.0, 0.0};                // warps 0..3: one 8x8 tile of the shared x shared table each
-    int buf = 0;
-    {
-        GrpPrefetch f;
-        grp_prefetch(P, blockIdx.x, t, f);
-        grp_store(s_hdr[0], t, f);
-    }
-    __syncthreads();
-    for (int grp = blockIdx.x; grp < P.nGrp; grp += gridDim.x, buf ^= 1) {
-        GrpHeader& H = s_hdr[buf];
-        GrpPrefetch nxt;
-        grp_prefetch(P, grp + gridDim.x, t, nxt);            // in flight during this group's work
-        const int m = H.m, ng = H.ng;
-        const int R = 6 * m, RT = (R + 7) >> 3;              // camera rows, 8-row tiles
-        const int K = 3 * ng, Kp = (K + 3) & ~3;
-        // ---- stage What: the 6x3 block of observation o of point gi goes to the rows of its image's
-        //      position in the union (obs_slot); rows of images a point does not see stay zero
-        {
-            const int per = 18 * H.maxobs;
-            for (int idx = t; idx < ng * per; idx += GRP_TH) {
-                const int gi = idx / per, e18 = idx - gi * per, o = e18 / 18, e = e18 - 18 * o;   // e = 3 a + c
-                if (o < H.nob[gi]) {
-                    const int ob = H.ob[gi] + o;
-                    const int a = e / 3, c = e - 3 * a;
-                    What[(6 * P.obs_slot[ob] + a) * GRP_LDK + 3 * gi + c] = P.W[(size_t)ob * DBAT_W_STRIDE + e];
-                }
-            }
-        }
-        for (int idx = t; idx < ng * 45; idx += GRP_TH) {
-            const int gi = idx / 45, e = idx - gi * 45, sidx = e / 3, c = e - 3 * sidx;
-            const double* rec = P.pt + (size_t)H.j[gi] * DBAT_PT_STRIDE;
-            Wsh[sidx * GRP_LDK + 3 * gi + c] = sidx < DBAT_NSLOT ? rec[DBAT_PT_WSH + 3 * sidx + c] : rec[6 + c];
-        }
-        if (Kp > K) {                                        // k padding may hold a previous group's data
-            for (int idx = t; idx < (2 * RT * 8 + 32) * (Kp - K); idx += GRP_TH) {
-                const int row = idx / (Kp - K), k = K + idx - row * (Kp - K);
-                // rows: What [0, 8RT), Yhat [0, 8RT) and its 16 shared rows, Wsh 16 rows
-                double* base = row < 8 * RT ? What + row * GRP_LDK
-                             : row < 16 * RT ? Yhat + (row - 8 * RT) * GRP_LDK
-                             : row < 16 * RT + 16 ? Yhat + (RWmax + row - 16 * RT) * GRP_LDK
-                             : Wsh + (row - 16 * RT - 16) * GRP_LDK;
-                base[k] = 0.0;
-            }
-        }
-        __syncthreads();
-        // ---- Yhat = What V^-1 (camera rows), Ysh = Wsh V^-1: one (row, point) per thread
-        for (int idx = t; idx < ng * (R + 15); idx += GRP_TH) {
-            const int gi = idx / (R + 15), r = idx - gi * (R + 15);
-            const double* sv = H.vi + 6 * gi;
-            const double Vi[6] = {sv[0], sv[1], sv[2], sv[3], sv[4], sv[5]};
-            const double* w = (r < R ? What + r * GRP_LDK : Wsh + (r - R) * GRP_LDK) + 3 * gi;
-            const double w3[3] = {w[0], w[1], w[2]};
-            double y[3];
-            symv3(Vi, w3, y);
-            double* yo = (r < R ? Yhat + r * GRP_LDK : Yhat + (RWmax + r - R) * GRP_LDK) + 3 * gi;
-            yo[0] = y[0]; yo[1] = y[1]; yo[2] = y[2];
-        }
-        grp_store(s_hdr[buf ^ 1], t, nxt);
-        __syncthreads();
-        // ---- tiles: pair tiles (ti >= tj) of Yhat What', then RT x 2 tiles of Yhat Wsh'
-        const int nPair = RT * (RT + 1) / 2, nTile = nPair + 2 * RT;
-        for (int tile = warp; tile < nTile; tile += GRP_TH / 32) {
-            int ti, tj; const double* Bm;
-            if (tile < nPair) {
-                ti = (int)((sqrtf(8.0f * tile + 1.0f) - 1.0f) * 0.5f);
-                while ((ti + 1) * (ti + 2) / 2 <= tile) ++ti;
-                while (ti * (ti + 1) / 2 > tile) --ti;
-                tj = tile - ti * (ti + 1) / 2;
-                Bm = What;
-            } else { ti = (tile - nPair) >> 1; tj = (tile - nPair) & 1; Bm = Wsh; }
-            const double* pa = Yhat + (8 * ti + fr) * GRP_LDK + fk;
-            const double* pb = Bm + (8 * tj + fr) * GRP_LDK + fk;
-            double c0 = 0.0, c1 = 0.0, d0 = 0.0, d1 = 0.0;
-            for (int k0 = 0; k0 < Kp; k0 += 8) {             // two accumulator pairs: shorter dependent chains
-                dmma_s(c0, c1, pa[k0], pb[k0]);
-                if (k0 + 4 < Kp) dmma_s(d0, d1, pa[k0 + 4], pb[k0 + 4]);
-            }
-            c0 += d0; c1 += d1;
-            const int r = 8 * ti + fr;
-            if (r < R) {
-                const int row = H.eoc[r];
-                if (row >= 0) {
-                    if (tile < nPair) {
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const int c = 8 * tj + 2 * fk + e;
-                            if (c < R) {
-                                const int col = H.eoc[c];
-                                const double v = e ? c1 : c0;                 // exact zero: image pair not shared by any point
-                                if (col >= 0 && col <= row && v != 0.0) atomicAdd(tc_at(P.T, row, col), -v);
-                            }
-                        }
-                    } else {
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const int sidx = 8 * tj + 2 * fk + e;
-                            if (sidx < DBAT_NSLOT) {
-                                const int srow = P.sh_s[sidx];
-                                if (srow >= 0) atomicAdd(tc_at(P.T, srow, row), -(e ? c1 : c0));
-                            } else if (sidx == DBAT_NSLOT) {
-                                atomicAdd(&P.rhs[row], e ? c1 : c0);
-                            }
-                        }
-                    }
-                }
-            }
-        }
-        // ---- shared x shared (+ rhs column): Ysh Wsh', 2 x 2 tiles kept in registers by warps 0..3
-        if (warp < 4) {
-            const int ta = warp >> 1, tb = warp & 1;
-            const double* pa = Yhat + (RWmax + 8 * ta + fr) * GRP_LDK + fk;
-            const double* pb = Wsh + (8 * tb + fr) * GRP_LDK + fk;
-            for (int k0 = 0; k0 < Kp; k0 += 4) dmma_s(accSh[0], accSh[1], pa[k0], pb[k0]);
-        }
-        __syncthreads();
-        // What must be all zero where the next group does not write (images a point does not see)
-        for (int i = t; i < 8 * RT * (Kp / 2); i += GRP_TH) {
-            const int row = i / (Kp / 2), k2 = i - row * (Kp / 2);
-            *reinterpret_cast<double2*>(What + row * GRP_LDK + 2 * k2) = make_double2(0.0, 0.0);
-        }
-        __syncthreads();
-    }
-    if (warp < 4) {
-        const int a = 8 * (warp >> 1) + fr;
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            const int b = 8 * (warp & 1) + 2 * fk + e;
-            if (a < DBAT_NSLOT && (b == DBAT_NSLOT || b <= a) && b <= DBAT_NSLOT) {
-                const double v = e ? accSh[1] : accSh[0];
-                if (v != 0.0) atomicAdd(&shAcc[a * (DBAT_NSLOT + 1) + b], v);
-            }
-        }
-    }
-}
-// ---------------------------------------------------------------------------------------------
-// k_schur_group2: the same contraction with a third fewer instructions (the first version issued 20 k warp
-// instructions per group, most of them index arithmetic).
-//   * staging by (point, observation, block row): warp w takes points w, w + 8; a lane reads the 3 consecutive
-//     doubles of one row of a cross block (consecutive lanes -> consecutive 24-byte pieces: coalesced), applies
-//     (V + lambda I)^-1 at once and stores BOTH the What and the Yhat entry - no second pass, one barrier less;
-//     all divisions are by constants;
-//   * the list of lower-triangular tile pairs is a table in shared memory, built once per CTA;
-//   * What / Yhat are cleared with 16-byte stores at the top of every group.
-// ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(GRP_TH, 3) k_schur_group2(DevProblem P, double* __restrict__ shAcc) {
-    extern __shared__ __align__(16) double dsm[];
-    __shared__ GrpHeader s_hdr[2];
-    __shared__ unsigned char s_tij[2 * 153];              // (ti, tj) of the tile pairs, RT <= 17
-    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-    const int fr = lane >> 2, fk = lane & 3;
-    const int RWmax = (6 * P.grpMaxRays + 7) & ~7;
-    double* What = dsm;
-    double* Yhat = What + RWmax * GRP_LDK;
-    double* Wsh = Yhat + (RWmax + 16) * GRP_LDK;
-    for (int i = t; i < (2 * RWmax + 32) * GRP_LDK; i += GRP_TH) dsm[i] = 0.0;
-    for (int u = t; u < 153; u += GRP_TH) {
-        int i = (int)((sqrtf(8.0f * u + 1.0f) - 1.0f) * 0.5f);
-        while ((i + 1) * (i + 2) / 2 <= u) ++i;
-        while (i * (i + 1) / 2 > u) --i;
-        s_tij[2 * u] = (unsigned char)i; s_tij[2 * u + 1] = (unsigned char)(u - i * (i + 1) / 2);
-    }
-    double accSh[2] = {0.0, 0.0};
-    int buf = 0;
-    {
-        GrpPrefetch f;
-        grp_prefetch(P, blockIdx.x, t, f);
-        grp_store(s_hdr[0], t, f);
-    }
-    __syncthreads();
-    for (int grp = blockIdx.x; grp < P.nGrp; grp += gridDim.x, buf ^= 1) {
-        GrpHeader& H = s_hdr[buf];
-        GrpPrefetch nxt;
-        grp_prefetch(P, grp + gridDim.x, t, nxt);
-        const int m = H.m, ng = H.ng;
-        const int R = 6 * m, RT = (R + 7) >> 3;
-        const int K = 3 * ng, Kp = (K + 3) & ~3;
-        // ---- stage What and Yhat = What V^-1, Wsh and Ysh: warp w owns points w, w + 8
-        for (int gi = warp; gi < ng; gi += GRP_TH / 32) {
-            const double* sv = H.vi + 6 * gi;
-            const double v0 = sv[0], v1 = sv[1], v2 = sv[2], v3 = sv[3], v4 = sv[4], v5 = sv[5];
-            const int ob0 = H.ob[gi], nIt = 6 * H.nob[gi];
-            for (int it = lane; it < nIt; it += 32) {
-                const int o = it / 6, a = it - 6 * o;
-                const double* w = P.W + (size_t)(ob0 + o) * DBAT_W_STRIDE + 3 * a;
-                const double w0 = w[0], w1 = w[1], w2 = w[2];
-                const int row = 6 * P.obs_slot[ob0 + o] + a;
-                double* pw = What + row * GRP_LDK + 3 * gi;
-                double* py = Yhat + row * GRP_LDK + 3 * gi;
-                pw[0] = w0; pw[1] = w1; pw[2] = w2;
-                py[0] = v0 * w0 + v1 * w1 + v2 * w2; py[1] = v1 * w0 + v3 * w1 + v4 * w2; py[2] = v2 * w0 + v4 * w1 + v5 * w2;
-            }
-            if (lane < 15) {                                  // 14 shared IO slots and the gradient
-                const double* rec = P.pt + (size_t)H.j[gi] * DBAT_PT_STRIDE;
-                const double* w = lane < DBAT_NSLOT ? rec + DBAT_PT_WSH + 3 * lane : rec + 6;
-                const double w0 = w[0], w1 = w[1], w2 = w[2];
-                double* pw = Wsh + lane * GRP_LDK + 3 * gi;
-                double* py = Yhat + (RWmax + lane) * GRP_LDK + 3 * gi;
-                pw[0] = w0; pw[1] = w1; pw[2] = w2;
-                py[0] = v0 * w0 + v1 * w1 + v2 * w2; py[1] = v1 * w0 + v3 * w1 + v4 * w2; py[2] = v2 * w0 + v4 * w1 + v5 * w2;
-            }
-        }
-        grp_store(s_hdr[buf ^ 1], t, nxt);
-        __syncthreads();
-        // ---- tiles: pair tiles (ti >= tj) of Yhat What', then RT x 2 tiles of Yhat Wsh'
-        const int nPair = RT * (RT + 1) / 2, nTile = nPair + 2 * RT;
-        for (int tile = warp; tile < nTile; tile += GRP_TH / 32) {
-            int ti, tj; const double* Bm;
-            if (tile < nPair) { ti = s_tij[2 * tile]; tj = s_tij[2 * tile + 1]; Bm = What; }
-            else { ti = (tile - nPair) >> 1; tj = (tile - nPair) & 1; Bm = Wsh; }
-            const double* pa = Yhat + (8 * ti + fr) * GRP_LDK + fk;
-            const double* pb = Bm + (8 * tj + fr) * GRP_LDK + fk;
-            double c0 = 0.0, c1 = 0.0, d0 = 0.0, d1 = 0.0;
-            for (int k0 = 0; k0 < Kp; k0 += 8) {
-                dmma_s(c0, c1, pa[k0], pb[k0]);
-                if (k0 + 4 < Kp) dmma_s(d0, d1, pa[k0 + 4], pb[k0 + 4]);
-            }
-            c0 += d0; c1 += d1;
-            const int r = 8 * ti + fr;
-            if (r < R) {
-                const int row = H.eoc[r];
-                if (row >= 0) {
-                    if (tile < nPair) {
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const int c = 8 * tj + 2 * fk + e;
-                            const double v = e ? c1 : c0;
-                            if (c < R && v != 0.0) {
-                                const int col = H.eoc[c];
-                                if (col >= 0 && col <= row) atomicAdd(tc_at(P.T, row, col), -v);
-                            }
-                        }
-                    } else {
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const int sidx = 8 * tj + 2 * fk + e;
-                            if (sidx < DBAT_NSLOT) {
-                                const int srow = P.sh_s[sidx];
-                                if (srow >= 0) atomicAdd(tc_at(P.T, srow, row), -(e ? c1 : c0));
-                            } else if (sidx == DBAT_NSLOT) {
-                                atomicAdd(&P.rhs[row], e ? c1 : c0);
-                            }
-                        }
-                    }
-                }
-            }
-        }
-        if (warp < 4) {
-            const int ta = warp >> 1, tb = warp & 1;
-            const double* pa = Yhat + (RWmax + 8 * ta + fr) * GRP_LDK + fk;
-            const double* pb = Wsh + (8 * tb + fr) * GRP_LDK + fk;
-            for (int k0 = 0; k0 < Kp; k0 += 4) dmma_s(accSh[0], accSh[1], pa[k0], pb[k0]);
-        }
-        __syncthreads();
-        // ---- clear what this group wrote (rows of images a point does not see must read as zero): lane = 16-byte
-        //      piece of a row (Kp <= 48: at most 24 pieces), warps stride the rows of What, Yhat, Ysh, Wsh
-        if (lane < (Kp >> 1)) {
-            const int nA = 8 * RT;
-            for (int row = warp; row < 2 * nA + 32; row += GRP_TH / 32) {
-                double* base = row < nA ? What + row * GRP_LDK
-                             : row < 2 * nA ? Yhat + (row - nA) * GRP_LDK
-                             : row < 2 * nA + 16 ? Yhat + (RWmax + row - 2 * nA) * GRP_LDK
-                             : Wsh + (row - 2 * nA - 16) * GRP_LDK;
-                *reinterpret_cast<double2*>(base + 2 * lane) = make_double2(0.0, 0.0);
-            }
-        }
-        __syncthreads();
-    }
-    if (warp < 4) {
-        const int a = 8 * (warp >> 1) + fr;
-#pragma unroll
-        for (int e = 0; e < 2; ++e) {
-            const int b = 8 * (warp & 1) + 2 * fk + e;
-            if (a < DBAT_NSLOT && (b == DBAT_NSLOT || b <= a) && b <= DBAT_NSLOT) {
-                const double v = e ? accSh[1] : accSh[0];
-                if (v != 0.0) atomicAdd(&shAcc[a * (DBAT_NSLOT + 1) + b], v);
-            }
-        }
-    }
-}
-__global__ void k_schur_sh_apply(DevProblem P, const double* __restrict__ shAcc) {
-    for (int e = threadIdx.x; e < DBAT_NSLOT * (DBAT_NSLOT + 1); e += blockDim.x) {
-        const int a = e / (DBAT_NSLOT + 1), b = e % (DBAT_NSLOT + 1);
-        const int row = P.sh_s[a];
-        if (row < 0) continue;
-        if (b < DBAT_NSLOT) {
-            const int col = P.sh_s[b];
-            if (col < 0 || b > a) continue;
-            *tc_at(P.T, row, col) -= shAcc[e];
-        } else {
-            P.rhs[row] += shAcc[e];
-        }
-    }
-}
-
 void launch_point_vinv(const DevProblem& P, double lambda, cudaStream_t st) {
     if (P.nOP > 0) { k_point_vinv<<<(P.nOP + 255) / 256, 256, 0, st>>>(P, lambda); count_launch(); }
 }
-static int g_schur_mode = -1;       // 0 = window (default, no atomics), 1 = deterministic pair index, 2 = per-point atomic, 3 = grouped atomic
 static thread_local double* g_shAcc = nullptr;       // per device (one host thread drives one device)
 void launch_schur(const DevProblem& P, double lambda, cudaStream_t st) {
     if (P.nOP <= 0) return;
     if (P.ioGeneral) { launch_schur_gen(P, lambda, st); return; }
-    if (g_schur_mode < 0) {
-        const char* e = getenv("DBAT_SCHUR");
-        g_schur_mode = (e && e[0] == 'd') ? 1 : (e && e[0] == 'p') ? 2 : (e && e[0] == 'g') ? 3 : 0;
-    }
-    if (g_schur_mode == 0) {
-        // window accumulation + fixed-order reduction (schur_win.cu); only points with more than DBAT_GRP_MAXM rays
-        // (none at BASELINE configs 4 / 5) go through the per-point kernel and its atomics
-        const double* shAcc = nullptr;
-        if (P.nBig > 0) {
-            if (!g_shAcc) cudaMalloc(&g_shAcc, sizeof(double) * DBAT_NSLOT * (DBAT_NSLOT + 1));
-            cudaMemsetAsync(g_shAcc, 0, sizeof(double) * DBAT_NSLOT * (DBAT_NSLOT + 1), st);
-            k_schur_atomic<<<std::min((P.nBig + 7) / 8, 148 * 8), 256, 0, st>>>(P, lambda, g_shAcc, P.big_pt, P.nBig);
-            count_launch();
-            shAcc = g_shAcc;
-        }
-        launch_schur_win(P, lambda, shAcc, st);
-        return;
-    }
-    if (g_schur_mode != 1) {
+    // window accumulation + fixed-order reduction (schur_win.cu); only points with more than DBAT_GRP_MAXM rays
+    // (none at BASELINE configs 4 / 5) go through the per-point kernel and its atomics
+    const double* shAcc = nullptr;
+    if (P.nBig > 0) {
         if (!g_shAcc) cudaMalloc(&g_shAcc, sizeof(double) * DBAT_NSLOT * (DBAT_NSLOT + 1));
         cudaMemsetAsync(g_shAcc, 0, sizeof(double) * DBAT_NSLOT * (DBAT_NSLOT + 1), st);
-        if (g_schur_mode == 2) {
-            int nb = (P.nOP + 7) / 8;
-            if (nb > 148 * 8) nb = 148 * 8;
-            k_schur_atomic<<<nb, 256, 0, st>>>(P, lambda, g_shAcc, nullptr, 0);
-            count_launch();
-        } else {
-            k_point_vinv<<<(P.nOP + 255) / 256, 256, 0, st>>>(P, lambda);
-            if (P.nGrp > 0) {
-                static thread_local bool attr = false;
-                auto smem_for = [](int mm) { return (2 * ((6 * mm + 7) & ~7) + 32) * GRP_LDK * 8; };
-                if (!attr) {
-                    cudaFuncSetAttribute(k_schur_group, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_for(DBAT_GRP_MAXM));
-                    cudaFuncSetAttribute(k_schur_group2, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_for(DBAT_GRP_MAXM));
-                    attr = true;
-                }
-                static const bool v1 = getenv("DBAT_SCHUR_GROUP_V1") != nullptr;
-                if (v1) k_schur_group<<<std::min(P.nGrp, 148 * 24), GRP_TH, smem_for(P.grpMaxRays), st>>>(P, g_shAcc);
-                else k_schur_group2<<<std::min(P.nGrp, 148 * 24), GRP_TH, smem_for(P.grpMaxRays), st>>>(P, g_shAcc);
-                count_launch();
-            }
-            if (P.nBig > 0) {
-                k_schur_atomic<<<std::min((P.nBig + 7) / 8, 148 * 8), 256, 0, st>>>(P, lambda, g_shAcc, P.big_pt, P.nBig);
-                count_launch();
-            }
-            count_launch();
-        }
-        k_schur_sh_apply<<<1, 256, 0, st>>>(P, g_shAcc);
+        k_schur_atomic<<<std::min((P.nBig + 7) / 8, 148 * 8), 256, 0, st>>>(P, lambda, g_shAcc, P.big_pt, P.nBig);
         count_launch();
-        return;
+        shAcc = g_shAcc;
     }
-    k_point_prep<<<(P.nOP + 127) / 128, 128, 0, st>>>(P, lambda);
-    if (P.nBlk > 0) {
-        int nb = (P.nBlk + 7) / 8;
-        if (nb > 148 * 8) nb = 148 * 8;
-        k_schur_pairs<<<nb, 256, 0, st>>>(P);
-    }
-    k_schur_cam<<<P.nImg, 128, 0, st>>>(P);
-    const int nPart = (P.nOP + DBAT_SHCHUNK - 1) / DBAT_SHCHUNK;
-    k_schur_sh<<<nPart, 256, 0, st>>>(P);
-    k_schur_sh_final<<<1, 256, 0, st>>>(P, nPart);
-    count_launch(5);
+    launch_schur_win(P, lambda, shAcc, st);
 }
 
 // Jacobi column scaling (gauss_newton_armijo.m:166-172) of the reduced system: dS[s] = d[x column of s]
@@ -915,7 +303,8 @@ void launch_unpermute(const DevProblem& P, const double* xs, const double* d, do
     count_launch();
 }
 
-// back-substitution for the object points; p[0:nC] must already hold the camera/IO step.
+// back-substitution for the object points of `list` (those with more than DBAT_PSB observations), one thread per
+// point; p[0:nC] must already hold the camera/IO step.
 // By-product (stats != nullptr): this block's share of  p'J'Jp = |Jp|^2  and  r'Jp = g'p  over the point
 // columns, from the blocks already in registers - with a_j = W~_j' p_c and the UNDAMPED V_j, g_j:
 //     |Jp|^2 = p_c' N_cc p_c + sum_j ( p_j' V_j p_j + 2 p_j' a_j ),     r'Jp = g_c' p_c + sum_j g_j' p_j
@@ -925,7 +314,7 @@ __global__ void __launch_bounds__(128) k_backsub(DevProblem P, double lambda, do
                                                   const int* __restrict__ list, int nList) {
     __shared__ double red[2][4];
     const int jj = blockIdx.x * blockDim.x + threadIdx.x;
-    const int j = list ? (jj < nList ? list[jj] : P.nOP) : jj;
+    const int j = jj < nList ? list[jj] : P.nOP;
     double jp2 = 0.0, rjp = 0.0;
     if (j < P.nOP) {
         const int* opc = P.op_col + 3 * (size_t)j;
@@ -977,15 +366,12 @@ __global__ void __launch_bounds__(128) k_backsub(DevProblem P, double lambda, do
         }
     }
 }
-// The same back-substitution with one thread per OBSERVATION for the streaming part (default): the blocks of
+// The same back-substitution with one thread per OBSERVATION for all other points: the blocks of
 // k_point_side_obs (whole points, at most DBAT_PSB observations).  Phase 1: thread o reads its cross block W_o
 // (144 contiguous bytes, consecutive threads consecutive blocks: fully coalesced) and the six EO entries of p_c
 // of its image and leaves a_o = W_o' p_c in shared memory.  Phase 2: one thread per point adds the a_o of its
 // observations in image order, the shared IO part, solves with (V_j + lambda I)^-1 and forms the |Jp|^2 / r'Jp terms.
-#ifndef BSO_V2
-#define BSO_V2 1                    // 0: column lookup + gather of p per observation, no prefetch (the earlier version)
-#endif
-// BSO_V2: the EO step of the observation's image comes from the dense table pEO (three 16-byte loads instead of a column
+// The EO step of the observation's image comes from the dense table pEO (three 16-byte loads instead of a column
 // lookup and a dependent gather); the lines phase 2 will need (point record, column map) start towards L1 at once and
 // the shared IO step is read once per block.  Measured and dropped: the point's (V + lambda I)^-1 before the barrier
 // (more registers, fewer resident blocks: slower).
@@ -999,7 +385,6 @@ __global__ void __launch_bounds__(DBAT_PSB) k_backsub_obs(DevProblem P, double l
     const int tid = threadIdx.x;
     const int p0 = P.psb_pt[2 * blockIdx.x], p1 = P.psb_pt[2 * blockIdx.x + 1];
     const int ob0 = P.pt_start[p0], nob = P.pt_start[p1] - ob0;
-#if BSO_V2
     if (p0 + tid < p1) {
         const char* rec = reinterpret_cast<const char*>(P.pt + (size_t)(p0 + tid) * DBAT_PT_STRIDE);
 #pragma unroll
@@ -1013,7 +398,6 @@ __global__ void __launch_bounds__(DBAT_PSB) k_backsub_obs(DevProblem P, double l
         psh[s] = c >= 0 ? p[c] : 0.0;
         pshOk[s] = c >= 0;
     }
-#endif
     if (tid < nob) {
         const int ob = ob0 + tid;
         const double2* Wo = reinterpret_cast<const double2*>(P.W + (size_t)ob * DBAT_W_STRIDE);
@@ -1021,21 +405,11 @@ __global__ void __launch_bounds__(DBAT_PSB) k_backsub_obs(DevProblem P, double l
 #pragma unroll
         for (int q = 0; q < 9; ++q) { const double2 t = Wo[q]; w[2 * q] = t.x; w[2 * q + 1] = t.y; }
         double a0 = 0.0, a1 = 0.0, a2 = 0.0;
-#if BSO_V2
         const double2* pe = reinterpret_cast<const double2*>(pEO + 6 * (size_t)P.img_pm[ob]);
         const double2 e01 = pe[0], e23 = pe[1], e45 = pe[2];
         const double pv[6] = {e01.x, e01.y, e23.x, e23.y, e45.x, e45.y};
 #pragma unroll
         for (int e = 0; e < 6; ++e) { a0 += w[3 * e] * pv[e]; a1 += w[3 * e + 1] * pv[e]; a2 += w[3 * e + 2] * pv[e]; }
-#else
-        const int* ec = P.eo_col + 6 * (size_t)P.img_pm[ob];
-#pragma unroll
-        for (int e = 0; e < 6; ++e) {
-            const int c = ec[e];
-            const double pv = c >= 0 ? p[c] : 0.0;
-            a0 += w[3 * e] * pv; a1 += w[3 * e + 1] * pv; a2 += w[3 * e + 2] * pv;
-        }
-#endif
         ao[3 * tid] = a0; ao[3 * tid + 1] = a1; ao[3 * tid + 2] = a2;
     }
     __syncthreads();
@@ -1050,14 +424,8 @@ __global__ void __launch_bounds__(DBAT_PSB) k_backsub_obs(DevProblem P, double l
             double a[3] = {0.0, 0.0, 0.0};
 #pragma unroll
             for (int s = 0; s < DBAT_NSLOT; ++s) {
-#if BSO_V2
                 if (!pshOk[s]) continue;
                 const double pv = psh[s];
-#else
-                const int c = P.sh_col[s];
-                if (c < 0) continue;
-                const double pv = p[c];
-#endif
                 const double* ws = rec + DBAT_PT_WSH + 3 * s;
                 a[0] += ws[0] * pv; a[1] += ws[1] * pv; a[2] += ws[2] * pv;
             }
@@ -1154,14 +522,12 @@ __global__ void __launch_bounds__(1024) k_sum_pair(const double* __restrict__ a,
 void launch_backsub(const DevProblem& P, double lambda, const double* pc, const double* pEO, double* p, double* partial,
                     const double* camDiag, const double* camG, double* jpOut, cudaStream_t st,
                     cudaStream_t st2, cudaEvent_t evFork, cudaEvent_t evJoin) {
-    static const bool perPoint = getenv("DBAT_POINT_SIDE_PER_POINT") != nullptr;
     if (pc != p) cudaMemcpyAsync(p, pc, sizeof(double) * P.nC, cudaMemcpyDeviceToDevice, st);
     // number of per-block partial pairs the point kernels will write (the camera part's partials follow them)
     int nb = 0;
     const int nbBig = P.nPsbig > 0 ? (P.nPsbig + 127) / 128 : 0;
-    const bool general = P.nOP > 0 && P.ioGeneral, onePerPoint = P.nOP > 0 && !P.ioGeneral && (perPoint || !P.psb_pt);
+    const bool general = P.nOP > 0 && P.ioGeneral;
     if (general) nb = (P.nOP + 127) / 128;        // launch_backsub_gen: one warp-free block per 128 points
-    else if (onePerPoint) nb = (P.nOP + 127) / 128;
     else if (P.nOP > 0) nb = P.nPsb + nbBig;
     const int nbc = (P.nImg + 3) / 4;
     const bool side = jpOut && st2 && evFork && evJoin;
@@ -1175,9 +541,6 @@ void launch_backsub(const DevProblem& P, double lambda, const double* pc, const 
     }
     if (general) {
         launch_backsub_gen(P, lambda, p, jpOut ? partial : nullptr, st);
-    } else if (onePerPoint) {
-        k_backsub<<<nb, 128, 0, st>>>(P, lambda, p, jpOut ? partial : nullptr, nb, nullptr, 0);
-        count_launch();
     } else if (P.nOP > 0) {
         if (P.nPsb > 0) { k_backsub_obs<<<P.nPsb, DBAT_PSB, 0, st>>>(P, lambda, p, pEO, jpOut ? partial : nullptr, nb); count_launch(); }
         if (nbBig > 0) { k_backsub<<<nbBig, 128, 0, st>>>(P, lambda, p, jpOut ? partial + P.nPsb : nullptr, nb, P.psbig, P.nPsbig); count_launch(); }

@@ -19,8 +19,8 @@
 //                   hold the block in the order of a CSR index built at create, and subtracts the sum from the
 //                   tile of S.  Same for the shared-IO x EO rows (per image) and the shared x shared table.
 //
-// Compared with the grouped kernel this replaces (k_schur_group2: one FP64 `red` per non-zero entry and group,
-// 60 M atomic lanes at BASELINE config 4), S is touched once per entry, and the result is bit-reproducible.
+// S is touched once per entry, and the result is bit-reproducible.  Points with more than DBAT_GRP_MAXM rays are not
+// grouped: k_schur_atomic (schur.cu) adds them with FP64 atomics before these kernels run.
 #include <algorithm>
 #include <cstdio>
 #include <vector>
@@ -92,15 +92,11 @@ struct WinPrefetch { int4 h; double2 m; };
 // fragment loads: lanes (fr, fk) of a half warp read Zt[(k0 + fk) * LDR + row0 + fr], fk * LDR mod 16 = 0, 4, 8, 12 in some order)
 __host__ __device__ constexpr int win_ldr(int rowsZ) { return ((rowsZ - 4 + 7) / 8) * 8 + 4; }
 
-#ifndef WIN_ILP
-#define WIN_ILP 1                       // 0: one DMMA chain per tile (cross-check)
-#endif
 // one work unit: CNT column tiles against one row tile; k offsets are immediates (LDR is a template parameter)
 template <int LDR, int CNT>
 __device__ __forceinline__ void win_unit_mma(const double* __restrict__ pa, const double* __restrict__ pb0,
                                              const double* __restrict__ pb1, const double* __restrict__ pb2, int Kp,
                                              double (&c)[3][2]) {
-#if WIN_ILP
     // even and odd k-steps into separate accumulators: two dependent DMMA chains per tile instead of one
     double d[3][2] = {{0.0, 0.0}, {0.0, 0.0}, {0.0, 0.0}};
 #pragma unroll
@@ -119,16 +115,6 @@ __device__ __forceinline__ void win_unit_mma(const double* __restrict__ pa, cons
     }
 #pragma unroll
     for (int n = 0; n < CNT; ++n) { c[n][0] += d[n][0]; c[n][1] += d[n][1]; }
-#else
-#pragma unroll
-    for (int ks = 0; ks < (3 * WIN_GP + 3) / 4; ++ks) {
-        if (4 * ks >= Kp) break;
-        const double a = pa[4 * ks * LDR];
-        dmma_w(c[0][0], c[0][1], a, pb0[4 * ks * LDR]);
-        if (CNT > 1) dmma_w(c[1][0], c[1][1], a, pb1[4 * ks * LDR]);
-        if (CNT > 2) dmma_w(c[2][0], c[2][1], a, pb2[4 * ks * LDR]);
-    }
-#endif
 }
 
 // dynamic shared memory: Zt[3 * WIN_GP + 2][LDR] | Acc[WIN_ACC] | AccSh[16][WIN_SHLD] | AccSS[16][16]

@@ -125,12 +125,15 @@ def test_value_dependent_sparsity_camcal_start():
 @pytest.mark.parametrize('lam,jacobi', [(0.0, False), (1e3, False), (0.0, True)])
 def test_damped_step(case, lam, jacobi):
     """Schur + dense Cholesky step equals the reference's full sparse solve
-    p=(J'J+lambda*I)\\(-J'r) (levenberg_marquardt.m:119)."""
+    p=(J'J+lambda*I)\\(-J'r) (levenberg_marquardt.m:119), and a second step on the same handle is
+    bit-identical (the Schur reduction has no atomics for points with up to DBAT_GRP_MAXM rays)."""
     s, _ = scene(**CASES[case])
     x0 = serialize(s)
     W = buildweightmatrix(s)
     P = dbat_b200.Problem(copy.deepcopy(s))
     p, st = P.normal_step(x0, lam, jacobi)
+    p2, _ = P.normal_step(x0, lam, jacobi)
+    assert np.array_equal(p, p2), 'not bit-reproducible'
     ro, Jo = brown_euler_cam4(x0, s, True)
     Jw = Jo.multiply(np.sqrt(W)[:, None]).tocsc()
     rw = ro * np.sqrt(W)
@@ -587,43 +590,11 @@ def test_camcal_all_models_golden_sigma0(model, sigma0):
     assert E.numParams == (422 if abs(model) < 3 else 423)
 
 
-def test_deterministic_schur_mode_subprocess():
-    """DBAT_SCHUR=det selects the atomics-free pair-index Schur kernels: same step as the oracle,
-    and bit-identical from run to run."""
-    import subprocess
-    import sys
-    code = r'''
-import sys, copy, numpy as np
-sys.path.insert(0, %r); sys.path.insert(0, %r)
-import dbat_b200
-from test_gpu_parity import scene, CASES
-from oracle.cameramodel import brown_euler_cam4
-from oracle.dbatstruct import buildweightmatrix, serialize
-s, _ = scene(**CASES['priors+fixed'])
-x0 = serialize(s); W = buildweightmatrix(s)
-P = dbat_b200.Problem(copy.deepcopy(s))
-p1, st1 = P.normal_step(x0, 10.0, False)
-p2, st2 = P.normal_step(x0, 10.0, False)
-assert np.array_equal(p1, p2), 'not bit-reproducible'
-ro, Jo = brown_euler_cam4(x0, s, True)
-Jw = Jo.multiply(np.sqrt(W)[:, None]).tocsc(); rw = ro * np.sqrt(W)
-N = (Jw.T @ Jw).toarray()
-po = np.linalg.solve(N + 10.0 * np.eye(N.shape[0]), -(Jw.T @ rw))
-assert np.abs(p1 - po).max() / np.abs(po).max() < 5e-9
-print('DET-OK')
-''' % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, DBAT_SCHUR='det')
-    out = subprocess.run([sys.executable, '-c', code], env=env, capture_output=True, text=True, timeout=600)
-    assert 'DET-OK' in out.stdout, out.stdout + out.stderr
-
-
-@pytest.mark.parametrize('mode', ['maxm', 'perpoint', 'grouped'])
+@pytest.mark.parametrize('mode', ['maxm'])
 def test_schur_fallback_paths_subprocess(mode):
     """The window Schur kernel hands points with more than 20 rays to the per-point kernel.  No small
     scene has such points, so the threshold is lowered (DBAT_GRP_MAXM=6: the 10-ray points of the test
-    scene take the per-point kernel, the ragged 3-ray ones stay grouped); DBAT_SCHUR=perpoint runs the
-    per-point kernel for everything, DBAT_SCHUR=grouped the round-1 kernel with one atomic per entry and group.
-    Same step as the oracle in all of them."""
+    scene take the per-point kernel, the ragged 3-ray ones stay grouped).  Same step as the oracle."""
     import subprocess
     import sys
     code = r'''
@@ -645,7 +616,7 @@ for case in ('priors+fixed', 'ragged'):
     assert np.abs(p1 - po).max() / np.abs(po).max() < 5e-9, case
 print('FALLBACK-OK')
 ''' % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, DBAT_GRP_MAXM='6') if mode == 'maxm' else dict(os.environ, DBAT_SCHUR=mode)
+    env = dict(os.environ, DBAT_GRP_MAXM='6')
     out = subprocess.run([sys.executable, '-c', code], env=env, capture_output=True, text=True, timeout=600)
     assert 'FALLBACK-OK' in out.stdout, out.stdout + out.stderr
 
