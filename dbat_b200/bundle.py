@@ -172,10 +172,12 @@ class Problem:
         return self
 
     def reduced_info(self):
-        """Structure of the reduced camera system (tile counts, factorisation work, chain depth)."""
+        """Structure of the reduced camera system (tile counts, factorisation work, chain depth) and the point-side
+        paths the problem takes (points over 128 rays, points over 20 rays, largest group union and group size)."""
         v = np.zeros(16, dtype=np.int64)
         self._check(_lib.lib().dbat_reduced_info(self._h, _lib.iptr(v)))
-        names = ['nT', 'ld', 'nS', 'nSlots', 'nSlotsS', 'nTasks', 'nTerms', 'depth', 'order_mode', 'nSeg', 'gridFactor', 'gridBwd']
+        names = ['nT', 'ld', 'nS', 'nSlots', 'nSlotsS', 'nTasks', 'nTerms', 'depth', 'order_mode', 'nSeg', 'gridFactor', 'gridBwd',
+                 'nPsbig', 'nBig', 'grpMaxRays', 'grpMaxPts']
         d = {k: int(v[i]) for i, k in enumerate(names)}
         d['flops'] = 2.0 * 64 ** 3 * d['nTerms'] + 64.0 ** 3 * (d['nSlots'] - d['nT']) + d['nT'] * 64.0 ** 3 / 3
         return d

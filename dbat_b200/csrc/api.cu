@@ -81,6 +81,7 @@ struct dbat_handle {
     DevProblem P{};
     int NC = 0, m = 0, nIOrec = 0;
     int nPriorIO = 0, nPriorEO = 0, nPriorOP = 0;
+    int grpMaxPts = 0;                  // most points in one window Schur group (dbat_reduced_info)
     // host copies (CSC export, covariance layout)
     std::vector<int> h_img_cm, h_pt_cm, h_img_start, h_pt_start, h_pm2cm;
     std::vector<int> h_sh_col, h_eo_col, h_op_col, h_io_col;   // io_col: NC x nImg
@@ -596,6 +597,7 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
             }
             for (int r : uni) gimg.push_back(h->tc.sym.imgOrder[r]);
             gimg_off.push_back((int)gimg.size());
+            h->grpMaxPts = std::max(h->grpMaxPts, (int)end - gstart.back());
             gstart.push_back((int)end);
             P.grpMaxRays = std::max(P.grpMaxRays, (int)uni.size());
         };
@@ -775,7 +777,7 @@ extern "C" int dbat_reduced_info(const dbat_handle* h, int64_t* info) {
     if (h->group) h = group_first(h);
     const TileSym& s = h->tc.sym;
     const int64_t v[16] = {s.nT, s.ld, s.nS, s.nSlots, s.nSlotsS, s.nTasks, s.nTerms, s.depth, s.order_mode, s.nSeg,
-                           h->tc.gridFactor, h->tc.gridBwd, 0, 0, 0, 0};
+                           h->tc.gridFactor, h->tc.gridBwd, h->P.nPsbig, h->P.nBig, h->P.grpMaxRays, h->grpMaxPts};
     memcpy(info, v, sizeof(v));
     return DBAT_OK;
 }

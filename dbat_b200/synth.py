@@ -171,6 +171,71 @@ def make_scene(nImg=1000, nOP=200000, rays=10, seed=SEED, noise_px=0.5, start_no
     return s, truth
 
 
+def _look_at_angles(d, kappa):
+    """(omega, phi, kappa) of M = R1(omega) R2(phi) R3(kappa) whose camera looks along the unit vectors d (3,N):
+    the camera's z axis, the third column of M, is -d (kappa turns the frame about it freely)."""
+    return np.stack([np.arctan2(d[1], -d[2]), np.arcsin(np.clip(-d[0], -1, 1)), kappa])
+
+
+def make_convergent_scene(nImg, nOP, ray_counts, seed=SEED, noise_px=0.5, start_noise=1.0, build_indices=True):
+    """Seeded close-range convergent network around a 3-D object, with a caller-given ray count per point.
+
+    Same camera, noise and start-value recipe as make_scene.  The stations sit on three rings around the x axis
+    at elevations -15, 10 and 35 degrees (phi = the elevation, far from the gimbal lock of the omega-phi-kappa
+    angles), 19-21 m from the centre, all looking at it with a random roll so that the principal point and the
+    distortion stay well determined.  The object points fill a cylinder of radius 4 m and length 6 m about the
+    same axis: every station sees all of it inside the 6000 x 4000 frame.  Point j is observed by the
+    ray_counts[j] stations nearest to it in azimuth, so points close to each other have overlapping, contiguous
+    image lists (which lets them share window Schur groups).  Datum: `seteoest(s,'depend',1)`.
+    """
+    ray_counts = np.asarray(ray_counts, dtype=np.int64)
+    if ray_counts.shape != (nOP,) or ray_counts.min() < 1 or ray_counts.max() > nImg:
+        raise ValueError('ray_counts must hold nOP counts in [1, nImg]')
+    rng = np.random.default_rng(seed)
+    nRing = 3
+    ring = np.arange(nImg) % nRing
+    elev = np.deg2rad(np.array([-15.0, 10.0, 35.0]))[ring]
+    per = np.bincount(ring, minlength=nRing)
+    az = np.empty(nImg)
+    for r in range(nRing):                             # evenly spaced per ring, rings offset, jittered
+        k = np.flatnonzero(ring == r)
+        az[k] = 2 * np.pi * (np.arange(len(k)) + r / nRing + rng.uniform(-0.2, 0.2, len(k))) / per[r]
+    az = np.mod(az, 2 * np.pi)
+    D = rng.uniform(19.0, 21.0, nImg)
+    q0 = D * np.stack([np.sin(elev), np.cos(elev) * np.cos(az), np.cos(elev) * np.sin(az)])
+    EO = np.empty((6, nImg))
+    EO[0:3] = q0
+    EO[3:6] = _look_at_angles(-q0 / D, rng.uniform(-np.pi, np.pi, nImg))
+    M = _rot(EO[3:6])
+    paz = rng.uniform(0, 2 * np.pi, nOP)
+    rho = np.sqrt(rng.uniform(0.0, 16.0, nOP))
+    OP = np.stack([rng.uniform(-3.0, 3.0, nOP), rho * np.cos(paz), rho * np.sin(paz)])
+    # the ray_counts[j] stations nearest in azimuth (circular distance; ties by station index)
+    dist = np.abs(np.angle(np.exp(1j * (paz[:, None] - az[None, :]))))
+    near = np.argsort(dist, axis=1, kind='stable')
+    take = np.arange(nImg)[None, :] < ray_counts[:, None]
+    ip_op = np.nonzero(take)[0]
+    ip_img = near[take]
+    l, depth = _ideal(OP.T[ip_op], EO[0:3, ip_img].T, M[ip_img], IO_TRUE[0])
+    inside = (depth < 0) & (l[:, 0] > -11.9) & (l[:, 0] < 11.8) & (l[:, 1] > -7.9) & (l[:, 1] < 7.8)
+    assert inside.all(), 'a station does not see the whole object volume'
+    uv = _pixel_from_ideal(l, IO_TRUE) + rng.normal(0, noise_px, (len(ip_op), 2))
+    EO0 = EO.copy()
+    EO0[0:3] += start_noise * rng.normal(0, 0.05, (3, nImg))
+    EO0[3:6] += start_noise * rng.normal(0, np.deg2rad(0.1), (3, nImg))
+    OP0 = OP + start_noise * rng.normal(0, 0.1, OP.shape)
+    s = new_struct(np.tile(IO_START[:, None], (1, nImg)), EO0, OP0, uv.T, ip_img, ip_op,
+                   np.array([[PX], [PX]]), np.array([[IM_W], [IM_H]]), 3, 3, 2, noise_px)
+    s.bundle.est.IO[:] = True
+    s.bundle.est.IO[4, :] = False                      # setcamest(s,'all','not','sk')
+    s.bundle.est.OP[:] = True
+    seteoest_depend(s, 0)
+    if build_indices:
+        buildserialindices(s)
+    truth = dict(IO=IO_TRUE.copy(), EO=EO, OP=OP)
+    return s, truth
+
+
 def make_scene_shard(nImg, nOP_total, rank, world, rays=10, seed=SEED, noise_px=0.5, start_noise=1.0):
     """One rank's share of a synthetic block for a point-sharded multi-GPU run: the stations (and their start
     values) are generated identically on every rank from `seed`; this rank's nOP_total/world object points, their

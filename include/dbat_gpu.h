@@ -186,7 +186,13 @@ int dbat_camera_order(int64_t nImg, int64_t nOP, int64_t nObs, const int64_t *ob
 
 /* Structure of the reduced camera system of a problem: info (16) = {nT (64 x 64 tile rows), ld, nS (camera-side
  * unknowns), nSlots (stored tiles incl. fill), nSlotsS (tiles of S itself), nTasks, nTerms (tile products per
- * factorisation), depth (longest dependency chain in tile columns), order mode, segments, ...}. */
+ * factorisation), depth (longest dependency chain in tile columns), order mode, segments, grid of the factorisation,
+ * grid of the backward solve, then which point-side paths the problem takes:
+ *   [12] points with more than 128 observations (one-thread-per-point assembly and back-substitution, or one block
+ *        per point in several passes with general IO),
+ *   [13] estimated points with more than 20 observations (per-point Schur kernel with FP64 atomics),
+ *   [14] largest union of image lists of one window Schur group (above 12 the wider window instantiation runs),
+ *   [15] most points in one window Schur group}. */
 int dbat_reduced_info(const dbat_handle *h, int64_t *info);
 
 /* Symbolic analysis of the reduced camera system on its own (host only; tests and tools): elimination order

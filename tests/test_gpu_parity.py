@@ -81,7 +81,7 @@ CASES = {
     'model1': dict(model=1),
     'model-1': dict(model=-1),
     'priors+fixed': dict(model=3, priors=True, fixed_pts=4),
-    'ragged': dict(model=3, rays=3, nOP=150, seed=11),
+    'rays3': dict(model=3, rays=3, nOP=150, seed=11),
 }
 
 
@@ -121,7 +121,7 @@ def test_value_dependent_sparsity_camcal_start():
     P.close()
 
 
-@pytest.mark.parametrize('case', ['model3', 'priors+fixed', 'model5', 'ragged'])
+@pytest.mark.parametrize('case', ['model3', 'priors+fixed', 'model5', 'rays3'])
 @pytest.mark.parametrize('lam,jacobi', [(0.0, False), (1e3, False), (0.0, True)])
 def test_damped_step(case, lam, jacobi):
     """Schur + dense Cholesky step equals the reference's full sparse solve
@@ -152,7 +152,7 @@ def _decisions(rr):
     return [bool(rr[i + 1] != rr[i]) for i in range(len(rr) - 1)]
 
 
-@pytest.mark.parametrize('case', ['model3', 'model4', 'model1', 'model-1', 'priors+fixed', 'ragged'])
+@pytest.mark.parametrize('case', ['model3', 'model4', 'model1', 'model-1', 'priors+fixed', 'rays3'])
 @pytest.mark.parametrize('damping', ['gna', 'lmp', 'lm'])
 def test_optimisers(case, damping):
     s, _ = scene(**CASES[case])
@@ -592,9 +592,10 @@ def test_camcal_all_models_golden_sigma0(model, sigma0):
 
 @pytest.mark.parametrize('mode', ['maxm'])
 def test_schur_fallback_paths_subprocess(mode):
-    """The window Schur kernel hands points with more than 20 rays to the per-point kernel.  No small
-    scene has such points, so the threshold is lowered (DBAT_GRP_MAXM=6: the 10-ray points of the test
-    scene take the per-point kernel, the ragged 3-ray ones stay grouped).  Same step as the oracle."""
+    """The window Schur kernel hands points with more than 20 rays to the per-point kernel.  The threshold is
+    lowered here (DBAT_GRP_MAXM=6): every point of priors+fixed has 10 rays and takes the per-point kernel, every
+    point of rays3 has 3 rays and stays grouped.  Same step as the oracle.  test_ray_spread.py runs the
+    per-point kernel at the production threshold, beside groups of 14 points."""
     import subprocess
     import sys
     code = r'''
@@ -604,7 +605,7 @@ import dbat_b200
 from test_gpu_parity import scene, CASES
 from oracle.cameramodel import brown_euler_cam4
 from oracle.dbatstruct import buildweightmatrix, serialize
-for case in ('priors+fixed', 'ragged'):
+for case in ('priors+fixed', 'rays3'):
     s, _ = scene(**CASES[case])
     x0 = serialize(s); W = buildweightmatrix(s)
     P = dbat_b200.Problem(copy.deepcopy(s))
@@ -734,10 +735,10 @@ def test_forwintersect_matches_oracle_camcal():
     assert np.array_equal(sg.OP.val[:, ~est], s.OP.val[:, ~est])       # control points untouched
 
 
-@pytest.mark.parametrize('case', ['model3', 'ragged'])
+@pytest.mark.parametrize('case', ['model3', 'rays3'])
 def test_forwintersect_matches_oracle_synthetic(case):
-    """Same on seeded synthetic blocks (ragged: points with different ray counts, incl. an explicit id list
-    and a point left with a single ray -> NaN)."""
+    """Same on seeded synthetic blocks, with an explicit id list and a point left with a single ray -> NaN
+    (rays3: every other point has 3 rays)."""
     from oracle.photogrammetry import forwintersect as ofwi
     s, truth = scene(**CASES[case])
     s.IO.val[5:10, :] = truth['IO'][5:10, None]                 # non-trivial lens correction
@@ -810,7 +811,7 @@ def test_resect_reports_failure_with_two_control_points():
     assert fail and np.isnan(sg.EO.val[:, [0, 1]]).all() and np.isinf(rms).all()
 
 
-@pytest.mark.parametrize('case', ['model3', 'priors+fixed', 'ragged'])
+@pytest.mark.parametrize('case', ['model3', 'priors+fixed', 'rays3'])
 def test_gauss_markov_direct_call(case):
     """gauss_markov.m called directly (numeric convTol; via bundle() the reference passes a function
     handle and fails): same iterates, iteration count and residual norms as the restatement."""
