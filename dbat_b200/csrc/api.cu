@@ -22,6 +22,7 @@
 #include "../../include/dbat_gpu.h"
 #include "kernels.cuh"
 #include "launch.h"
+#include "plan.h"
 #include "tilechol.h"
 
 int64_t g_dbat_launches = 0;
@@ -79,17 +80,7 @@ struct dbat_handle {
     cudaStream_t st = nullptr, st2 = nullptr;
     cudaEvent_t evFork = nullptr, evJoin = nullptr, evStep = nullptr;
     DevProblem P{};
-    int NC = 0, m = 0, nIOrec = 0;
-    int nPriorIO = 0, nPriorEO = 0, nPriorOP = 0;
-    int grpMaxPts = 0;                  // most points in one window Schur group (dbat_reduced_info)
-    // host copies (CSC export, covariance layout)
-    std::vector<int> h_img_cm, h_pt_cm, h_img_start, h_pt_start, h_pm2cm;
-    std::vector<int> h_sh_col, h_eo_col, h_op_col, h_io_col;   // io_col: NC x nImg
-    std::vector<int> h_io_colx;         // nImg x NSLOT: x column of every (image, IO slot)
-    std::vector<int> h_glob_x;          // IO columns used by more than one image (all of them with one shared block)
-    std::vector<int> h_colLocalImg;     // per camera-side x column: the one image that uses this IO column, or -1
-    std::vector<int> h_prior_col;
-    std::vector<double> h_prior_isig;
+    ProblemPlan plan;                   // host-side index of the problem (plan.cu)
     // device allocations
     std::vector<void*> allocs;
     int *d_IOsrc = nullptr, *d_IOdst = nullptr, *d_EOsrc = nullptr, *d_EOdst = nullptr, *d_OPsrc = nullptr, *d_OPdst = nullptr;
@@ -107,10 +98,8 @@ struct dbat_handle {
     double *d_evalRed = nullptr, *d_prr = nullptr; size_t nEvalRed = 0;
     double *d_r = nullptr;              // m doubles (export)
     TChol tc;                           // sparse tile Cholesky of the reduced system (tilechol.cu)
-    std::vector<int> h_x2s;             // x column (camera side) -> S index
     double* d_dS = nullptr;             // Jacobi scale per S index
     unsigned long long* d_stats = nullptr;   // pivot statistics exchanged between the ranks
-    std::vector<double> h_xyz; std::vector<int> h_nEO; int h_nIOest = 0; std::vector<int64_t> h_adjPtr; std::vector<int32_t> h_adj;   // for re-tiling in dbat_comm_init
     const double* jp_vec = nullptr;     // vector whose |Jp|^2, r'Jp came out of the last back-substitution (nullptr: none)
     double jp_cache[2] = {0, 0};
     bool params_valid = false;          // parameter arrays correspond to d_x
@@ -137,12 +126,14 @@ static int dev_alloc(dbat_handle* h, T** p, size_t count) {
     h->allocs.push_back(*p);
     return 0;
 }
-template <typename T>
-static int dev_upload(dbat_handle* h, T** p, const std::vector<T>& v) {
-    int rc = dev_alloc(h, p, v.size());
+template <typename T, typename U>        // U: T or const T
+static int dev_upload(dbat_handle* h, U** p, const std::vector<T>& v) {
+    T* q = nullptr;
+    int rc = dev_alloc(h, &q, v.size());
+    *p = q;
     if (rc) return rc;
     if (!v.empty()) {
-        cudaError_t e = cudaMemcpy(*p, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice);
+        cudaError_t e = cudaMemcpy(q, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice);
         if (e != cudaSuccess) { h->err = std::string("cudaMemcpy: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
     }
     return 0;
@@ -194,53 +185,39 @@ static void free_desc(DescCopy* c);
 static void group_destroy(dbat_handle* h);
 static thread_local bool g_in_group_create = false;
 
-// (Re)build everything that depends on the tiling of the reduced system: symbolic analysis for nParts parts, the S
-// index maps, the tile storage and the S-ordered work vectors.  dbat_create calls it for one part; dbat_comm_init
-// again when the factorisation is distributed over the ranks.
-static int setup_reduced(dbat_handle* h, int nParts, int myPart) {
-    DevProblem& P = h->P;
-    const int nImg = P.nImg, nC = P.nC;
-    TileSym sym;
-    if (tile_symbolic(nImg, h->h_adjPtr.data(), h->h_adj.data(), h->h_nEO.data(), h->h_nIOest, -1, 120, sym, nParts, myPart,
-                      h->h_xyz.size() == 3 * (size_t)nImg ? h->h_xyz.data() : nullptr)) {
+// Symbolic analysis of the reduced system for nParts parts (tilesym.cu).  dbat_create analyses it for one part;
+// dbat_comm_init again when the factorisation is distributed over the ranks.
+static int analyse_reduced(dbat_handle* h, int nParts, int myPart, TileSym& sym) {
+    const ProblemPlan& pl = h->plan;
+    if (tile_symbolic(pl.nImg, pl.adjPtr.data(), pl.adj.data(), pl.nEO.data(), (int)pl.glob_x.size(), -1, 120, sym, nParts,
+                      myPart, pl.xyz.data())) {
         h->err = "symbolic analysis of the reduced system failed"; return DBAT_E_STATE;
     }
-    std::vector<int> sh_s(DBAT_NSLOT, -1), eo_s((size_t)6 * nImg, -1), s2x(sym.ld, -1);
-    std::vector<int> cam_colx((size_t)DBAT_NCAM * nImg, -1), cam_s((size_t)DBAT_NCAM * nImg, -1);
-    h->h_x2s.assign(std::max(1, nC), -1);
-    for (size_t k = 0; k < h->h_glob_x.size(); ++k) h->h_x2s[h->h_glob_x[k]] = sym.ioS + (int)k;     // global IO columns, x order
-    for (int i = 0; i < nImg; ++i) {
-        int q = 0;
-        for (int a = 0; a < 6; ++a) {
-            const int c = h->h_eo_col[(size_t)i * 6 + a];
-            if (c >= 0) { eo_s[(size_t)i * 6 + a] = sym.imgS[i] + q; h->h_x2s[c] = sym.imgS[i] + q; ++q; }
-        }
-        for (int sl = 0; sl < DBAT_NSLOT; ++sl) {             // this image's own IO columns follow its EO elements
-            const int c = h->h_io_colx[(size_t)i * DBAT_NSLOT + sl];
-            if (c >= 0 && h->h_colLocalImg[c] == i && h->h_x2s[c] < 0) { h->h_x2s[c] = sym.imgS[i] + q; ++q; }
-        }
-    }
-    for (int c = 0; c < nC; ++c) if (h->h_x2s[c] >= 0) s2x[h->h_x2s[c]] = c;
-    for (int sl = 0; sl < DBAT_NSLOT; ++sl) if (h->h_sh_col[sl] >= 0) sh_s[sl] = h->h_x2s[h->h_sh_col[sl]];
-    for (int i = 0; i < nImg; ++i)
-        for (int a = 0; a < DBAT_NCAM; ++a) {
-            const int c = a < DBAT_NSLOT ? h->h_io_colx[(size_t)i * DBAT_NSLOT + a] : h->h_eo_col[(size_t)i * 6 + a - DBAT_NSLOT];
-            cam_colx[(size_t)i * DBAT_NCAM + a] = c;
-            cam_s[(size_t)i * DBAT_NCAM + a] = c >= 0 ? h->h_x2s[c] : -1;
-        }
+    return 0;
+}
+
+// (Re)build everything that depends on the tiling of the reduced system: the S index maps, the tile storage and the
+// S-ordered work vectors.
+static int setup_reduced(dbat_handle* h, const TileSym& sym) {
+    DevProblem& P = h->P;
+    const ReducedMaps mp = plan_reduced_maps(h->plan, sym);
     if (h->tc.d.tiles) tchol_free(h->tc);
     if (tchol_alloc(h->tc, sym)) { h->err = "out of memory for the reduced system"; return DBAT_E_OOM; }
     int rc = 0;
-    int *d_shs = nullptr, *d_eos = nullptr, *d_s2x = nullptr, *d_ccx = nullptr, *d_cs = nullptr, *d_gx = nullptr;
-    if ((rc = dev_upload(h, &d_shs, sh_s)) || (rc = dev_upload(h, &d_eos, eo_s)) || (rc = dev_upload(h, &d_s2x, s2x)) ||
-        (rc = dev_upload(h, &d_ccx, cam_colx)) || (rc = dev_upload(h, &d_cs, cam_s)) || (rc = dev_upload(h, &d_gx, h->h_glob_x))) return rc;
-    P.sh_s = d_shs; P.eo_s = d_eos; P.s2x = d_s2x; P.T = h->tc.d;
-    P.cam_colx = d_ccx; P.cam_s = d_cs; P.glob_x = d_gx; P.nGlob = (int)h->h_glob_x.size();
-    P.ldS = sym.ld;
+    if ((rc = dev_upload(h, &P.sh_s, mp.sh_s)) || (rc = dev_upload(h, &P.eo_s, mp.eo_s)) || (rc = dev_upload(h, &P.s2x, mp.s2x)) ||
+        (rc = dev_upload(h, &P.cam_colx, mp.cam_colx)) || (rc = dev_upload(h, &P.cam_s, mp.cam_s)) ||
+        (rc = dev_upload(h, &P.glob_x, h->plan.glob_x))) return rc;
+    P.T = h->tc.d; P.nGlob = (int)h->plan.glob_x.size(); P.ldS = sym.ld;
     if ((rc = dev_alloc(h, &h->d_dS, (size_t)sym.ld)) || (rc = dev_alloc(h, &P.rhs, (size_t)sym.ld)) ||
         (rc = dev_alloc(h, &h->d_pc, (size_t)sym.ld))) return rc;
     if (!h->d_stats && (rc = dev_alloc(h, &h->d_stats, (size_t)4))) return rc;
     return 0;
+}
+
+static std::vector<int> zero_based(const int64_t* p, int64_t cnt) {
+    std::vector<int> v(cnt);
+    for (int64_t k = 0; k < cnt; ++k) v[k] = (int)(p[k] - 1);
+    return v;
 }
 
 extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
@@ -250,263 +227,64 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail_create(nullptr, DBAT_E_CUDA, "no CUDA device available (libdbatgpu has no CPU fallback)");
     dbat_handle* h = new dbat_handle();
-    const int nImg = (int)d->nImg, nOP = (int)d->nOP, nObs = (int)d->nIP;
-    const int nK = d->nK, nP = d->nP, NC = 5 + nK + nP;
-    const bool legacy = (d->distModel == 1 || d->distModel == -1);
-    if (!legacy && (d->distModel < 2 || d->distModel > 5))
-        return fail_create(h, DBAT_E_BADARG, "distModel must be -1, 1, 2, 3, 4 or 5");
-    if (nK > DBAT_KMAX || nP > DBAT_PMAX || nK < 0 || nP < 0 || nP == 1)
-        return fail_create(h, DBAT_E_UNSUPPORTED, "nK/nP outside the compiled limits");
-    if (d->n <= 0 || nImg <= 0) return fail_create(h, DBAT_E_BADARG, "empty problem");
-    h->NC = NC;
-    DevProblem& P = h->P;
-    P.nImg = nImg; P.nOP = nOP; P.nObs = nObs; P.nK = nK; P.nP = nP; // kernel MODEL: 0..3 = res_euler_brown_0..3 (distModel 2..5); legacy 1 == model 2 arithmetic; -1 = forward Brown
-    P.model = legacy ? (d->distModel == 1 ? 0 : 4) : d->distModel - 2;
-    P.n = (int)d->n;
+    PlanOpts opts{DBAT_GRP_MAXM, getenv("DBAT_EVAL_GENERIC") != nullptr};
+    // DBAT_GRP_MAXM=k lowers the threshold (tests of the per-point path)
+    if (const char* e = getenv("DBAT_GRP_MAXM")) opts.grpMaxM = std::max(1, std::min(DBAT_GRP_MAXM, atoi(e)));
 
-    // ---- column maps from the deserialisation indices (multi_res.m:58-63)
-    std::vector<int> colIO((size_t)NC * nImg, -1), colEO((size_t)6 * nImg, -1), colOP((size_t)3 * nOP, -1);
-    auto fill = [&](std::vector<int>& col, const int64_t* src, const int64_t* dst, int64_t cnt) -> bool {
-        for (int64_t k = 0; k < cnt; ++k) {
-            const int64_t dd = dst[k] - 1, ss = src[k] - 1;
-            if (dd < 0 || dd >= (int64_t)col.size() || ss < 0 || ss >= d->n) return false;
-            col[dd] = (int)ss;
-        }
-        return true;
-    };
-    if (!fill(colIO, d->IOdes_src, d->IOdes_dest, d->nIOdes) || !fill(colEO, d->EOdes_src, d->EOdes_dest, d->nEOdes) ||
-        !fill(colOP, d->OPdes_src, d->OPdes_dest, d->nOPdes))
-        return fail_create(h, DBAT_E_BADARG, "deserialisation index out of range");
-    // camera-side unknowns x[0:nC]: everything up to the last IO/EO column (a point-sharded problem
-    // lists only its own OP columns, so n - nOPdes would be wrong there)
-    int nC = 0;
-    for (int c : colIO) nC = std::max(nC, c + 1);
-    for (int c : colEO) nC = std::max(nC, c + 1);
-    for (int c : colOP) if (c >= 0 && c < nC) return fail_create(h, DBAT_E_UNSUPPORTED, "x must be ordered [IO;EO;OP]");
-    for (int c : colIO) if (c >= nC) return fail_create(h, DBAT_E_UNSUPPORTED, "x must be ordered [IO;EO;OP]");
-    for (int c : colEO) if (c >= nC) return fail_create(h, DBAT_E_UNSUPPORTED, "x must be ordered [IO;EO;OP]");
-    P.nC = nC;
-
-    // ---- observations: 0-based, verify (image, OP) ordering
-    h->h_img_cm.resize(nObs); h->h_pt_cm.resize(nObs);
-    std::vector<char> imgHasObs(nImg, 0);
-    for (int k = 0; k < nObs; ++k) {
-        const int64_t i = d->IPimg[k] - 1, j = d->IPop[k] - 1;
-        if (i < 0 || i >= nImg || j < 0 || j >= nOP) return fail_create(h, DBAT_E_BADARG, "IPimg/IPop out of range");
-        if (k > 0 && (i < h->h_img_cm[k - 1] || (i == h->h_img_cm[k - 1] && j <= h->h_pt_cm[k - 1])))
-            return fail_create(h, DBAT_E_BADARG, "image points must be sorted by (image, OP) without duplicates");
-        h->h_img_cm[k] = (int)i; h->h_pt_cm[k] = (int)j; imgHasObs[i] = 1;
-    }
-    // ---- structure checks: one shared IO block; every EO column owned by one image
-    h->h_sh_col.assign(DBAT_NSLOT, -1);
-    auto slot_of = [&](int row) { return row < 5 ? row : (row < 5 + nK ? DBAT_SLOT_K + (row - 5) : DBAT_SLOT_P + (row - 5 - nK)); };
-    int firstImg = -1;
-    for (int i = 0; i < nImg; ++i) if (imgHasObs[i]) { firstImg = i; break; }
-    if (legacy) {
-        // brown_euler_cam4.m:39-41,186-188: est.IO(:,2:end)=false, EO.cam(:)=1, IP.cam(:)=1
-        for (int i = 1; i < nImg; ++i)
-            for (int r = 0; r < NC; ++r) colIO[(size_t)i * NC + r] = colIO[r];
-        colIO[3] = -1; colIO[4] = -1;          // aspect / skew do not exist in the legacy models
-        for (int i = 1; i < nImg; ++i) { colIO[(size_t)i * NC + 3] = -1; colIO[(size_t)i * NC + 4] = -1; }
-    }
-    // IO column of every (image, slot); one block shared by all images -> fast path, anything else (image-variant
-    // parameters, several cameras: IO.struct.block, multi_res.m:92-111) -> general path
-    h->h_io_colx.assign((size_t)nImg * DBAT_NSLOT, -1);
-    for (int i = 0; i < nImg; ++i)
-        for (int r = 0; r < NC; ++r) h->h_io_colx[(size_t)i * DBAT_NSLOT + slot_of(r)] = colIO[(size_t)i * NC + r];
-    bool general = false;
-    for (int r = 0; r < NC; ++r) {
-        int v = firstImg >= 0 ? colIO[(size_t)firstImg * NC + r] : -1;
-        for (int i = 0; i < nImg; ++i)
-            if (imgHasObs[i] && colIO[(size_t)i * NC + r] != v) general = true;
-        h->h_sh_col[slot_of(r)] = v;
-    }
-    if (general && legacy) return fail_create(h, DBAT_E_UNSUPPORTED, "the legacy models take one camera");
-    if (general) h->h_sh_col.assign(DBAT_NSLOT, -1);      // no column is "the" shared column of a slot
-    P.ioGeneral = general ? 1 : 0;
-    {
-        std::vector<int> owner(nC, -1);
-        for (int i = 0; i < nImg; ++i)
-            for (int a = 0; a < 6; ++a) {
-                const int c = colEO[(size_t)i * 6 + a];
-                if (c < 0) continue;
-                if (owner[c] >= 0 && owner[c] != i) return fail_create(h, DBAT_E_UNSUPPORTED, "shared EO blocks are not built yet");
-                owner[c] = i;
-            }
-        int prev = -1;   // EO columns must ascend with (image, element): serialisation order
-        for (int i = 0; i < nImg; ++i)
-            for (int a = 0; a < 6; ++a) {
-                const int c = colEO[(size_t)i * 6 + a];
-                if (c < 0) continue;
-                if (c <= prev) return fail_create(h, DBAT_E_UNSUPPORTED, "EO columns must be in serialisation order");
-                prev = c;
-            }
-        if (prev >= 0) {
-            int minEO = nC;
-            for (int c : colEO) if (c >= 0) minEO = std::min(minEO, c);
-            for (int c : h->h_io_colx) if (c > minEO) return fail_create(h, DBAT_E_UNSUPPORTED, "IO columns must precede EO columns in x");
-        }
-    }
-    h->h_io_col = colIO; h->h_eo_col = colEO; h->h_op_col = colOP;
-
-    // ---- unique IO records (by value of the whole IO column + pixel size)
-    std::vector<int> ioOfImg(nImg, 0), rep;
-    {
-        std::map<std::vector<double>, int> seen;
-        for (int i = 0; i < nImg; ++i) {
-            const int src = legacy ? 0 : i;
-            std::vector<double> key(d->IOval + (size_t)src * NC, d->IOval + (size_t)(src + 1) * NC);
-            if (general) key.push_back((double)i);          // estimated per-image parameters diverge: one record per image
-            auto it = seen.find(key);
-            if (it == seen.end()) { it = seen.emplace(key, (int)rep.size()).first; rep.push_back(i); }
-            ioOfImg[i] = it->second;
-        }
-    }
-    h->nIOrec = (int)rep.size();
-
-    // ---- weights, orderings, chunks
-    std::vector<double2> uv_cm(nObs), isig_cm(nObs), uv_pm(nObs), isig_pm(nObs);
-    for (int k = 0; k < nObs; ++k) {
-        const int i = h->h_img_cm[k];
-        uv_cm[k] = make_double2(d->IPval[2 * (size_t)k], d->IPval[2 * (size_t)k + 1]);
-        const int ic = legacy ? 0 : i;
-        const double sx = d->IPstd[2 * (size_t)k] * d->pxSize[2 * (size_t)ic];
-        const double sy = d->IPstd[2 * (size_t)k + 1] * d->pxSize[2 * (size_t)ic + 1];
-        isig_cm[k] = make_double2(1.0 / sx, 1.0 / sy);           // buildweightmatrix.m:13-23, R = chol(W)
-    }
-    h->h_img_start.assign(nImg + 1, 0);
-    for (int k = 0; k < nObs; ++k) h->h_img_start[h->h_img_cm[k] + 1]++;
-    for (int i = 0; i < nImg; ++i) h->h_img_start[i + 1] += h->h_img_start[i];
-    h->h_pt_start.assign(nOP + 1, 0);
-    for (int k = 0; k < nObs; ++k) h->h_pt_start[h->h_pt_cm[k] + 1]++;
-    for (int j = 0; j < nOP; ++j) h->h_pt_start[j + 1] += h->h_pt_start[j];
-    h->h_pm2cm.resize(nObs);
-    std::vector<int> img_pm(nObs);
-    {
-        std::vector<int> fillp(h->h_pt_start.begin(), h->h_pt_start.end() - 1);
-        for (int k = 0; k < nObs; ++k) {                       // stable: images ascend inside a point
-            const int o = fillp[h->h_pt_cm[k]]++;
-            h->h_pm2cm[o] = k; img_pm[o] = h->h_img_cm[k]; uv_pm[o] = uv_cm[k]; isig_pm[o] = isig_cm[k];
-        }
-    }
-    std::vector<Chunk> chunks;
-    std::vector<int> img_chunk_start(nImg + 1, 0);
-    for (int i = 0; i < nImg; ++i) {
-        img_chunk_start[i] = (int)chunks.size();
-        for (int s = h->h_img_start[i]; s < h->h_img_start[i + 1]; s += DBAT_CHUNK)
-            chunks.push_back({i, s, std::min(DBAT_CHUNK, h->h_img_start[i + 1] - s), 0});
-    }
-    img_chunk_start[nImg] = (int)chunks.size();
-    P.nChunks = (int)chunks.size();
-
-    // ---- prior observations
-    const int nPrior = (int)(d->nPriorIO + d->nPriorEO + d->nPriorOP);
-    h->nPriorIO = (int)d->nPriorIO; h->nPriorEO = (int)d->nPriorEO; h->nPriorOP = (int)d->nPriorOP;
-    P.nPrior = nPrior;
-    h->h_prior_col.resize(nPrior); h->h_prior_isig.resize(nPrior);
-    std::vector<double> prior_val(nPrior);
-    for (int k = 0; k < nPrior; ++k) {
-        const int64_t c = d->prior_x[k] - 1;
-        if (c < 0 || c >= d->n) return fail_create(h, DBAT_E_BADARG, "prior_x out of range");
-        if (!(d->prior_std[k] > 0)) return fail_create(h, DBAT_E_BADARG, "prior std must be positive");
-        h->h_prior_col[k] = (int)c; prior_val[k] = d->prior_val[k]; h->h_prior_isig[k] = 1.0 / d->prior_std[k];
-    }
-    h->m = 2 * nObs + nPrior;
-    std::vector<int> col2pt(std::max(1, P.n - nC), -1);
-    for (int e = 0; e < 3 * nOP; ++e) if (colOP[e] >= 0) col2pt[colOP[e] - nC] = e;
+    // ---- host side: the plan (plan.cu) and the symbolic analysis of the reduced system
+    ProblemPlan& pl = h->plan;
+    PlanUpload up;
+    TileSym sym;
+    std::string msg;
+    int rc = plan_columns(d, pl, msg);
+    if (!rc) { plan_observations(d, pl, up); rc = plan_priors(d, pl, up, msg); }
+    if (!rc) rc = plan_cameras(d, pl, up, msg);
+    if (rc) return fail_create(h, rc, msg);
+    if ((rc = analyse_reduced(h, 1, 0, sym))) return fail_create(h, rc, h->err);
+    plan_point_blocks(pl, up);
+    plan_schur_windows(pl, up, sym, opts);
 
     // ---- device side
+    DevProblem& P = h->P;
+    // kernel MODEL: 0..3 = res_euler_brown_0..3 (distModel 2..5); legacy 1 == model 2 arithmetic; -1 = forward Brown
+    P.nImg = pl.nImg; P.nOP = pl.nOP; P.nObs = pl.nObs; P.nK = d->nK; P.nP = d->nP;
+    P.model = pl.legacy ? (d->distModel == 1 ? 0 : 4) : d->distModel - 2;
+    P.n = pl.n; P.nC = pl.nC; P.nChunks = (int)up.chunks.size(); P.nPrior = (int)pl.prior_col.size();
+    P.ioGeneral = pl.general ? 1 : 0;
+    P.evalCompact = plan_eval_compact(pl, d->nK, d->nP, opts) ? 1 : 0;
+    P.nPsb = up.nPsb; P.nPsbig = up.nPsbig;
+    P.nCand = up.nCand; P.nBig = up.nBig; P.grpMaxRays = up.grpMaxRays; P.nClu = up.nClu; P.nRedBlk = up.nRedBlk;
     if (cudaStreamCreate(&h->st) != cudaSuccess || cudaStreamCreateWithFlags(&h->st2, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->evFork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->evJoin, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->evStep, cudaEventDisableTiming) != cudaSuccess)
         return fail_create(h, DBAT_E_CUDA, "cudaStreamCreate failed");
-    int rc = 0;
-#define UP(ptr, vec) if ((rc = dev_upload(h, &ptr, vec))) return fail_create(h, rc, h->err)
+#define UP(ptr, vec) if ((rc = dev_upload(h, &ptr, vec)) != 0) return fail_create(h, rc, h->err)
 #define AL(ptr, cnt) if ((rc = dev_alloc(h, &ptr, (size_t)(cnt)))) return fail_create(h, rc, h->err)
-    double2 *d_uv_cm, *d_isig_cm, *d_uv_pm, *d_isig_pm; int *d_pt_cm, *d_img_cm, *d_img_pm, *d_pm2cm, *d_pt_start;
-    Chunk* d_chunks; int *d_sh, *d_eo, *d_op, *d_pc; double *d_pv, *d_pi;
-    UP(d_uv_cm, uv_cm); UP(d_isig_cm, isig_cm); UP(d_uv_pm, uv_pm); UP(d_isig_pm, isig_pm);
-    UP(d_pt_cm, h->h_pt_cm); UP(d_img_cm, h->h_img_cm); UP(d_img_pm, img_pm); UP(d_pm2cm, h->h_pm2cm);
-    UP(d_pt_start, h->h_pt_start); UP(d_chunks, chunks);
-    UP(d_sh, h->h_sh_col); UP(d_eo, colEO); UP(d_op, colOP);
-    UP(d_pc, h->h_prior_col); UP(d_pv, prior_val); UP(d_pi, h->h_prior_isig);
-    P.uv_cm = d_uv_cm; P.isig_cm = d_isig_cm; P.pt_cm = d_pt_cm; P.img_cm = d_img_cm;
-    P.uv_pm = d_uv_pm; P.isig_pm = d_isig_pm; P.img_pm = d_img_pm; P.pm2cm = d_pm2cm; P.pt_start = d_pt_start;
-    P.chunks = d_chunks; P.sh_col = d_sh; P.eo_col = d_eo; P.op_col = d_op;
-    P.prior_col = d_pc; P.prior_val = d_pv; P.prior_isig = d_pi;
+    UP(P.uv_cm, up.uv_cm); UP(P.isig_cm, up.isig_cm); UP(P.uv_pm, up.uv_pm); UP(P.isig_pm, up.isig_pm);
+    UP(P.pt_cm, pl.pt_cm); UP(P.img_cm, pl.img_cm); UP(P.img_pm, up.img_pm); UP(P.pm2cm, pl.pm2cm);
+    UP(P.pt_start, pl.pt_start); UP(P.chunks, up.chunks);
+    UP(P.sh_col, pl.sh_col); UP(P.eo_col, pl.eo_col); UP(P.op_col, pl.op_col);
+    UP(P.prior_col, pl.prior_col); UP(P.prior_val, up.prior_val); UP(P.prior_isig, pl.prior_isig);
     {
-        std::vector<double> io(d->IOval, d->IOval + (size_t)NC * nImg), eo(d->EOval, d->EOval + (size_t)6 * nImg),
-            op(d->OPval, d->OPval + (size_t)3 * nOP);
+        std::vector<double> io(d->IOval, d->IOval + (size_t)pl.NC * pl.nImg), eo(d->EOval, d->EOval + (size_t)6 * pl.nImg),
+            op(d->OPval, d->OPval + (size_t)3 * pl.nOP);
         UP(P.IOval, io); UP(P.EOval, eo); UP(P.OPval, op);
-        std::vector<ImgRec> recs(nImg);
-        for (int i = 0; i < nImg; ++i) {
-            memset(&recs[i], 0, sizeof(ImgRec));
-            recs[i].sz = d->pxSize[2 * (size_t)(legacy ? 0 : i)];   // multi_res.m:138 passes sz(1)
-            recs[i].szy = legacy ? d->pxSize[1] : recs[i].sz;        // legacy: multiscalepts uses both axes
-            recs[i].io = ioOfImg[i];
-        }
-        UP(P.img, recs);
-        { int* d_imgio; UP(d_imgio, ioOfImg); P.img_io = d_imgio; }
-        AL(P.io, h->nIOrec);
-        UP(h->d_rep, rep);
     }
-    auto to_int = [&](const int64_t* p, int64_t cnt, bool isDest) { std::vector<int> v(cnt); for (int64_t k = 0; k < cnt; ++k) v[k] = (int)(p[k] - 1); (void)isDest; return v; };
+    UP(P.img, up.recs); UP(P.img_io, up.ioOfImg);
+    AL(P.io, pl.nIOrec);
+    UP(h->d_rep, up.rep);
     h->nIOdes = (int)d->nIOdes; h->nEOdes = (int)d->nEOdes; h->nOPdes = (int)d->nOPdes;
-    { auto v = to_int(d->IOdes_src, d->nIOdes, false); UP(h->d_IOsrc, v); }
-    { auto v = to_int(d->IOdes_dest, d->nIOdes, true); UP(h->d_IOdst, v); }
-    { auto v = to_int(d->EOdes_src, d->nEOdes, false); UP(h->d_EOsrc, v); }
-    { auto v = to_int(d->EOdes_dest, d->nEOdes, true); UP(h->d_EOdst, v); }
-    { auto v = to_int(d->OPdes_src, d->nOPdes, false); UP(h->d_OPsrc, v); }
-    { auto v = to_int(d->OPdes_dest, d->nOPdes, true); UP(h->d_OPdst, v); }
-    UP(h->d_img_chunk_start, img_chunk_start); UP(h->d_col2pt, col2pt);
-    {   // ---- reduced system: elimination order of the images, tile pattern, symbolic factorisation
-        covis_graph(nImg, nOP, h->h_pt_start.data(), img_pm.data(), h->h_adjPtr, h->h_adj);
-        std::vector<int64_t>& adjPtr = h->h_adjPtr; std::vector<int32_t>& adj = h->h_adj;
-        if (d->nCovis > 0 && d->covis_a && d->covis_b) {      // the whole project's graph (sharded problems)
-            std::vector<std::vector<int32_t>> nb(nImg);
-            for (int i = 0; i < nImg; ++i) nb[i].assign(adj.begin() + adjPtr[i], adj.begin() + adjPtr[i + 1]);
-            for (int64_t e = 0; e < d->nCovis; ++e) {
-                const int64_t a = d->covis_a[e] - 1, b = d->covis_b[e] - 1;
-                if (a < 0 || a >= nImg || b < 0 || b >= nImg) return fail_create(h, DBAT_E_BADARG, "covis edge out of range");
-                if (a == b) continue;
-                nb[a].push_back((int32_t)b); nb[b].push_back((int32_t)a);
-            }
-            adj.clear();
-            for (int i = 0; i < nImg; ++i) {
-                std::sort(nb[i].begin(), nb[i].end());
-                nb[i].erase(std::unique(nb[i].begin(), nb[i].end()), nb[i].end());
-                adjPtr[i] = (int64_t)adj.size();
-                adj.insert(adj.end(), nb[i].begin(), nb[i].end());
-            }
-            adjPtr[nImg] = (int64_t)adj.size();
-        }
-        h->h_xyz.resize((size_t)3 * nImg);
-        for (int i = 0; i < nImg; ++i) for (int a = 0; a < 3; ++a) h->h_xyz[3 * (size_t)i + a] = d->EOval[6 * (size_t)i + a];
-        h->h_nEO.assign(nImg, 0);
-        for (int i = 0; i < nImg; ++i) for (int a = 0; a < 6; ++a) if (colEO[(size_t)i * 6 + a] >= 0) h->h_nEO[i]++;
-        // IO columns: used by one image -> they travel with that image (like its EO elements); used by several ->
-        // "global", last in S.  (One shared block: every estimated IO column is global.)
-        std::vector<int> users(std::max(1, nC), 0), lastUser(std::max(1, nC), -1);
-        for (int i = 0; i < nImg; ++i)
-            for (int sl = 0; sl < DBAT_NSLOT; ++sl) {
-                const int c = h->h_io_colx[(size_t)i * DBAT_NSLOT + sl];
-                if (c >= 0 && lastUser[c] != i) { users[c]++; lastUser[c] = i; }
-            }
-        h->h_glob_x.clear();
-        h->h_colLocalImg.assign(std::max(1, nC), -1);
-        for (int c = 0; c < nC; ++c) {
-            if (users[c] >= 2 || (users[c] == 1 && !general)) h->h_glob_x.push_back(c);
-            else if (users[c] == 1) { h->h_colLocalImg[c] = lastUser[c]; h->h_nEO[lastUser[c]]++; }
-        }
-        h->h_nIOest = (int)h->h_glob_x.size();
-        if ((rc = setup_reduced(h, 1, 0))) return fail_create(h, rc, h->err);
-    }
-    const std::vector<int>& imgRank = h->tc.sym.imgRank;
+    UP(h->d_IOsrc, zero_based(d->IOdes_src, d->nIOdes)); UP(h->d_IOdst, zero_based(d->IOdes_dest, d->nIOdes));
+    UP(h->d_EOsrc, zero_based(d->EOdes_src, d->nEOdes)); UP(h->d_EOdst, zero_based(d->EOdes_dest, d->nEOdes));
+    UP(h->d_OPsrc, zero_based(d->OPdes_src, d->nOPdes)); UP(h->d_OPdst, zero_based(d->OPdes_dest, d->nOPdes));
+    UP(h->d_img_chunk_start, up.img_chunk_start); UP(h->d_col2pt, up.col2pt);
+    if ((rc = setup_reduced(h, sym))) return fail_create(h, rc, h->err);
+    const int nImg = pl.nImg, nOP = pl.nOP, nObs = pl.nObs;
     AL(P.chunkG, (size_t)std::max(1, P.nChunks) * DBAT_GSZ);
     {   // per-image Grams, their sum, camera-side prior terms and the prior r'r in ONE buffer: a multi-rank
         // evaluation sums it with a single allreduce
-        const size_t nCp = (size_t)std::max(1, nC);
+        const size_t nCp = (size_t)std::max(1, pl.nC);
         h->nEvalRed = (size_t)nImg * DBAT_GSZ + DBAT_GSZ + 2 * nCp + 8;
         AL(h->d_evalRed, h->nEvalRed);
         P.imgG = h->d_evalRed;
@@ -520,223 +298,26 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     }
     AL(P.pt, (size_t)std::max(1, nOP) * DBAT_PT_STRIDE);
     cudaMemset(P.pt, 0, sizeof(double) * (size_t)std::max(1, nOP) * DBAT_PT_STRIDE);   // the compact assembly leaves the rows of unestimated IO slots alone
-    {   // compact evaluation kernels (eval.cu): one shared IO block whose estimated slots all lie in f, pp, b1, K1-K3, P1-P2
-        bool ok = !general && nK <= 3 && nP <= 2 && getenv("DBAT_EVAL_GENERIC") == nullptr;
-        for (int sl = 0; sl < DBAT_NSLOT; ++sl) if (h->h_sh_col[sl] >= 0 && !((0x0CEFu >> sl) & 1)) ok = false;
-        P.evalCompact = ok ? 1 : 0;
-    }
     AL(P.W, (size_t)std::max(1, nObs) * DBAT_W_STRIDE);
     if (P.ioGeneral) AL(P.Wfull, (size_t)std::max(1, nObs) * DBAT_WF_STRIDE);
-    {   // point of every point-major observation
-        std::vector<int> pt_pm(nObs);
-        for (int o = 0; o < nObs; ++o) pt_pm[o] = h->h_pt_cm[h->h_pm2cm[o]];
-        int* d_pt_pm;
-        UP(d_pt_pm, pt_pm);
-        P.pt_pm = d_pt_pm;
-    }
-    {   // point-side assembly blocks: runs [begin, end) of whole points with at most DBAT_PSB observations (and at most
-        // DBAT_PSB / 2 points); a point with more observations than that goes to the one-thread-per-point kernel
-        std::vector<int> pairs, bigp;
-        int begin = 0, cnt = 0;
-        auto close = [&](int end) { if (end > begin) { pairs.push_back(begin); pairs.push_back(end); } begin = end; cnt = 0; };
-        for (int j = 0; j < nOP; ++j) {
-            const int k = h->h_pt_start[j + 1] - h->h_pt_start[j];
-            if (k > DBAT_PSB) { close(j); bigp.push_back(j); begin = j + 1; continue; }
-            if (cnt + k > DBAT_PSB || j - begin >= DBAT_PSB / 2) close(j);
-            cnt += k;
-        }
-        close(nOP);
-        P.nPsb = (int)pairs.size() / 2;
-        P.nPsbig = (int)bigp.size();
-        if (pairs.empty()) pairs.assign(2, 0);
-        if (bigp.empty()) bigp.push_back(0);
-        int *d_pairs, *d_bigp;
-        UP(d_pairs, pairs); UP(d_bigp, bigp);
-        P.psb_pt = d_pairs; P.psbig = d_bigp;
-    }
-    {   // grouped Schur index: estimated points sorted by (ray count, image list)
-        std::vector<int> cand, big;
-        cand.reserve(nOP);
-        int maxm = DBAT_GRP_MAXM;                 // DBAT_GRP_MAXM=k lowers the threshold (tests of the per-point path)
-        if (const char* e = getenv("DBAT_GRP_MAXM")) maxm = std::max(1, std::min(DBAT_GRP_MAXM, atoi(e)));
-        for (int j = 0; j < nOP; ++j) {
-            const int k = h->h_pt_start[j + 1] - h->h_pt_start[j];
-            const int* oc = &h->h_op_col[3 * (size_t)j];
-            if (k == 0 || (oc[0] < 0 && oc[1] < 0 && oc[2] < 0)) continue;
-            (k <= maxm ? cand : big).push_back(j);
-        }
-        const int* ps = h->h_pt_start.data();
-        // image lists in elimination-order rank (ascending inside a point): the union of a group is then
-        // ascending in S order, which the lower-triangular window blocks of k_schur_win rely on
-        std::vector<int> rk(std::max(1, nObs));
-        for (int j = 0; j < nOP; ++j) {
-            for (int o = ps[j]; o < ps[j + 1]; ++o) rk[o] = imgRank[img_pm[o]];
-            std::sort(rk.begin() + ps[j], rk.begin() + ps[j + 1]);
-        }
-        const int* im = rk.data();
-        // lexicographic order of the (ascending) image lists: points with similar lists become neighbours
-        std::sort(cand.begin(), cand.end(), [&](int a, int b) {
-            const int ka = ps[a + 1] - ps[a], kb = ps[b + 1] - ps[b];
-            const int* la = im + ps[a]; const int* lb = im + ps[b];
-            for (int t = 0; t < std::min(ka, kb); ++t) if (la[t] != lb[t]) return la[t] < lb[t];
-            return ka != kb ? ka < kb : a < b;
-        });
-        // greedy groups of consecutive points: at most gcap points, union of their image lists at most
-        // `mu` images (a single point always fits).  A point that lacks an image of the union simply
-        // has zero rows there.
-        const int gcap = std::max(1, std::min(WIN_GP, (int)(cand.size() / (148 * 8))));
-        const int mu = 12;
-        std::vector<int> gstart, gimg_off, gimg, uni, tmp;
-        std::vector<unsigned char> slot(std::max(1, nObs), 0);
-        gstart.push_back(0); gimg_off.push_back(0);
-        auto close_group = [&](size_t end) {
-            for (size_t i = gstart.back(); i < end; ++i) {
-                const int j = cand[i];
-                for (int o = ps[j]; o < ps[j + 1]; ++o)
-                    slot[o] = (unsigned char)(std::lower_bound(uni.begin(), uni.end(), imgRank[img_pm[o]]) - uni.begin());
-            }
-            for (int r : uni) gimg.push_back(h->tc.sym.imgOrder[r]);
-            gimg_off.push_back((int)gimg.size());
-            h->grpMaxPts = std::max(h->grpMaxPts, (int)end - gstart.back());
-            gstart.push_back((int)end);
-            P.grpMaxRays = std::max(P.grpMaxRays, (int)uni.size());
-        };
-        P.grpMaxRays = 1;
-        for (size_t i = 0; i < cand.size(); ++i) {
-            const int j = cand[i];
-            tmp.clear();
-            std::set_union(uni.begin(), uni.end(), im + ps[j], im + ps[j + 1], std::back_inserter(tmp));
-            const int cnt = (int)(i - gstart.back());
-            if (cnt > 0 && ((int)tmp.size() > mu || cnt >= gcap)) {
-                close_group(i);
-                uni.assign(im + ps[j], im + ps[j + 1]);
-            } else {
-                uni.swap(tmp);
-            }
-        }
-        if (!cand.empty()) close_group(cand.size());
-        const bool noCand = cand.empty();
-        if (noCand) { cand.push_back(0); gstart.assign(1, 0); gimg_off.assign(1, 0); gimg.push_back(0); }
-        if (big.empty()) big.push_back(0); else P.nBig = (int)big.size();
-        const int nGrp = (int)gstart.size() - 1;
-        int *d_gp, *d_big;
-        UP(d_gp, cand); UP(d_big, big);
-        P.grp_pt = d_gp; P.big_pt = d_big;
-        AL(P.vinv, (size_t)std::max(1, nOP) * 8);
-        // ---- window Schur (schur_win.cu): group headers, clusters of consecutive groups whose unions span at most
-        //      WIN_MAXW images, and the fixed-order reduction index of the cluster images
-        P.nCand = noCand ? 0 : (int)cand.size();
-        std::vector<WinHdr> hdr((size_t)std::max(1, nGrp));
-        std::vector<int> clu_grp(1, 0), clu_img_off(1, 0), clu_img;
-        std::vector<long long> clu_stg(1, 0);
-        struct Contrib { long long key, off; };
-        std::vector<Contrib> contrib;
-        std::vector<std::pair<int, long long>> icontrib;         // (image, staging offset of its shared rows)
-        const std::vector<int>& imgOrder = h->tc.sym.imgOrder;
-        for (int g = 0; g < nGrp; ++g) {
-            WinHdr& H = hdr[g];
-            memset(&H, 0, sizeof(H));
-            memset(H.obsOf, 255, sizeof(H.obsOf));
-            H.m = gimg_off[g + 1] - gimg_off[g];
-            H.ng = gstart[g + 1] - gstart[g];
-            H.p0 = gstart[g];
-            for (int gi = 0; gi < H.ng; ++gi) {
-                const int j = cand[gstart[g] + gi];
-                H.j[gi] = j; H.ob[gi] = ps[j];
-                for (int o = ps[j]; o < ps[j + 1]; ++o) H.obsOf[gi][slot[o]] = (unsigned char)(o - ps[j]);
-            }
-        }
-        {
-            const int capG = std::max(4, std::min(48, nGrp / (148 * 8)));
-            std::vector<int> win, tmpw, rg;
-            unsigned char bm[WIN_MAXW][WIN_MAXW];
-            auto close_cluster = [&](int gEnd) {
-                const int c = (int)clu_grp.size() - 1, mw = (int)win.size();
-                const long long base = clu_stg.back(), nb36 = (long long)(mw * (mw + 1) / 2) * 36;
-                memset(bm, 0, sizeof(bm));
-                for (int g = clu_grp.back(); g < gEnd; ++g) {
-                    WinHdr& H = hdr[g];
-                    for (int k = 0; k < H.m; ++k)
-                        H.wslot[k] = (unsigned char)(std::lower_bound(win.begin(), win.end(), imgRank[gimg[gimg_off[g] + k]]) - win.begin());
-                    for (int gi = 0; gi < H.ng; ++gi) {
-                        const int j = H.j[gi];
-                        for (int o1 = ps[j]; o1 < ps[j + 1]; ++o1)
-                            for (int o2 = ps[j]; o2 < ps[j + 1]; ++o2) {
-                                const int wa = H.wslot[slot[o1]], wb = H.wslot[slot[o2]];
-                                if (wa >= wb) bm[wa][wb] = 1;
-                            }
-                    }
-                }
-                for (int wa = 0; wa < mw; ++wa)
-                    for (int wb = 0; wb <= wa; ++wb)
-                        if (bm[wa][wb]) contrib.push_back({(long long)win[wa] * nImg + win[wb], base + (long long)(wa * (wa + 1) / 2 + wb) * 36});
-                for (int w = 0; w < mw; ++w) {
-                    clu_img.push_back(imgOrder[win[w]]);
-                    icontrib.push_back({imgOrder[win[w]], base + nb36 + 6 * w});
-                }
-                (void)c;
-                clu_img_off.push_back((int)clu_img.size());
-                clu_stg.push_back(base + nb36 + 16 * 6 * WIN_MAXW + 256);
-                clu_grp.push_back(gEnd);
-            };
-            for (int g = 0; g < nGrp; ++g) {
-                rg.clear();
-                for (int k = gimg_off[g]; k < gimg_off[g + 1]; ++k) rg.push_back(imgRank[gimg[k]]);
-                tmpw.clear();
-                std::set_union(win.begin(), win.end(), rg.begin(), rg.end(), std::back_inserter(tmpw));
-                const int cnt = g - clu_grp.back();
-                if (cnt > 0 && ((int)tmpw.size() > WIN_MAXW || cnt >= capG)) { close_cluster(g); win = rg; }
-                else win.swap(tmpw);
-            }
-            if (nGrp > 0) close_cluster(nGrp);
-        }
-        P.nClu = (int)clu_grp.size() - 1;
-        std::stable_sort(contrib.begin(), contrib.end(), [](const Contrib& a, const Contrib& b) { return a.key < b.key; });
-        std::vector<int> red_ptr, red_imgA, red_imgB;
-        std::vector<long long> red_off(std::max<size_t>(1, contrib.size()));
-        for (size_t k = 0; k < contrib.size(); ++k) {
-            if (k == 0 || contrib[k].key != contrib[k - 1].key) {
-                red_ptr.push_back((int)k);
-                red_imgA.push_back(imgOrder[(int)(contrib[k].key / nImg)]);
-                red_imgB.push_back(imgOrder[(int)(contrib[k].key % nImg)]);
-            }
-            red_off[k] = contrib[k].off;
-        }
-        P.nRedBlk = (int)red_ptr.size();
-        red_ptr.push_back((int)contrib.size());
-        if (red_imgA.empty()) { red_imgA.push_back(0); red_imgB.push_back(0); }
-        std::stable_sort(icontrib.begin(), icontrib.end(), [](const std::pair<int, long long>& a, const std::pair<int, long long>& b) { return a.first < b.first; });
-        std::vector<int> redi_ptr(nImg + 1, 0);
-        std::vector<long long> redi_off(std::max<size_t>(1, icontrib.size()));
-        for (size_t k = 0; k < icontrib.size(); ++k) { redi_ptr[icontrib[k].first + 1]++; redi_off[k] = icontrib[k].second; }
-        for (int i = 0; i < nImg; ++i) redi_ptr[i + 1] += redi_ptr[i];
-        if (clu_img.empty()) clu_img.push_back(0);
-        {
-            std::vector<int> order((size_t)std::max(1, P.nClu), 0);
-            for (int c = 0; c < P.nClu; ++c) order[c] = c;
-            std::stable_sort(order.begin(), order.begin() + P.nClu, [&](int a, int b) { return clu_grp[a + 1] - clu_grp[a] > clu_grp[b + 1] - clu_grp[b]; });
-            int* d_co; UP(d_co, order); P.clu_order = d_co;
-        }
-        {
-            WinHdr* d_h; int *d_cg, *d_cio, *d_ci, *d_rp, *d_ra, *d_rb, *d_ip; long long *d_cs, *d_ro, *d_io;
-            UP(d_h, hdr); UP(d_cg, clu_grp); UP(d_cio, clu_img_off); UP(d_ci, clu_img); UP(d_cs, clu_stg);
-            UP(d_rp, red_ptr); UP(d_ra, red_imgA); UP(d_rb, red_imgB); UP(d_ro, red_off); UP(d_ip, redi_ptr); UP(d_io, redi_off);
-            P.win_hdr = d_h; P.clu_grp = d_cg; P.clu_img_off = d_cio; P.clu_img = d_ci; P.clu_stg = d_cs;
-            P.red_ptr = d_rp; P.red_imgA = d_ra; P.red_imgB = d_rb; P.red_off = d_ro; P.redi_ptr = d_ip; P.redi_off = d_io;
-        }
-        AL(P.winM, ((size_t)P.nCand + WIN_GP) * 6);
-        AL(P.win_stg, (size_t)std::max<long long>(2, clu_stg.back()));
-        AL(P.win_ssPart, (size_t)((P.nClu + 255) / 256 + 1) * 256);
-    }
+    UP(P.pt_pm, up.pt_pm);
+    UP(P.psb_pt, up.psb_pt); UP(P.psbig, up.psbig);
+    UP(P.grp_pt, up.grp_pt); UP(P.big_pt, up.big_pt);
+    AL(P.vinv, (size_t)std::max(1, nOP) * 8);
+    UP(P.clu_order, up.clu_order);
+    UP(P.win_hdr, up.win_hdr); UP(P.clu_grp, up.clu_grp); UP(P.clu_img_off, up.clu_img_off); UP(P.clu_img, up.clu_img);
+    UP(P.clu_stg, up.clu_stg); UP(P.red_ptr, up.red_ptr); UP(P.red_imgA, up.red_imgA); UP(P.red_imgB, up.red_imgB);
+    UP(P.red_off, up.red_off); UP(P.redi_ptr, up.redi_ptr); UP(P.redi_off, up.redi_off);
+    AL(P.winM, ((size_t)P.nCand + WIN_GP) * 6);
+    AL(P.win_stg, (size_t)std::max<long long>(2, up.clu_stg.back()));
+    AL(P.win_ssPart, (size_t)((P.nClu + 255) / 256 + 1) * 256);
     AL(h->d_tmpG, (size_t)64 * DBAT_GSZ);
-    const int nPartial = std::max(2 * ((std::max(nObs, P.n) + 255) / 256),
-                                  2 * (P.nPsb + (P.nPsbig + 127) / 128 + (nOP + 127) / 128 + 1) + 2 * ((nImg + 3) / 4 + 1)) + 64;
-    AL(h->d_partial, nPartial);
+    AL(h->d_partial, plan_partials(pl, up));
     AL(h->d_scal, SC_N);
     AL(h->d_x, P.n); AL(h->d_t, P.n); AL(h->d_p, P.n); AL(h->d_pgn, P.n); AL(h->d_g, P.n);
     AL(h->d_diagN, P.n); AL(h->d_dscale, P.n);
     AL(h->d_pEO, (size_t)6 * std::max(1, nImg) + 2);
-    AL(h->d_r, h->m);
+    AL(h->d_r, pl.m);
     if (cudaMallocHost((void**)&h->h_scal, sizeof(double) * SC_N) != cudaSuccess ||
         cudaMallocHost((void**)&h->h_G, sizeof(double) * DBAT_GSZ) != cudaSuccess ||
         cudaMallocHost((void**)&h->h_piv, sizeof(unsigned long long) * 4) != cudaSuccess)
@@ -745,7 +326,7 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     for (auto& e : h->ev) cudaEventCreate(&e);
     cudaMemset(h->d_p, 0, sizeof(double) * P.n);
     if (cudaDeviceSynchronize() != cudaSuccess) return fail_create(h, DBAT_E_CUDA, "device error during create");
-    if (!g_in_group_create) h->dcopy = copy_desc(d, NC);
+    if (!g_in_group_create) h->dcopy = copy_desc(d, pl.NC);
     *out = h;
     return DBAT_OK;
 }
@@ -771,13 +352,13 @@ extern "C" void dbat_destroy(dbat_handle* h) {
 }
 extern "C" const char* dbat_last_error(const dbat_handle* h) { return h ? h->err.c_str() : g_create_err.c_str(); }
 extern "C" int64_t dbat_num_unknowns(const dbat_handle* h) { return h ? h->P.n : 0; }
-extern "C" int64_t dbat_num_residuals(const dbat_handle* h) { return h ? h->m : 0; }
+extern "C" int64_t dbat_num_residuals(const dbat_handle* h) { return h ? h->plan.m : 0; }
 extern "C" int dbat_reduced_info(const dbat_handle* h, int64_t* info) {
     if (!h || !info) return DBAT_E_BADARG;
     if (h->group) h = group_first(h);
     const TileSym& s = h->tc.sym;
     const int64_t v[16] = {s.nT, s.ld, s.nS, s.nSlots, s.nSlotsS, s.nTasks, s.nTerms, s.depth, s.order_mode, s.nSeg,
-                           h->tc.gridFactor, h->tc.gridBwd, h->P.nPsbig, h->P.nBig, h->P.grpMaxRays, h->grpMaxPts};
+                           h->tc.gridFactor, h->tc.gridBwd, h->P.nPsbig, h->P.nBig, h->P.grpMaxRays, h->plan.grpMaxPts};
     memcpy(info, v, sizeof(v));
     return DBAT_OK;
 }
@@ -819,7 +400,7 @@ static int allreduce_max_u64(dbat_handle* h, unsigned long long* buf, size_t cnt
 static void set_params(dbat_handle* h, const double* xdev) {
     launch_set_params(h->P, xdev, ScatterList{h->d_IOsrc, h->d_IOdst, h->P.IOval, h->nIOdes, 0},
                       ScatterList{h->d_EOsrc, h->d_EOdst, h->P.EOval, h->nEOdes, 0},
-                      ScatterList{h->d_OPsrc, h->d_OPdst, h->P.OPval, h->nOPdes, 0}, h->d_rep, h->nIOrec, h->st);
+                      ScatterList{h->d_OPsrc, h->d_OPdst, h->P.OPval, h->nOPdes, 0}, h->d_rep, h->plan.nIOrec, h->st);
 }
 
 static inline double gram_host(const double* G, int R, int C) {
@@ -1053,7 +634,7 @@ extern "C" int dbat_eval(dbat_handle* h, const double* x, double* r, int weighte
     set_params(h, h->d_x);
     h->params_valid = true; h->normal_valid = false; h->cscWeighted = -1;
     launch_resid(h->P, h->d_x, h->d_partial, h->d_scal, SC_RR, h->d_r, weighted, h->st);
-    if (r) CK(cudaMemcpyAsync(r, h->d_r, sizeof(double) * h->m, cudaMemcpyDeviceToHost, h->st));
+    if (r) CK(cudaMemcpyAsync(r, h->d_r, sizeof(double) * h->plan.m, cudaMemcpyDeviceToHost, h->st));
     CK(cudaStreamSynchronize(h->st));
     return DBAT_OK;
 }
@@ -1079,14 +660,14 @@ static int build_csc(dbat_handle* h, int weighted) {
     std::vector<std::vector<int>> ioUsers(n);   // IO column -> (image * NSLOT + slot) of every image that uses it, ascending
     for (int i = 0; i < P.nImg; ++i)
         for (int s = 0; s < DBAT_NSLOT; ++s) {
-            const int c = h->h_io_colx[(size_t)i * DBAT_NSLOT + s];
+            const int c = h->plan.io_colx[(size_t)i * DBAT_NSLOT + s];
             if (c >= 0) { kind[c] = 0; ioUsers[c].push_back(i * DBAT_NSLOT + s); }
         }
-    for (int e2 = 0; e2 < 6 * P.nImg; ++e2) if (h->h_eo_col[e2] >= 0) { kind[h->h_eo_col[e2]] = 1; idx[h->h_eo_col[e2]] = e2; }
-    for (int e2 = 0; e2 < 3 * P.nOP; ++e2) if (h->h_op_col[e2] >= 0) { kind[h->h_op_col[e2]] = 2; idx[h->h_op_col[e2]] = e2; }
+    for (int e2 = 0; e2 < 6 * P.nImg; ++e2) if (h->plan.eo_col[e2] >= 0) { kind[h->plan.eo_col[e2]] = 1; idx[h->plan.eo_col[e2]] = e2; }
+    for (int e2 = 0; e2 < 3 * P.nOP; ++e2) if (h->plan.op_col[e2] >= 0) { kind[h->plan.op_col[e2]] = 2; idx[h->plan.op_col[e2]] = e2; }
     std::vector<std::vector<int>> priorOfCol;   // rows of prior observations per column (rare)
     std::map<int, std::vector<int>> priorMap;
-    for (int k = 0; k < P.nPrior; ++k) priorMap[h->h_prior_col[k]].push_back(k);
+    for (int k = 0; k < P.nPrior; ++k) priorMap[h->plan.prior_col[k]].push_back(k);
     h->cscJc.assign(n + 1, 0); h->cscIr.clear(); h->cscV.clear();
     h->cscIr.reserve((size_t)P.nObs * 2 * 18); h->cscV.reserve((size_t)P.nObs * 2 * 18);
     auto push = [&](int64_t row, double v) { if (v != 0.0) { h->cscIr.push_back(row); h->cscV.push_back(v); } };
@@ -1095,28 +676,28 @@ static int build_csc(dbat_handle* h, int weighted) {
         if (kind[c] == 0) {
             for (int u : ioUsers[c]) {                        // the observations of every image that uses the column
                 const int i = u / DBAT_NSLOT, s = u % DBAT_NSLOT;
-                for (int k = h->h_img_start[i]; k < h->h_img_start[i + 1]; ++k) {
+                for (int k = h->plan.img_start[i]; k < h->plan.img_start[i + 1]; ++k) {
                     push(2 * (int64_t)k, J[((size_t)k * 2) * LD + s]);
                     push(2 * (int64_t)k + 1, J[((size_t)k * 2 + 1) * LD + s]);
                 }
             }
         } else if (kind[c] == 1) {
             const int i = idx[c] / 6, a2 = idx[c] % 6;
-            for (int k = h->h_img_start[i]; k < h->h_img_start[i + 1]; ++k) {
+            for (int k = h->plan.img_start[i]; k < h->plan.img_start[i + 1]; ++k) {
                 push(2 * (int64_t)k, J[((size_t)k * 2) * LD + DBAT_NSLOT + a2]);
                 push(2 * (int64_t)k + 1, J[((size_t)k * 2 + 1) * LD + DBAT_NSLOT + a2]);
             }
         } else if (kind[c] == 2) {
             const int j = idx[c] / 3, t = idx[c] % 3;
-            for (int o = h->h_pt_start[j]; o < h->h_pt_start[j + 1]; ++o) {
-                const int k = h->h_pm2cm[o];
+            for (int o = h->plan.pt_start[j]; o < h->plan.pt_start[j + 1]; ++o) {
+                const int k = h->plan.pm2cm[o];
                 push(2 * (int64_t)k, J[((size_t)k * 2) * LD + DBAT_NSLOT + 6 + t]);
                 push(2 * (int64_t)k + 1, J[((size_t)k * 2 + 1) * LD + DBAT_NSLOT + 6 + t]);
             }
         }
         auto it = priorMap.find(c);
         if (it != priorMap.end())
-            for (int k : it->second) push(2 * (int64_t)P.nObs + k, weighted ? h->h_prior_isig[k] : 1.0);
+            for (int k : it->second) push(2 * (int64_t)P.nObs + k, weighted ? h->plan.prior_isig[k] : 1.0);
         h->cscJc[c + 1] = (int64_t)h->cscIr.size();
     }
     h->cscWeighted = weighted;
@@ -1242,7 +823,7 @@ static bool term_fun(const dbat_opts* o, double jp2, double rr) {
 static bool matching_deficient(dbat_handle* h) {
     DevProblem& P = h->P;
     if (!h->params_valid) { set_params(h, h->d_x); h->params_valid = true; }
-    const int n = P.n, m = h->m, nObs = P.nObs;
+    const int n = P.n, m = h->plan.m, nObs = P.nObs;
     const int LD = DBAT_NSLOT + 9;
     std::vector<unsigned long long> mask(std::max(1, nObs));
     {
@@ -1260,22 +841,22 @@ static bool matching_deficient(dbat_handle* h) {
     std::vector<std::vector<int64_t>> ioCum(n);          // ... and the running count of their observations
     for (int i = 0; i < P.nImg; ++i)
         for (int s = 0; s < DBAT_NSLOT; ++s) {
-            const int c = h->h_io_colx[(size_t)i * DBAT_NSLOT + s];
+            const int c = h->plan.io_colx[(size_t)i * DBAT_NSLOT + s];
             if (c < 0) continue;
             kind[c] = 0;
             ioUsers[c].push_back(i * DBAT_NSLOT + s);
-            ioCum[c].push_back((ioCum[c].empty() ? 0 : ioCum[c].back()) + (h->h_img_start[i + 1] - h->h_img_start[i]));
+            ioCum[c].push_back((ioCum[c].empty() ? 0 : ioCum[c].back()) + (h->plan.img_start[i + 1] - h->plan.img_start[i]));
         }
-    for (int e2 = 0; e2 < 6 * P.nImg; ++e2) if (h->h_eo_col[e2] >= 0) { kind[h->h_eo_col[e2]] = 1; idx[h->h_eo_col[e2]] = e2; }
-    for (int e2 = 0; e2 < 3 * P.nOP; ++e2) if (h->h_op_col[e2] >= 0) { kind[h->h_op_col[e2]] = 2; idx[h->h_op_col[e2]] = e2; }
+    for (int e2 = 0; e2 < 6 * P.nImg; ++e2) if (h->plan.eo_col[e2] >= 0) { kind[h->plan.eo_col[e2]] = 1; idx[h->plan.eo_col[e2]] = e2; }
+    for (int e2 = 0; e2 < 3 * P.nOP; ++e2) if (h->plan.op_col[e2] >= 0) { kind[h->plan.op_col[e2]] = 2; idx[h->plan.op_col[e2]] = e2; }
     std::vector<std::vector<int>> priorRows(n);
-    for (int k = 0; k < P.nPrior; ++k) priorRows[h->h_prior_col[k]].push_back(2 * nObs + k);
+    for (int k = 0; k < P.nPrior; ++k) priorRows[h->plan.prior_col[k]].push_back(2 * nObs + k);
     // adjacency of column c: position pos in [0, deg(c)) -> row or -1 (entry is an exact zero)
     auto degree = [&](int c) -> int64_t {
         int64_t d = (int64_t)priorRows[c].size();
         if (kind[c] == 0) d += 2 * (ioCum[c].empty() ? 0 : ioCum[c].back());
-        else if (kind[c] == 1) { const int i = idx[c] / 6; d += 2 * (int64_t)(h->h_img_start[i + 1] - h->h_img_start[i]); }
-        else if (kind[c] == 2) { const int j = idx[c] / 3; d += 2 * (int64_t)(h->h_pt_start[j + 1] - h->h_pt_start[j]); }
+        else if (kind[c] == 1) { const int i = idx[c] / 6; d += 2 * (int64_t)(h->plan.img_start[i + 1] - h->plan.img_start[i]); }
+        else if (kind[c] == 2) { const int j = idx[c] / 3; d += 2 * (int64_t)(h->plan.pt_start[j + 1] - h->plan.pt_start[j]); }
         return d;
     };
     auto row_at = [&](int c, int64_t pos) -> int {
@@ -1287,10 +868,10 @@ static bool matching_deficient(dbat_handle* h) {
             const int64_t q = pos >> 1;
             const size_t u = (size_t)(std::upper_bound(ioCum[c].begin(), ioCum[c].end(), q) - ioCum[c].begin());
             const int i = ioUsers[c][u] / DBAT_NSLOT;
-            k = h->h_img_start[i] + (int)(q - (u ? ioCum[c][u - 1] : 0)); slot = ioUsers[c][u] % DBAT_NSLOT;
+            k = h->plan.img_start[i] + (int)(q - (u ? ioCum[c][u - 1] : 0)); slot = ioUsers[c][u] % DBAT_NSLOT;
         }
-        else if (kind[c] == 1) { k = h->h_img_start[idx[c] / 6] + (int)(pos >> 1); slot = DBAT_NSLOT + idx[c] % 6; }
-        else { k = h->h_pm2cm[h->h_pt_start[idx[c] / 3] + (int)(pos >> 1)]; slot = DBAT_NSLOT + 6 + idx[c] % 3; }
+        else if (kind[c] == 1) { k = h->plan.img_start[idx[c] / 6] + (int)(pos >> 1); slot = DBAT_NSLOT + idx[c] % 6; }
+        else { k = h->plan.pm2cm[h->plan.pt_start[idx[c] / 3] + (int)(pos >> 1)]; slot = DBAT_NSLOT + 6 + idx[c] % 3; }
         return ((mask[k] >> (LD * r + slot)) & 1ull) ? 2 * k + r : -1;
     };
     std::vector<int> matchRow(m, -1), matchCol(n, -1), stamp(m, -1);
@@ -1333,18 +914,18 @@ static bool matching_deficient(dbat_handle* h) {
 static bool structurally_deficient(dbat_handle* h) {
     DevProblem& P = h->P;
     if (h->nranks > 1) return false;
-    if (h->m < P.n) return true;
+    if (h->plan.m < P.n) return true;
     std::vector<int> priorCnt(P.n, 0);
-    for (int c : h->h_prior_col) priorCnt[c]++;
+    for (int c : h->plan.prior_col) priorCnt[c]++;
     for (int j = 0; j < P.nOP; ++j) {
         int freec = 0, pri = 0;
-        for (int t = 0; t < 3; ++t) { const int c = h->h_op_col[3 * (size_t)j + t]; if (c >= 0) { ++freec; pri += priorCnt[c]; } }
-        if (freec && 2 * (h->h_pt_start[j + 1] - h->h_pt_start[j]) + pri < freec) return true;
+        for (int t = 0; t < 3; ++t) { const int c = h->plan.op_col[3 * (size_t)j + t]; if (c >= 0) { ++freec; pri += priorCnt[c]; } }
+        if (freec && 2 * (h->plan.pt_start[j + 1] - h->plan.pt_start[j]) + pri < freec) return true;
     }
     for (int i = 0; i < P.nImg; ++i) {
         int freec = 0, pri = 0;
-        for (int a = 0; a < 6; ++a) { const int c = h->h_eo_col[6 * (size_t)i + a]; if (c >= 0) { ++freec; pri += priorCnt[c]; } }
-        if (freec && 2 * (h->h_img_start[i + 1] - h->h_img_start[i]) + pri < freec) return true;
+        for (int a = 0; a < 6; ++a) { const int c = h->plan.eo_col[6 * (size_t)i + a]; if (c >= 0) { ++freec; pri += priorCnt[c]; } }
+        if (freec && 2 * (h->plan.img_start[i + 1] - h->plan.img_start[i]) + pri < freec) return true;
     }
     static const bool skipExact = getenv("DBAT_NO_SPRANK") != nullptr;
     if (skipExact) return false;
@@ -1642,12 +1223,12 @@ extern "C" int dbat_solve(dbat_handle* h, int method, const dbat_opts* opts, con
         set_params(h, h->d_x); h->params_valid = true;
         if (res->r_w) {
             launch_resid(h->P, h->d_x, h->d_partial, h->d_scal, SC_PRR, h->d_r, 1, h->st);
-            CK(cudaMemcpyAsync(res->r_w, h->d_r, sizeof(double) * h->m, cudaMemcpyDeviceToHost, h->st));
+            CK(cudaMemcpyAsync(res->r_w, h->d_r, sizeof(double) * h->plan.m, cudaMemcpyDeviceToHost, h->st));
             CK(cudaStreamSynchronize(h->st));
         }
         if (res->r_u) {
             launch_resid(h->P, h->d_x, h->d_partial, h->d_scal, SC_PRR, h->d_r, 0, h->st);
-            CK(cudaMemcpyAsync(res->r_u, h->d_r, sizeof(double) * h->m, cudaMemcpyDeviceToHost, h->st));
+            CK(cudaMemcpyAsync(res->r_u, h->d_r, sizeof(double) * h->plan.m, cudaMemcpyDeviceToHost, h->st));
         }
     }
     ph_collect(h);
@@ -1833,7 +1414,7 @@ extern "C" int dbat_cov(dbat_handle* h, int which, double s0, double* out) {
     cudaError_t e = cudaSuccess;
     const double s02 = s0 * s0;
     const int nC = P.nC, ld = ldd;
-    const std::vector<int>& x2s = h->h_x2s;
+    const std::vector<int>& x2s = h->plan.x2s;
     if ((which == DBAT_COV_CXX || which == DBAT_COV_CXX_OP) && P.ioGeneral) {
         cudaFree(Z); cudaFree(C);
         h->err = "the dense point covariance (CXX / COPF) is built for one shared IO block only; use CIO / CEO / COP";
@@ -1908,8 +1489,8 @@ extern "C" int dbat_cov(dbat_handle* h, int which, double s0, double* out) {
         if (which == DBAT_COV_CXX_CAM) {
             for (int b = 0; b < nC; ++b) for (int a = 0; a < nC; ++a) out[(size_t)b * nC + a] = cv(a, b);
         } else if (which == DBAT_COV_CEO || which == DBAT_COV_CIO) {
-            const int R = which == DBAT_COV_CEO ? 6 : h->NC;
-            const std::vector<int>& col = which == DBAT_COV_CEO ? h->h_eo_col : h->h_io_col;
+            const int R = which == DBAT_COV_CEO ? 6 : h->plan.NC;
+            const std::vector<int>& col = which == DBAT_COV_CEO ? h->plan.eo_col : h->plan.io_col;
             for (int i = 0; i < P.nImg; ++i)
                 for (int b = 0; b < R; ++b)
                     for (int a = 0; a < R; ++a) {
@@ -1943,17 +1524,17 @@ extern "C" int dbat_cov_stats(dbat_handle* h, double s0, double thres, double* s
     if ((rc = cov_factor(h, &Z, &C, &ld, &info))) return rc;
     cudaFree(Z);
     const double s02 = s0 * s0;
-    const int NC = h->NC, nImg = P.nImg;
+    const int NC = h->plan.NC, nImg = P.nImg;
     int *d_x2s = nullptr, *d_iocol = nullptr;
     double *d_std = nullptr, *d_blk = nullptr;
     const size_t nBlk = std::max<size_t>(std::max<size_t>((size_t)NC * NC * nImg, (size_t)36 * nImg), (size_t)9 * std::max(1, P.nOP));
-    if (cudaMalloc(&d_x2s, sizeof(int) * std::max<size_t>(1, h->h_x2s.size())) || cudaMalloc(&d_iocol, sizeof(int) * std::max<size_t>(1, h->h_io_col.size())) ||
+    if (cudaMalloc(&d_x2s, sizeof(int) * std::max<size_t>(1, h->plan.x2s.size())) || cudaMalloc(&d_iocol, sizeof(int) * std::max<size_t>(1, h->plan.io_col.size())) ||
         cudaMalloc(&d_std, sizeof(double) * std::max(1, P.n)) || cudaMalloc(&d_blk, sizeof(double) * std::max<size_t>(1, nBlk))) {
         cudaFree(C); cudaFree(d_x2s); cudaFree(d_iocol); cudaFree(d_std); cudaFree(d_blk);
         h->err = "out of memory for the covariance statistics"; return DBAT_E_OOM;
     }
-    cudaMemcpyAsync(d_x2s, h->h_x2s.data(), sizeof(int) * h->h_x2s.size(), cudaMemcpyHostToDevice, h->st);
-    cudaMemcpyAsync(d_iocol, h->h_io_col.data(), sizeof(int) * h->h_io_col.size(), cudaMemcpyHostToDevice, h->st);
+    cudaMemcpyAsync(d_x2s, h->plan.x2s.data(), sizeof(int) * h->plan.x2s.size(), cudaMemcpyHostToDevice, h->st);
+    cudaMemcpyAsync(d_iocol, h->plan.io_col.data(), sizeof(int) * h->plan.io_col.size(), cudaMemcpyHostToDevice, h->st);
     cudaMemsetAsync(d_std, 0, sizeof(double) * std::max(1, P.n), h->st);
     int ce = 0;
     auto run = [&](const int* cols, int k, long long N, dbat_cov_hit_list* L) {
@@ -2322,7 +1903,7 @@ extern "C" int dbat_set_devices(dbat_handle* h, const int* dev, int ndev) {
     // global co-visibility edges (the front handle analysed the whole project at create)
     std::vector<int64_t> ea, eb;
     for (int i = 0; i < nImg; ++i)
-        for (int64_t k = h->h_adjPtr[i]; k < h->h_adjPtr[i + 1]; ++k) if (h->h_adj[k] > i) { ea.push_back(i + 1); eb.push_back(h->h_adj[k] + 1); }
+        for (int64_t k = h->plan.adjPtr[i]; k < h->plan.adjPtr[i + 1]; ++k) if (h->plan.adj[k] > i) { ea.push_back(i + 1); eb.push_back(h->plan.adj[k] + 1); }
     G->obs.resize(ndev); G->prow.resize(ndev); G->ownCols.resize(ndev); G->sd.resize(ndev);
     const int64_t nPr = D.nPriorIO + D.nPriorEO + D.nPriorOP;
     for (int r = 0; r < ndev; ++r) {
@@ -2484,7 +2065,7 @@ static int group_cov(dbat_handle* h, int which, double s0, double* out) {
     if (which == DBAT_COV_CXX || which == DBAT_COV_CXX_OP) { h->err = "the dense point covariance is single-device only; use COP"; return DBAT_E_UNSUPPORTED; }
     std::vector<int> rcs(G->ndev, 0);
     std::vector<std::vector<double>> part(G->ndev);
-    const size_t camSize = which == DBAT_COV_CIO ? (size_t)h->NC * h->NC * h->P.nImg : which == DBAT_COV_CEO ? (size_t)36 * h->P.nImg : (size_t)G->nC * G->nC;
+    const size_t camSize = which == DBAT_COV_CIO ? (size_t)h->plan.NC * h->plan.NC * h->P.nImg : which == DBAT_COV_CEO ? (size_t)36 * h->P.nImg : (size_t)G->nC * G->nC;
     G->run_all([&](int k) {
         part[k].assign(which == DBAT_COV_COP ? (size_t)9 * std::max(1, G->hi[k] - G->lo[k]) : std::max<size_t>(1, camSize), 0.0);
         rcs[k] = dbat_cov(G->sub[k], which, s0, part[k].data());
@@ -2518,6 +2099,13 @@ extern "C" int dbat_comm_init(dbat_handle* h, int nranks, int rank, const void* 
     if (rc != 0) { h->err = std::string("ncclCommInitRank: ") + (g_nccl.GetErrorString ? g_nccl.GetErrorString(rc) : "?"); return DBAT_E_NCCL; }
     h->nranks = nranks; h->rank = rank;
     // distribute the factorisation: cut the elimination tree into one subtree per rank (tilesym.cu)
-    if ((rc = setup_reduced(h, nranks, rank))) return rc;
-    return DBAT_OK;
+    TileSym sym;
+    if ((rc = analyse_reduced(h, nranks, rank, sym))) return rc;
+    // the window Schur index was built at create for the one-part order: its camera-pair blocks are lower
+    // triangular in S only while the images with columns in S keep that order
+    if (!plan_same_order(h->plan, h->tc.sym, sym)) {
+        h->err = "the distributed elimination order differs from the one the window Schur index was built for";
+        return DBAT_E_STATE;
+    }
+    return setup_reduced(h, sym);
 }

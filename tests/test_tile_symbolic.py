@@ -259,3 +259,24 @@ def test_distributed_schedule_factors_the_reduced_system(built_lib, parts):
         keep = np.repeat((owner == g) | ((owner < 0) & (g == 0)), T)
         xsum += x * keep
     np.testing.assert_allclose(xsum[:n1], np.linalg.solve(S[:n1, :n1], rhs[:n1]), rtol=1e-9, atol=1e-12)
+
+
+@pytest.mark.parametrize('nImg,nOP', [(300, 20000), (1000, 40000)])
+def test_distributed_analysis_keeps_the_image_order(built_lib, nImg, nOP):
+    """The window Schur index is built at create from the one-part elimination order, and dbat_comm_init refuses a
+    distributed analysis that orders the images with columns in S differently.  On synthetic blocks with a datum
+    camera without columns, every part of a 2-, 4- or 8-part analysis keeps the one-part order."""
+    s, _ = make_scene(nImg, nOP, rays=8, seed=17, build_indices=False)
+    nEO = s.bundle.est.EO[:6].sum(axis=0).astype(int)
+    assert (nEO == 0).any()
+    has = np.flatnonzero(nEO > 0)
+
+    def order(parts, part):
+        sym = _lib.tile_symbolic(s.IP.img, s.IP.op, nImg, nOP, nEO, 9, parts=parts, part=part)
+        assert sym['nParts'] == parts
+        return has[np.argsort(sym['imgS'][has])]
+
+    ref = order(1, 0)
+    for parts in (2, 4, 8):
+        for part in range(parts):
+            assert np.array_equal(order(parts, part), ref), (parts, part)

@@ -6,7 +6,7 @@ cd "$(dirname "$0")/.."
 name=$1; shift
 mkdir -p variants/obj_$name
 objs=""
-for f in eval schur schur_win chol tilechol tilesym general_io covstats api startval order; do
+for f in eval schur schur_win chol tilechol tilesym plan general_io covstats api startval order; do
   o=dbat_b200/csrc/$f.o
   if grep -q "$VARIANT_FILES_PLACEHOLDER" /dev/null 2>/dev/null; then :; fi
   case " $VARIANT_FILES " in
