@@ -1276,50 +1276,54 @@ __global__ void k_cov_rows(DevProblem P, double* __restrict__ T, int* __restrict
 __global__ void k_cov_U(DevProblem P, const double* __restrict__ C, int ldc, const double* __restrict__ dsc,
                         const double* __restrict__ T, const int* __restrict__ Tc, const int* __restrict__ x2s,
                         double* __restrict__ U) {
-    const int rx = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;
+    const int rx = blockIdx.x * blockDim.x + threadIdx.x;
     if (rx >= P.nC) return;
     const int r = x2s[rx];
-    const int* opc = P.op_col + 3 * (size_t)j;
-    if (opc[0] < 0 && opc[1] < 0 && opc[2] < 0) return;
-    const size_t r0 = (size_t)DBAT_NSLOT * j + 6 * (size_t)P.pt_start[j];
-    const int rows = DBAT_NSLOT + 6 * (P.pt_start[j + 1] - P.pt_start[j]);
-    double u[3] = {0.0, 0.0, 0.0};
     const double dr = dsc[r];
-    for (int a = 0; a < rows; ++a) {
-        const int ca = Tc[r0 + a];
-        if (ca < 0) continue;
-        const double c = C[(size_t)ca * ldc + r] * dr * dsc[ca];
-        const double* t = T + 3 * (r0 + a);
-        u[0] += c * t[0]; u[1] += c * t[1]; u[2] += c * t[2];
+    for (int j = blockIdx.y; j < P.nOP; j += gridDim.y) {       // gridDim.y stops at 65535, nOP does not
+        const int* opc = P.op_col + 3 * (size_t)j;
+        if (opc[0] < 0 && opc[1] < 0 && opc[2] < 0) continue;
+        const size_t r0 = (size_t)DBAT_NSLOT * j + 6 * (size_t)P.pt_start[j];
+        const int rows = DBAT_NSLOT + 6 * (P.pt_start[j + 1] - P.pt_start[j]);
+        double u[3] = {0.0, 0.0, 0.0};
+        for (int a = 0; a < rows; ++a) {
+            const int ca = Tc[r0 + a];
+            if (ca < 0) continue;
+            const double c = C[(size_t)ca * ldc + r] * dr * dsc[ca];
+            const double* t = T + 3 * (r0 + a);
+            u[0] += c * t[0]; u[1] += c * t[1]; u[2] += c * t[2];
+        }
+        for (int t = 0; t < 3; ++t) if (opc[t] >= 0) U[(size_t)(opc[t] - P.nC) * P.nC + rx] = u[t];
     }
-    for (int t = 0; t < 3; ++t) if (opc[t] >= 0) U[(size_t)(opc[t] - P.nC) * P.nC + rx] = u[t];
 }
 __global__ void k_cov_pp(DevProblem P, const double* __restrict__ T, const int* __restrict__ Tc,
                          const double* __restrict__ U, const int* __restrict__ col2pt, double* __restrict__ Cpp) {
     const int m3 = P.n - P.nC;
-    const int xc = blockIdx.x * blockDim.x + threadIdx.x, j = blockIdx.y;      // column xc (point j'), row point j
+    const int xc = blockIdx.x * blockDim.x + threadIdx.x;      // column xc (point j'), row point j
     if (xc >= m3) return;
-    const int* opc = P.op_col + 3 * (size_t)j;
-    if (opc[0] < 0 && opc[1] < 0 && opc[2] < 0) return;
-    const size_t r0 = (size_t)DBAT_NSLOT * j + 6 * (size_t)P.pt_start[j];
-    const int rows = DBAT_NSLOT + 6 * (P.pt_start[j + 1] - P.pt_start[j]);
-    double acc[3] = {0.0, 0.0, 0.0};
     const double* Uc = U + (size_t)xc * P.nC;
-    for (int a = 0; a < rows; ++a) {
-        const int ca = Tc[r0 + a];
-        if (ca < 0) continue;
-        const double u = Uc[P.s2x[ca]];
-        const double* t = T + 3 * (r0 + a);
-        acc[0] += t[0] * u; acc[1] += t[1] * u; acc[2] += t[2] * u;
-    }
     const int code = col2pt[xc];                          // 3 j' + t' of OP column nC + xc
-    if (code / 3 == j) {
-        const double* v = P.vinv + (size_t)j * 8;
-        const int tp = code % 3;
-        const double Vrow[3][3] = {{v[0], v[1], v[2]}, {v[1], v[3], v[4]}, {v[2], v[4], v[5]}};
-        acc[0] += Vrow[0][tp]; acc[1] += Vrow[1][tp]; acc[2] += Vrow[2][tp];
+    for (int j = blockIdx.y; j < P.nOP; j += gridDim.y) {
+        const int* opc = P.op_col + 3 * (size_t)j;
+        if (opc[0] < 0 && opc[1] < 0 && opc[2] < 0) continue;
+        const size_t r0 = (size_t)DBAT_NSLOT * j + 6 * (size_t)P.pt_start[j];
+        const int rows = DBAT_NSLOT + 6 * (P.pt_start[j + 1] - P.pt_start[j]);
+        double acc[3] = {0.0, 0.0, 0.0};
+        for (int a = 0; a < rows; ++a) {
+            const int ca = Tc[r0 + a];
+            if (ca < 0) continue;
+            const double u = Uc[P.s2x[ca]];
+            const double* t = T + 3 * (r0 + a);
+            acc[0] += t[0] * u; acc[1] += t[1] * u; acc[2] += t[2] * u;
+        }
+        if (code / 3 == j) {
+            const double* v = P.vinv + (size_t)j * 8;
+            const int tp = code % 3;
+            const double Vrow[3][3] = {{v[0], v[1], v[2]}, {v[1], v[3], v[4]}, {v[2], v[4], v[5]}};
+            acc[0] += Vrow[0][tp]; acc[1] += Vrow[1][tp]; acc[2] += Vrow[2][tp];
+        }
+        for (int t = 0; t < 3; ++t) if (opc[t] >= 0) Cpp[(size_t)xc * m3 + (opc[t] - P.nC)] = acc[t];
     }
-    for (int t = 0; t < 3; ++t) if (opc[t] >= 0) Cpp[(size_t)xc * m3 + (opc[t] - P.nC)] = acc[t];
 }
 
 __global__ void k_dense_unit_diag(double* __restrict__ A, int ld, int from) {
@@ -1355,6 +1359,7 @@ static int cov_factor(dbat_handle* h, double** Zp, double** Cp, int* ldp, int* i
     // identical everywhere, COP covers the points of this rank (it shards by point like the solve, bundle_cov.m:400-455)
     DevProblem& P = h->P;
     int rc;
+    cudaGetLastError();                      // a launch error reported by this call is one of its own launches
     if (!h->normal_valid) { if ((rc = eval_full(h))) return rc; }
     launch_build_S(P, h->d_camDiag, h->d_camG, 0.0, h->st);
     if (h->nranks > 1 && h->rank != 0) { tchol_zero(h->tc, h->st); cudaMemsetAsync(P.rhs, 0, sizeof(double) * P.ldS, h->st); }
@@ -1386,14 +1391,19 @@ static int cov_factor(dbat_handle* h, double** Zp, double** Cp, int* ldp, int* i
     // factorisation of the full normal matrix fail (bundle_cov.m:87-107): report that, not huge numbers
     if (P.nOP > 0) k_point_pd_check<<<(P.nOP + 255) / 256, 256, 0, h->st>>>(P, d_bad);
     count_launch(2);
+    // a failed launch leaves no trace a stream synchronisation reports: ask for it (before chol_factor, whose
+    // fall-back from graph capture clears the error state)
+    cudaError_t le = cudaGetLastError();
     CholWork cw;
     chol_alloc(cw, P.ldS - 1, ldd);
     chol_factor(cw, Sd, h->st);
     chol_inverse(cw, Sd, Z, C, h->st);
+    if (le == cudaSuccess) le = cudaGetLastError();
     int info = 0, badPts = 0;
     cudaMemcpyAsync(&info, cw.info, sizeof(int), cudaMemcpyDeviceToHost, h->st);
     cudaMemcpyAsync(&badPts, d_bad, sizeof(int), cudaMemcpyDeviceToHost, h->st);
     cudaError_t e = cudaStreamSynchronize(h->st);
+    if (e == cudaSuccess) e = le;
     chol_free(cw);
     cudaFree(Sd); cudaFree(d_bad);
     if (e != cudaSuccess) { cudaFree(Z); cudaFree(C); h->err = std::string("dbat_cov: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
@@ -1442,10 +1452,12 @@ extern "C" int dbat_cov(dbat_handle* h, int which, double s0, double* out) {
         if (P.nOP > 0 && m3 > 0) {
             launch_point_vinv(P, 0.0, h->st);
             k_cov_rows<<<(P.nOP + 127) / 128, 128, 0, h->st>>>(P, T, Tc);
-            k_cov_U<<<dim3((nC + 127) / 128, P.nOP), 128, 0, h->st>>>(P, C, ld, h->d_dS, T, Tc, d_x2s, U);
-            k_cov_pp<<<dim3((m3 + 127) / 128, P.nOP), 128, 0, h->st>>>(P, T, Tc, U, h->d_col2pt, Cpp);
+            const unsigned gy = (unsigned)std::min(P.nOP, 65535);
+            k_cov_U<<<dim3((nC + 127) / 128, gy), 128, 0, h->st>>>(P, C, ld, h->d_dS, T, Tc, d_x2s, U);
+            k_cov_pp<<<dim3((m3 + 127) / 128, gy), 128, 0, h->st>>>(P, T, Tc, U, h->d_col2pt, Cpp);
             count_launch(3);
         }
+        const cudaError_t le = cudaGetLastError();
         std::vector<double> hpp((size_t)m3 * m3), hu, hc, dsc;
         cudaMemcpyAsync(hpp.data(), Cpp, sizeof(double) * hpp.size(), cudaMemcpyDeviceToHost, h->st);
         if (which == DBAT_COV_CXX) {
@@ -1455,7 +1467,9 @@ extern "C" int dbat_cov(dbat_handle* h, int which, double s0, double* out) {
             cudaMemcpyAsync(dsc.data(), h->d_dscale, sizeof(double) * nC, cudaMemcpyDeviceToHost, h->st);
         }
         e = cudaStreamSynchronize(h->st);
+        if (e == cudaSuccess) e = le;
         cudaFree(d_x2s); cudaFree(T); cudaFree(Tc); cudaFree(U); cudaFree(Cpp);
+        if (e != cudaSuccess) { cudaFree(Z); cudaFree(C); h->err = std::string("dbat_cov: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
         const double nanv = NAN;
         if (which == DBAT_COV_CXX_OP) {
             for (size_t k = 0; k < hpp.size(); ++k) out[k] = info != 0 ? nanv : s02 * hpp[k];
@@ -1477,14 +1491,17 @@ extern "C" int dbat_cov(dbat_handle* h, int which, double s0, double* out) {
         cudaMemsetAsync(dOut, 0, sizeof(double) * 9 * (size_t)std::max(1, P.nOP), h->st);
         if (P.nOP > 0 && P.ioGeneral) launch_cop_gen(P, C, ld, h->d_dS, s02, dOut, h->st);
         else if (P.nOP > 0) { k_cop<<<(P.nOP + 3) / 4, 128, 0, h->st>>>(P, C, ld, h->d_dS, s02, dOut); count_launch(); }
+        const cudaError_t le = cudaGetLastError();
         cudaMemcpyAsync(out, dOut, sizeof(double) * 9 * (size_t)P.nOP, cudaMemcpyDeviceToHost, h->st);
         e = cudaStreamSynchronize(h->st);
+        if (e == cudaSuccess) e = le;
         cudaFree(dOut);
     } else {
         // bring the camera covariance to the host and unscale: C = D Cs D
         std::vector<double> hc((size_t)ld * ld), dsc(std::max(1, nC));
-        cudaMemcpy(hc.data(), C, sz, cudaMemcpyDeviceToHost);
-        cudaMemcpy(dsc.data(), h->d_dscale, sizeof(double) * nC, cudaMemcpyDeviceToHost);
+        e = cudaMemcpy(hc.data(), C, sz, cudaMemcpyDeviceToHost);
+        if (e == cudaSuccess) e = cudaMemcpy(dsc.data(), h->d_dscale, sizeof(double) * nC, cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) { cudaFree(Z); cudaFree(C); h->err = std::string("dbat_cov: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
         auto cv = [&](int a, int b) { return (info != 0) ? NAN : s02 * hc[(size_t)x2s[b] * ld + x2s[a]] * dsc[a] * dsc[b]; };
         if (which == DBAT_COV_CXX_CAM) {
             for (int b = 0; b < nC; ++b) for (int a = 0; a < nC; ++a) out[(size_t)b * nC + a] = cv(a, b);
@@ -1555,8 +1572,10 @@ extern "C" int dbat_cov_stats(dbat_handle* h, double s0, double thres, double* s
     if (P.nOP > 0 && P.ioGeneral) launch_cop_gen(P, C, ld, h->d_dS, s02, d_blk, h->st);
     else if (P.nOP > 0) { k_cop<<<(P.nOP + 3) / 4, 128, 0, h->st>>>(P, C, ld, h->d_dS, s02, d_blk); count_launch(); }
     run(P.op_col, 3, P.nOP, op);
+    const cudaError_t le = cudaGetLastError();
     cudaMemcpyAsync(std_x, d_std, sizeof(double) * P.n, cudaMemcpyDeviceToHost, h->st);
     cudaError_t e = cudaStreamSynchronize(h->st);
+    if (e == cudaSuccess) e = le;
     cudaFree(C); cudaFree(d_x2s); cudaFree(d_iocol); cudaFree(d_std); cudaFree(d_blk);
     if (e != cudaSuccess || ce) { h->err = std::string("dbat_cov_stats: ") + cudaGetErrorString(e != cudaSuccess ? e : (cudaError_t)ce); return DBAT_E_CUDA; }
     if (info != 0) { for (int c = 0; c < P.n; ++c) std_x[c] = NAN; return DBAT_E_NOTSPD; }

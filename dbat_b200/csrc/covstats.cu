@@ -74,7 +74,8 @@ int cov_block_stats(const double* d_blocks, const int* d_cols, int k, long long 
     long long lastOff = 0; int lastCnt = 0;
     cudaMemcpyAsync(&lastOff, d_off + (N - 1), sizeof(long long), cudaMemcpyDeviceToHost, st);
     cudaMemcpyAsync(&lastCnt, d_cnt + (N - 1), sizeof(int), cudaMemcpyDeviceToHost, st);
-    cudaError_t e = cudaStreamSynchronize(st);
+    cudaError_t e = cudaGetLastError();                 // launch errors (of these and the caller's earlier kernels)
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     if (e == cudaSuccess) {
         *nHits = lastOff + lastCnt;
         const long long m = *nHits < cap ? *nHits : cap;
