@@ -57,7 +57,7 @@ class Result(C.Structure):
 EXPORTS = ['dbat_create', 'dbat_destroy', 'dbat_last_error', 'dbat_num_unknowns',
            'dbat_num_residuals', 'dbat_eval', 'dbat_jacobian_nnz', 'dbat_jacobian_csc',
            'dbat_default_opts', 'dbat_solve', 'dbat_normal_step', 'dbat_cov', 'dbat_cov_stats',
-           'dbat_comm_unique_id', 'dbat_comm_init', 'dbat_phase_times', 'dbat_dense_chol_solve',
+           'dbat_comm_unique_id', 'dbat_comm_init', 'dbat_phase_times', 'dbat_dense_chol_inverse',
            'dbat_forwintersect', 'dbat_forwintersect_error', 'dbat_resect3', 'dbat_camera_order',
            'dbat_tile_symbolic', 'dbat_tile_symbolic_get', 'dbat_tile_symbolic_get2', 'dbat_tile_symbolic_coords',
            'dbat_tile_chol_solve',
@@ -129,8 +129,8 @@ def lib():
     L.dbat_comm_init.restype = C.c_int
     L.dbat_phase_times.argtypes = [vp, C.POINTER(C.c_char_p), c_dp, c_ip, C.c_int]
     L.dbat_phase_times.restype = C.c_int
-    L.dbat_dense_chol_solve.argtypes = [C.c_int64, c_dp, c_dp, c_dp, c_dp, C.c_int, c_dp]
-    L.dbat_dense_chol_solve.restype = C.c_int
+    L.dbat_dense_chol_inverse.argtypes = [C.c_int64, c_dp, c_dp, C.c_int, c_dp]
+    L.dbat_dense_chol_inverse.restype = C.c_int
     L.dbat_forwintersect.argtypes = [C.POINTER(FwiDesc), c_dp, c_dp, c_dp]
     L.dbat_forwintersect.restype = C.c_int
     L.dbat_forwintersect_error.argtypes = []
@@ -180,19 +180,17 @@ class DbatError(RuntimeError):
         self.code = code
 
 
-def dense_chol_solve(A, b, want_inverse=False, repeat=1):
-    """x = A^-1 b (and optionally A^-1) on the device; returns (x, Ainv or None, ms)."""
+def dense_chol_inverse(A, repeat=1):
+    """A^-1 through the dense factor + inverse of dbat_cov on the device; returns (Ainv, ms), ms the best device time
+    of `repeat` passes."""
     A = np.asfortranarray(np.asarray(A, dtype=np.float64))
     n = A.shape[0]
-    b = f64(b)
-    x = np.empty(n)
-    Ainv = np.empty((n, n), order='F') if want_inverse else None
+    Ainv = np.empty((n, n), order='F')
     ms = C.c_double()
-    rc = lib().dbat_dense_chol_solve(n, A.ctypes.data_as(c_dp), dptr(b), dptr(x),
-                                     Ainv.ctypes.data_as(c_dp) if want_inverse else None, repeat, C.byref(ms))
+    rc = lib().dbat_dense_chol_inverse(n, A.ctypes.data_as(c_dp), Ainv.ctypes.data_as(c_dp), repeat, C.byref(ms))
     if rc != 0:
         raise DbatError(rc, lib().dbat_last_error(None).decode())
-    return x, Ainv, ms.value
+    return Ainv, ms.value
 
 
 def camera_order(img, op, nImg, nOP):

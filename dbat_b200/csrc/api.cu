@@ -1378,8 +1378,9 @@ static int cov_factor(dbat_handle* h, double** Zp, double** Cp, int* ldp, int* i
     double *Sd = nullptr, *Z = nullptr, *C = nullptr;
     const size_t sz = sizeof(double) * (size_t)ldd * ldd;
     int* d_bad = nullptr;
+    CholWork cw;
     if (cudaMalloc(&Sd, sz) != cudaSuccess || cudaMalloc(&Z, sz) != cudaSuccess || cudaMalloc(&C, sz) != cudaSuccess ||
-        cudaMalloc(&d_bad, sizeof(int)) != cudaSuccess) {
+        cudaMalloc(&d_bad, sizeof(int)) != cudaSuccess || chol_alloc(cw, ldd)) {
         cudaFree(Sd); cudaFree(Z); cudaFree(C); cudaFree(d_bad);
         h->err = "out of memory for the covariance workspace"; return DBAT_E_OOM;
     }
@@ -1391,14 +1392,10 @@ static int cov_factor(dbat_handle* h, double** Zp, double** Cp, int* ldp, int* i
     // factorisation of the full normal matrix fail (bundle_cov.m:87-107): report that, not huge numbers
     if (P.nOP > 0) k_point_pd_check<<<(P.nOP + 255) / 256, 256, 0, h->st>>>(P, d_bad);
     count_launch(2);
-    // a failed launch leaves no trace a stream synchronisation reports: ask for it (before chol_factor, whose
-    // fall-back from graph capture clears the error state)
-    cudaError_t le = cudaGetLastError();
-    CholWork cw;
-    chol_alloc(cw, P.ldS - 1, ldd);
     chol_factor(cw, Sd, h->st);
     chol_inverse(cw, Sd, Z, C, h->st);
-    if (le == cudaSuccess) le = cudaGetLastError();
+    // a failed launch leaves no trace a stream synchronisation reports: ask for it
+    const cudaError_t le = cudaGetLastError();
     int info = 0, badPts = 0;
     cudaMemcpyAsync(&info, cw.info, sizeof(int), cudaMemcpyDeviceToHost, h->st);
     cudaMemcpyAsync(&badPts, d_bad, sizeof(int), cudaMemcpyDeviceToHost, h->st);
@@ -1649,67 +1646,46 @@ __global__ void __launch_bounds__(128) k_cop(DevProblem P, const double* __restr
 }
 
 // --------------------------------------------------------------------------------------------
-// stand-alone access to the dense solver (unit tests, profiling)
+// stand-alone access to the dense factor + inverse of the covariances (unit tests, profiling)
 // --------------------------------------------------------------------------------------------
-extern "C" int dbat_dense_chol_solve(int64_t n, const double* A, const double* b, double* x, double* Ainv,
-                                     int repeat, double* ms_out) {
-    if (n <= 0 || !A || !b || !x) return DBAT_E_BADARG;
+extern "C" int dbat_dense_chol_inverse(int64_t n, const double* A, double* Ainv, int repeat, double* ms_out) {
+    if (n <= 0 || !A || !Ainv) return DBAT_E_BADARG;
+    // the layout cov_factor factors: room for the rhs row of S, identity padding
     const int ld = std::max(128, (int)((n + 1 + 127) / 128) * 128);
-    double *dA = nullptr, *dA0 = nullptr, *drhs = nullptr, *dx = nullptr, *Z = nullptr, *Cc = nullptr;
     const size_t sz = sizeof(double) * (size_t)ld * ld;
-    std::vector<double> hA((size_t)ld * ld, 0.0), hb(ld, 0.0);
+    std::vector<double> hA((size_t)ld * ld, 0.0);
     for (int64_t c = 0; c < n; ++c) for (int64_t r = 0; r < n; ++r) hA[(size_t)c * ld + r] = A[(size_t)c * n + r];
     for (int64_t k = n; k < ld; ++k) hA[(size_t)k * ld + k] = 1.0;
-    for (int64_t k = 0; k < n; ++k) hb[k] = b[k];
-    if (cudaMalloc(&dA, sz) || cudaMalloc(&dA0, sz) || cudaMalloc(&drhs, sizeof(double) * ld) || cudaMalloc(&dx, sizeof(double) * ld)) {
-        g_create_err = "dbat_dense_chol_solve: out of memory"; return DBAT_E_OOM;
+    double *dA0 = nullptr, *dA = nullptr, *Z = nullptr, *Cc = nullptr;
+    CholWork w;
+    cudaGetLastError();                      // a launch error reported by this call is one of its own launches
+    if (cudaMalloc(&dA0, sz) || cudaMalloc(&dA, sz) || cudaMalloc(&Z, sz) || cudaMalloc(&Cc, sz) || chol_alloc(w, ld)) {
+        cudaFree(dA0); cudaFree(dA); cudaFree(Z); cudaFree(Cc);
+        g_create_err = "dbat_dense_chol_inverse: out of memory"; return DBAT_E_OOM;
     }
     cudaMemcpy(dA0, hA.data(), sz, cudaMemcpyHostToDevice);
-    cudaMemcpy(drhs, hb.data(), sizeof(double) * ld, cudaMemcpyHostToDevice);
-    CholWork w; chol_alloc(w, (int)n, ld);
     cudaStream_t st; cudaStreamCreate(&st);
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
     float best = 1e30f;
     for (int it = 0; it < std::max(1, repeat); ++it) {
         cudaMemcpyAsync(dA, dA0, sz, cudaMemcpyDeviceToDevice, st);
         cudaEventRecord(e0, st);
-        chol_put_rhs(w, dA, drhs, st);
         chol_factor(w, dA, st);
-        chol_solve(w, dA, dx, st);
+        chol_inverse(w, dA, Z, Cc, st);
         cudaEventRecord(e1, st);
         cudaStreamSynchronize(st);
         float ms = 0; cudaEventElapsedTime(&ms, e0, e1); best = std::min(best, ms);
     }
     int info = 0;
     cudaMemcpy(&info, w.info, sizeof(int), cudaMemcpyDeviceToHost);
-    cudaMemcpy(hb.data(), dx, sizeof(double) * ld, cudaMemcpyDeviceToHost);
-    for (int64_t k = 0; k < n; ++k) x[k] = hb[k];
-    if (Ainv) {
-        // the inverse needs the plain factor (no rhs row)
-        cudaMemcpyAsync(dA, dA0, sz, cudaMemcpyDeviceToDevice, st);
-        chol_factor(w, dA, st);
-        if (cudaMalloc(&Z, sz) || cudaMalloc(&Cc, sz)) { g_create_err = "out of memory"; return DBAT_E_OOM; }
-        chol_inverse(w, dA, Z, Cc, st);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(hA.data(), Cc, sz, cudaMemcpyDeviceToHost);
-        for (int64_t c = 0; c < n; ++c) for (int64_t r = 0; r < n; ++r) Ainv[(size_t)c * n + r] = hA[(size_t)c * ld + r];
-        cudaFree(Z); cudaFree(Cc);
-    }
+    cudaMemcpy(hA.data(), Cc, sz, cudaMemcpyDeviceToHost);
+    for (int64_t c = 0; c < n; ++c) for (int64_t r = 0; r < n; ++r) Ainv[(size_t)c * n + r] = hA[(size_t)c * ld + r];
     if (ms_out) *ms_out = best;
-#ifdef POTRF_PROFILE
-    {   // per warp, per panel: [end of D / W] [after S1] [end of R] [after S2], then the end of the tail
-        double pr[16 + 16 * 40]; cudaMemcpy(pr, w.minmax, sizeof(pr), cudaMemcpyDeviceToHost);
-        for (int wp = 0; wp < 16; ++wp) {
-            printf("potrf trace warp %d:", wp);
-            for (int k = 0; k < 33; ++k) printf(" %.0f", pr[16 + wp * 40 + k]);
-            printf("\n");
-        }
-    }
-#endif
     cudaError_t e = cudaDeviceSynchronize();
-    chol_free(w); cudaFree(dA); cudaFree(dA0); cudaFree(drhs); cudaFree(dx);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    chol_free(w); cudaFree(dA0); cudaFree(dA); cudaFree(Z); cudaFree(Cc);
     cudaEventDestroy(e0); cudaEventDestroy(e1); cudaStreamDestroy(st);
-    if (e != cudaSuccess) { g_create_err = std::string("dbat_dense_chol_solve: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
+    if (e != cudaSuccess) { g_create_err = std::string("dbat_dense_chol_inverse: ") + cudaGetErrorString(e); return DBAT_E_CUDA; }
     return info != 0 ? DBAT_E_NOTSPD : DBAT_OK;
 }
 

@@ -56,23 +56,14 @@ void launch_io_diag_grad_gen(const DevProblem& P, const double* camDiag, const d
 
 // chol.cu
 struct CholWork {
-    int n = 0, ld = 0, nb = 0;      // order, leading dimension (multiple of 128), # 128-blocks
+    int ld = 0, nb = 0;             // leading dimension (multiple of 128), # 128-blocks
     double* invL = nullptr;         // nb x 128 x 128 inverses of the diagonal blocks
-    int* info = nullptr;            // device flag: 0 ok, k>0 = first non-positive pivot (1-based)
-    double* minmax = nullptr;       // device: [0]=min pivot, [1]=max pivot (of L's diagonal)
-    void* graphExec = nullptr;      // captured launch sequence of chol_factor (cudaGraphExec_t)
-    const double* graphA = nullptr; const double* seen = nullptr; cudaStream_t graphStream = nullptr;
-    int graphLaunches = 0;
+    int* info = nullptr;            // device flag: 0 ok, k > 0: block k - 1 holds the first non-positive pivot
 };
-void chol_alloc(CholWork& w, int n, int ld);
+int chol_alloc(CholWork& w, int ld);          // 0 ok, 1 out of memory (nothing left allocated)
 void chol_free(CholWork& w);
-// In-place lower Cholesky of the ld x ld column-major matrix A (rows/cols >= n are padding and
-// must hold the identity).  Asynchronous; read w.info afterwards.
-void chol_factor(CholWork& w, double* A, cudaStream_t st);
-// Store rhs' in the last padding row of A (before chol_factor): the forward substitution then
-// happens inside the factorisation.  Requires ld > n.
-void chol_put_rhs(const CholWork& w, double* A, const double* rhs, cudaStream_t st);
-// After chol_factor on a matrix prepared with chol_put_rhs: x (length ld) = A^-1 rhs.
-void chol_solve(const CholWork& w, const double* A, double* x, cudaStream_t st);
-// Z = inv(L) (lower) into Zout (ld x ld); then C = Z'Z (= inv(A)) full symmetric into Cout.
+// In-place lower Cholesky of the ld x ld column-major matrix A (rows/cols past the order of the
+// matrix are padding and must hold the identity).  Asynchronous; read w.info afterwards.
+void chol_factor(const CholWork& w, double* A, cudaStream_t st);
+// After chol_factor: Z (ld x ld) = inv(L)', C (ld x ld) = inv(A), full symmetric.
 void chol_inverse(const CholWork& w, const double* A, double* Z, double* C, cudaStream_t st);

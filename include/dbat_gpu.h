@@ -222,12 +222,11 @@ int dbat_tile_symbolic_coords(int64_t nImg, const double *xyz);
 int dbat_tile_chol_solve(int64_t n, const double *A, const double *b, double *x, int64_t mode, int64_t leafImages,
                          int repeat, double *stats);
 
-/* The dense solver on its own (unit tests / profiling): x = A^-1 b for a symmetric positive
- * definite column-major n x n matrix through the same blocked FP64 Cholesky the reduced camera
- * system uses; Ainv (n x n, may be NULL) receives the explicit inverse used by dbat_cov.
- * ms_out: best device time of `repeat` factor+solve passes (CUDA events). */
-int dbat_dense_chol_solve(int64_t n, const double *A, const double *b, double *x, double *Ainv,
-                          int repeat, double *ms_out);
+/* The dense inverse on its own (unit tests / profiling): Ainv (n x n) = A^-1 for a symmetric
+ * positive definite column-major n x n matrix, through the blocked FP64 Cholesky and explicit
+ * inverse dbat_cov runs on the reduced camera system.  DBAT_E_NOTSPD if a pivot is not positive.
+ * ms_out (may be NULL): best device time of `repeat` factor+inverse passes (CUDA events). */
+int dbat_dense_chol_inverse(int64_t n, const double *A, double *Ainv, int repeat, double *ms_out);
 
 /* One process, several devices (SURVEY §8b; a MEX gateway has one interpreter thread): after dbat_create and before
  * the first evaluation, turn the handle into the front of `ndev` sub-problems, one per listed CUDA device.  The object

@@ -175,23 +175,23 @@ def _spd(n, family, rng):
 
 
 @pytest.mark.parametrize('family', ['mmt', 'unitdiag-1e8'])
-@pytest.mark.parametrize('n', [1, 2, 127, 128, 129, 255, 256, 511, 512, 513, 1000, 6001])
-def test_dense_inverse(n, family):
-    """chol_factor + chol_solve + chol_inverse on their own at every padding situation of the last block (rhs row
-    with no padding at n = 127, a full padding block at n = 128, ...), below and above the 4 blocks where the
-    factorisation is replayed from a captured graph, and at the size of BASELINE config 4's reduced system."""
+@pytest.mark.parametrize('n', [1, 2, 100, 127, 128, 129, 255, 256, 511, 512, 513, 700, 1000, 6001])
+def test_dense_chol_inverse(n, family):
+    """chol_factor + chol_inverse on their own at every padding situation of the last block (rhs row with no padding
+    at n = 127, a full padding block at n = 128, ...), from one block to the size of BASELINE config 4's reduced
+    system."""
     rng = np.random.default_rng(1000 + n)
     A, cond = _spd(n, family, rng)
-    b = rng.standard_normal(n)
     bound = 64 * np.sqrt(n) * cond * EPS
-    x, Ai, _ = dlib.dense_chol_solve(A, b, want_inverse=True, repeat=1)
-    xr = sla.cho_solve(sla.cho_factor(A, lower=True), b)
-    assert np.linalg.norm(x - xr) <= bound * np.linalg.norm(xr), np.linalg.norm(x - xr) / np.linalg.norm(xr) / (cond * EPS)
+    Ai, _ = dlib.dense_chol_inverse(A, repeat=1)
     Ar = sla.inv(A)
     err = np.max(np.abs(Ai - Ar)) / np.max(np.abs(Ar))
     assert err <= bound, err / (cond * EPS)
-    x3, Ai3, _ = dlib.dense_chol_solve(A, b, want_inverse=True, repeat=3)    # the graph replay of chol_factor
-    assert np.array_equal(x3, x) and np.array_equal(Ai3, Ai)
+    Ai3, _ = dlib.dense_chol_inverse(A, repeat=3)
+    assert np.array_equal(Ai3, Ai)
+    # the first pivot not positive
+    with pytest.raises(dlib.DbatError):
+        dlib.dense_chol_inverse(A - 2 * A[0, 0] * np.eye(n))
     # only the last pivot (index n - 1) not positive
     Ab = A.copy()
     if n == 1:
@@ -200,7 +200,7 @@ def test_dense_inverse(n, family):
         a = A[:n - 1, n - 1]
         Ab[n - 1, n - 1] = a @ sla.cho_solve(sla.cho_factor(A[:n - 1, :n - 1], lower=True), a) - 1e-3 * A[n - 1, n - 1]
     with pytest.raises(dlib.DbatError):
-        dlib.dense_chol_solve(Ab, b)
+        dlib.dense_chol_inverse(Ab)
 
 
 # --------------------------------------------------------------------------------------------- block-path scenes
@@ -320,9 +320,9 @@ EDGES = {
 
 @pytest.mark.parametrize('edge', list(EDGES))
 def test_block_edges_of_the_dense_copy(edge):
-    """The padding and rhs-row handling of cov_factor (k_dense_unit_diag, chol_alloc(ldS - 1, ldd)) where the rhs
-    row ld - 1 is the dense matrix's last row, where 64 padding rows follow it, and where no tile padding sits
-    between the last unknown and the rhs row: CEO / COP / CXX against the dense oracle."""
+    """The padding and rhs-row handling of cov_factor (k_dense_unit_diag, chol_factor at ldd = ld rounded up to 128)
+    where the rhs row ld - 1 is the dense matrix's last row, where 64 padding rows follow it, and where no tile padding
+    sits between the last unknown and the rhs row: CEO / COP / CXX against the dense oracle."""
     nImg, nIO, want = EDGES[edge]
     s = _edge_scene(nImg, nIO)
     x0 = serialize(s)

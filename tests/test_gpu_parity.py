@@ -495,23 +495,6 @@ def test_full_size_step_against_the_oracle():
     P.close()
 
 
-@pytest.mark.parametrize('n', [100, 129, 700])
-def test_dense_cholesky_solver(n):
-    """The reduced-system solver on its own: blocked DMMA Cholesky, folded forward
-    substitution, backward solve and explicit inverse against LAPACK."""
-    from dbat_b200 import _lib
-    rng = np.random.default_rng(n)
-    M = rng.standard_normal((n, n + 8))
-    A = M @ M.T + 0.5 * n * np.eye(n)
-    b = rng.standard_normal(n)
-    x, Ai, _ = _lib.dense_chol_solve(A, b, want_inverse=True)
-    np.testing.assert_allclose(x, np.linalg.solve(A, b), rtol=1e-10, atol=1e-13)
-    Ar = np.linalg.inv(A)
-    assert relmax(Ai, Ar) < 1e-10
-    with pytest.raises(_lib.DbatError):
-        _lib.dense_chol_solve(A - 2 * n * np.eye(n), b)        # not positive definite
-
-
 def _banded_arrow_spd(n, bw, border, rng, blocks=None):
     """SPD test matrix with the structure of a reduced camera system: a band (or the given list of coupled
     6-column block pairs), `border` dense rows at the end, diagonally dominant."""
