@@ -58,9 +58,8 @@ EXPORTS = ['dbat_create', 'dbat_destroy', 'dbat_last_error', 'dbat_num_unknowns'
            'dbat_num_residuals', 'dbat_eval', 'dbat_jacobian_nnz', 'dbat_jacobian_csc',
            'dbat_default_opts', 'dbat_solve', 'dbat_normal_step', 'dbat_cov', 'dbat_cov_stats',
            'dbat_comm_unique_id', 'dbat_comm_init', 'dbat_phase_times', 'dbat_dense_chol_inverse',
-           'dbat_forwintersect', 'dbat_forwintersect_error', 'dbat_resect3', 'dbat_camera_order',
-           'dbat_tile_symbolic', 'dbat_tile_symbolic_get', 'dbat_tile_symbolic_get2', 'dbat_tile_symbolic_coords',
-           'dbat_tile_chol_solve',
+           'dbat_forwintersect', 'dbat_forwintersect_error', 'dbat_resect3',
+           'dbat_tile_symbolic', 'dbat_tile_symbolic_get', 'dbat_tile_symbolic_get2', 'dbat_tile_chol_solve',
            'dbat_reduced_info', 'dbat_set_devices']
 
 _lib = None
@@ -137,8 +136,6 @@ def lib():
     L.dbat_forwintersect_error.restype = C.c_char_p
     L.dbat_resect3.argtypes = [C.POINTER(ResectDesc), c_dp, c_dp]
     L.dbat_resect3.restype = C.c_int
-    L.dbat_camera_order.argtypes = [C.c_int64, C.c_int64, C.c_int64, c_ip, c_ip, c_ip, C.POINTER(C.c_int64)]
-    L.dbat_camera_order.restype = C.c_int
     L.dbat_set_devices.argtypes = [vp, C.POINTER(C.c_int), C.c_int]
     L.dbat_set_devices.restype = C.c_int
     L.dbat_reduced_info.argtypes = [vp, c_ip]
@@ -148,8 +145,6 @@ def lib():
     L.dbat_tile_symbolic.restype = C.c_int
     L.dbat_tile_symbolic_get.argtypes = [c_ip] * 8
     L.dbat_tile_symbolic_get.restype = C.c_int
-    L.dbat_tile_symbolic_coords.argtypes = [C.c_int64, c_dp]
-    L.dbat_tile_symbolic_coords.restype = C.c_int
     L.dbat_tile_symbolic_get2.argtypes = [c_ip] * 3
     L.dbat_tile_symbolic_get2.restype = C.c_int
     L.dbat_tile_chol_solve.argtypes = [C.c_int64, c_dp, c_dp, c_dp, C.c_int64, C.c_int64, C.c_int, c_dp]
@@ -193,29 +188,12 @@ def dense_chol_inverse(A, repeat=1):
     return Ainv, ms.value
 
 
-def camera_order(img, op, nImg, nOP):
-    """Reverse Cuthill-McKee order of the images on the co-visibility graph (host code in the library):
-    returns (perm, bandwidth) with perm 0-based."""
-    img1, op1 = i64(np.asarray(img) + 1), i64(np.asarray(op) + 1)
-    perm = np.empty(nImg, dtype=np.int64)
-    bw = C.c_int64()
-    rc = lib().dbat_camera_order(nImg, nOP, len(img1), iptr(img1), iptr(op1), iptr(perm), C.byref(bw))
-    if rc != 0:
-        raise DbatError(rc, 'dbat_camera_order: bad argument')
-    return perm - 1, int(bw.value)
-
-
-def tile_symbolic(img, op, nImg, nOP, nEO, nIO, mode=-1, leaf=120, parts=1, part=0, xyz=None):
+def tile_symbolic(img, op, nImg, nOP, nEO, nIO, mode=-1, leaf=120, parts=1, part=0):
     """Symbolic analysis of the reduced camera system (host code in the library): dict of counts + arrays.
     parts / part: task lists of one part of a distributed factorisation."""
     img1, op1, ne = i64(np.asarray(img) + 1), i64(np.asarray(op) + 1), i64(nEO)
     cnt = np.zeros(16, dtype=np.int64)
     cnt[14], cnt[15] = parts, part
-    if xyz is not None:
-        c = np.ascontiguousarray(np.asarray(xyz, dtype=np.float64).T)      # 3 x nImg column-major = nImg x 3 C order
-        lib().dbat_tile_symbolic_coords(nImg, dptr(c))
-    else:
-        lib().dbat_tile_symbolic_coords(0, None)
     rc = lib().dbat_tile_symbolic(nImg, nOP, len(img1), iptr(img1), iptr(op1), iptr(ne), nIO, mode, leaf, iptr(cnt))
     if rc != 0:
         raise DbatError(rc, 'dbat_tile_symbolic failed')

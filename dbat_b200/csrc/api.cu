@@ -190,7 +190,7 @@ static thread_local bool g_in_group_create = false;
 static int analyse_reduced(dbat_handle* h, int nParts, int myPart, TileSym& sym) {
     const ProblemPlan& pl = h->plan;
     if (tile_symbolic(pl.nImg, pl.adjPtr.data(), pl.adj.data(), pl.nEO.data(), (int)pl.glob_x.size(), -1, 120, sym, nParts,
-                      myPart, pl.xyz.data())) {
+                      myPart)) {
         h->err = "symbolic analysis of the reduced system failed"; return DBAT_E_STATE;
     }
     return 0;
@@ -227,9 +227,9 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail_create(nullptr, DBAT_E_CUDA, "no CUDA device available (libdbatgpu has no CPU fallback)");
     dbat_handle* h = new dbat_handle();
-    PlanOpts opts{DBAT_GRP_MAXM, getenv("DBAT_EVAL_GENERIC") != nullptr};
-    // DBAT_GRP_MAXM=k lowers the threshold (tests of the per-point path)
-    if (const char* e = getenv("DBAT_GRP_MAXM")) opts.grpMaxM = std::max(1, std::min(DBAT_GRP_MAXM, atoi(e)));
+    // points with more than grpMaxM rays go to k_schur_atomic; DBAT_GRP_MAXM=k lowers it (tests of the per-point path)
+    int grpMaxM = DBAT_GRP_MAXM;
+    if (const char* e = getenv("DBAT_GRP_MAXM")) grpMaxM = std::max(1, std::min(DBAT_GRP_MAXM, atoi(e)));
 
     // ---- host side: the plan (plan.cu) and the symbolic analysis of the reduced system
     ProblemPlan& pl = h->plan;
@@ -242,7 +242,7 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     if (rc) return fail_create(h, rc, msg);
     if ((rc = analyse_reduced(h, 1, 0, sym))) return fail_create(h, rc, h->err);
     plan_point_blocks(pl, up);
-    plan_schur_windows(pl, up, sym, opts);
+    plan_schur_windows(pl, up, sym, grpMaxM);
 
     // ---- device side
     DevProblem& P = h->P;
@@ -251,7 +251,7 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     P.model = pl.legacy ? (d->distModel == 1 ? 0 : 4) : d->distModel - 2;
     P.n = pl.n; P.nC = pl.nC; P.nChunks = (int)up.chunks.size(); P.nPrior = (int)pl.prior_col.size();
     P.ioGeneral = pl.general ? 1 : 0;
-    P.evalCompact = plan_eval_compact(pl, d->nK, d->nP, opts) ? 1 : 0;
+    P.evalCompact = plan_eval_compact(pl, d->nK, d->nP) ? 1 : 0;
     P.nPsb = up.nPsb; P.nPsbig = up.nPsbig;
     P.nCand = up.nCand; P.nBig = up.nBig; P.grpMaxRays = up.grpMaxRays; P.nClu = up.nClu; P.nRedBlk = up.nRedBlk;
     if (cudaStreamCreate(&h->st) != cudaSuccess || cudaStreamCreateWithFlags(&h->st2, cudaStreamNonBlocking) != cudaSuccess ||
@@ -927,8 +927,6 @@ static bool structurally_deficient(dbat_handle* h) {
         for (int a = 0; a < 6; ++a) { const int c = h->plan.eo_col[6 * (size_t)i + a]; if (c >= 0) { ++freec; pri += priorCnt[c]; } }
         if (freec && 2 * (h->plan.img_start[i + 1] - h->plan.img_start[i]) + pri < freec) return true;
     }
-    static const bool skipExact = getenv("DBAT_NO_SPRANK") != nullptr;
-    if (skipExact) return false;
     return matching_deficient(h);          // exact at any size: 8 bytes per observation cross the bus
 }
 

@@ -211,8 +211,6 @@ int plan_cameras(const dbat_problem_desc* d, ProblemPlan& p, const PlanUpload& u
         }
         adjPtr[nImg] = (int64_t)adj.size();
     }
-    p.xyz.resize((size_t)3 * nImg);
-    for (int i = 0; i < nImg; ++i) for (int a = 0; a < 3; ++a) p.xyz[3 * (size_t)i + a] = d->EOval[6 * (size_t)i + a];
     p.nEO.assign(nImg, 0);
     for (int i = 0; i < nImg; ++i) for (int a = 0; a < 6; ++a) if (p.eo_col[(size_t)i * 6 + a] >= 0) p.nEO[i]++;
     // IO columns: used by one image -> they travel with that image (like its EO elements); used by several ->
@@ -281,19 +279,18 @@ void plan_point_blocks(const ProblemPlan& p, PlanUpload& u) {
     if (bigp.empty()) bigp.push_back(0);
 }
 
-void plan_schur_windows(ProblemPlan& p, PlanUpload& u, const TileSym& sym, const PlanOpts& opts) {
+void plan_schur_windows(ProblemPlan& p, PlanUpload& u, const TileSym& sym, int grpMaxM) {
     const int nImg = p.nImg, nOP = p.nOP, nObs = p.nObs;
     const std::vector<int>& imgRank = sym.imgRank;
     const std::vector<int>& img_pm = u.img_pm;
     // grouped Schur index: estimated points sorted by (ray count, image list)
     std::vector<int>& cand = u.grp_pt; std::vector<int>& big = u.big_pt;
     cand.reserve(nOP);
-    const int maxm = opts.grpMaxM;
     for (int j = 0; j < nOP; ++j) {
         const int k = p.pt_start[j + 1] - p.pt_start[j];
         const int* oc = &p.op_col[3 * (size_t)j];
         if (k == 0 || (oc[0] < 0 && oc[1] < 0 && oc[2] < 0)) continue;
-        (k <= maxm ? cand : big).push_back(j);
+        (k <= grpMaxM ? cand : big).push_back(j);
     }
     const int* ps = p.pt_start.data();
     // image lists in elimination-order rank (ascending inside a point): the union of a group is then
@@ -449,9 +446,9 @@ bool plan_same_order(const ProblemPlan& p, const TileSym& a, const TileSym& b) {
     return oa == ob;
 }
 
-bool plan_eval_compact(const ProblemPlan& p, int nK, int nP, const PlanOpts& opts) {
+bool plan_eval_compact(const ProblemPlan& p, int nK, int nP) {
     // one shared IO block whose estimated slots all lie in f, pp, b1, K1-K3, P1-P2
-    bool ok = !p.general && nK <= 3 && nP <= 2 && !opts.evalGeneric;
+    bool ok = !p.general && nK <= 3 && nP <= 2;
     for (int sl = 0; sl < DBAT_NSLOT; ++sl) if (p.sh_col[sl] >= 0 && !((0x0CEFu >> sl) & 1)) ok = false;
     return ok;
 }

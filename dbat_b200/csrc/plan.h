@@ -10,12 +10,6 @@
 #include "kernels.cuh"
 #include "tilesym.h"
 
-// settings dbat_create reads from the environment once
-struct PlanOpts {
-    int grpMaxM;          // points with more rays go to k_schur_atomic (DBAT_GRP_MAXM, at most the compiled limit)
-    bool evalGeneric;     // never select the compact evaluation kernels (DBAT_EVAL_GENERIC)
-};
-
 // What the handle keeps on the host for the life of the problem: Jacobian export, rank tests, covariance layout
 // and the re-tiling for several ranks or devices.
 struct ProblemPlan {
@@ -45,11 +39,10 @@ struct ProblemPlan {
     // prior observations
     std::vector<int> prior_col;
     std::vector<double> prior_isig;
-    // reduced system: co-visibility graph (CSR), station coordinates (3 x nImg) and the columns every image has in S
-    // (EO elements and the IO columns only it uses)
+    // reduced system: co-visibility graph (CSR) and the columns every image has in S (EO elements and the IO
+    // columns only it uses)
     std::vector<int64_t> adjPtr;
     std::vector<int32_t> adj;
-    std::vector<double> xyz;
     std::vector<int> nEO;
 };
 
@@ -92,18 +85,19 @@ int plan_columns(const dbat_problem_desc* d, ProblemPlan& p, std::string& err);
 void plan_observations(const dbat_problem_desc* d, ProblemPlan& p, PlanUpload& u);
 // prior observations, m, col2pt
 int plan_priors(const dbat_problem_desc* d, ProblemPlan& p, PlanUpload& u, std::string& err);
-// co-visibility graph (with the description's covis edges), station coordinates, S columns per image, global IO
+// co-visibility graph (with the description's covis edges), S columns per image, global IO
 int plan_cameras(const dbat_problem_desc* d, ProblemPlan& p, const PlanUpload& u, std::string& err);
 // runs of whole points for the point-side assembly and the list of long points
 void plan_point_blocks(const ProblemPlan& p, PlanUpload& u);
-// window Schur index for the elimination order of sym: groups, clusters, headers, reduction CSR, cluster order
-void plan_schur_windows(ProblemPlan& p, PlanUpload& u, const TileSym& sym, const PlanOpts& opts);
+// window Schur index for the elimination order of sym: groups, clusters, headers, reduction CSR, cluster order;
+// estimated points with more than grpMaxM rays go to k_schur_atomic instead
+void plan_schur_windows(ProblemPlan& p, PlanUpload& u, const TileSym& sym, int grpMaxM);
 // sets p.x2s and returns the other S index maps
 ReducedMaps plan_reduced_maps(ProblemPlan& p, const TileSym& sym);
 
 // true when the images with columns in S come in the same elimination order in a and b
 bool plan_same_order(const ProblemPlan& p, const TileSym& a, const TileSym& b);
 // the compact evaluation kernels (eval.cu) apply
-bool plan_eval_compact(const ProblemPlan& p, int nK, int nP, const PlanOpts& opts);
+bool plan_eval_compact(const ProblemPlan& p, int nK, int nP);
 // doubles of the block-partials buffer of the reductions
 int plan_partials(const ProblemPlan& p, const PlanUpload& u);

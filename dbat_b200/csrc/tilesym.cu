@@ -3,7 +3,6 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
-#include <cstring>
 #include <numeric>
 #include <vector>
 
@@ -96,52 +95,7 @@ struct Orderer {
     std::vector<std::vector<int>> segs;       // elimination order as a list of segments
     std::vector<int> segOwner;                // owning part of every segment, -1 = above the cut ("top")
     int cutDepth = 0;                         // the tree is cut into 2^cutDepth parts
-    const double* xyz = nullptr;              // optional 3 x n station coordinates: geometric bisection
     Orderer(const Graph& gg, int lf) : g(gg), leaf(lf), mark(gg.n, 0), level(gg.n, -1) {}
-
-    // Geometric bisection of a component: cut at the median of the coordinate with the largest extent; the
-    // separator is the smaller of the two boundary layers (the nodes of one side with a neighbour on the other).
-    // Straight cuts through a photogrammetric block are shorter than the level sets of a breadth-first search
-    // (which run diagonally through a square block), and the cost of a separator grows with its cube.
-    bool geometric_split(const std::vector<int>& comp, int ctag, std::vector<int>& A, std::vector<int>& B,
-                         std::vector<int>& S) {
-        if (!xyz || comp.size() < 8) return false;
-        double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
-        for (int v : comp) for (int a = 0; a < 3; ++a) { lo[a] = std::min(lo[a], xyz[3 * (size_t)v + a]); hi[a] = std::max(hi[a], xyz[3 * (size_t)v + a]); }
-        size_t bestSep = (size_t)-1;
-        std::vector<int> sorted(comp), side(g.n, 0), cand;
-        int axes[3] = {0, 1, 2};
-        std::sort(axes, axes + 3, [&](int p, int q) { return hi[p] - lo[p] > hi[q] - lo[q]; });
-        for (int t = 0; t < 2; ++t) {                       // the two longest axes
-            const int ax = axes[t];
-            if (!(hi[ax] - lo[ax] > 0.35 * (hi[axes[0]] - lo[axes[0]]))) break;      // do not cut a strip lengthwise
-            std::sort(sorted.begin(), sorted.end(), [&](int p, int q) {
-                const double a = xyz[3 * (size_t)p + ax], b = xyz[3 * (size_t)q + ax];
-                return a != b ? a < b : p < q;
-            });
-            const size_t half = sorted.size() / 2;
-            for (size_t k = 0; k < sorted.size(); ++k) side[sorted[k]] = k < half ? 1 : 2;
-            std::vector<int> sa, sb;
-            for (int v : sorted) {
-                bool touch = false;
-                for (int64_t k = g.ptr[v]; k < g.ptr[v + 1] && !touch; ++k) {
-                    const int u = g.adj[k];
-                    if (mark[u] == ctag && side[u] != side[v]) touch = true;
-                }
-                if (touch) (side[v] == 1 ? sa : sb).push_back(v);
-            }
-            const std::vector<int>& sep = sa.size() <= sb.size() ? sa : sb;
-            if (sep.empty() || sep.size() >= bestSep) continue;
-            bestSep = sep.size();
-            const int sepSide = sa.size() <= sb.size() ? 1 : 2;
-            std::vector<char> inSep(g.n, 0);
-            for (int v : sep) inSep[v] = 1;
-            A.clear(); B.clear(); S.assign(sep.begin(), sep.end());
-            for (int v : sorted) { if (inSep[v]) continue; (side[v] == 1 ? A : B).push_back(v); }
-            (void)sepSide;
-        }
-        return bestSep != (size_t)-1 && !A.empty() && !B.empty() && S.size() * 3 < comp.size();
-    }
 
     // nodes: a node set (all currently marked with `tag`); nd = dissect, else one RCM segment.
     // depth / path: position in the dissection tree (path = bits of the left/right choices so far)
@@ -180,18 +134,6 @@ struct Orderer {
                 if (cost < bestCost) { bestCost = cost; best = l; }
             }
             std::vector<int> A, B, S;
-            if (geometric_split(comp, ctag, A, B, S)) {
-                const int ta = nextTag++, tb = nextTag++;
-                for (int v : A) mark[v] = ta;
-                for (int v : B) mark[v] = tb;
-                for (int v : S) mark[v] = -1;
-                run(A, ta, true, depth + 1, 2 * path);
-                run(B, tb, true, depth + 1, 2 * path + 1);
-                segs.push_back(S);
-                segOwner.push_back(depth >= cutDepth ? ownerHere : -1);
-                continue;
-            }
-            A.clear(); B.clear(); S.clear();
             for (int v : order) {
                 if (level[v] < best) A.push_back(v);
                 else if (level[v] > best) B.push_back(v);
@@ -219,21 +161,19 @@ struct Orderer {
 
 }  // namespace
 
+#ifndef TC_CHUNK
+#define TC_CHUNK 10                    // terms per partial-sum link of a long task (see emit_chain)
+#endif
 int tile_symbolic(int nImg, const int64_t* adjPtr, const int32_t* adj, const int* nEO, int nIO, int mode,
-                  int leafImages, TileSym& out, int nParts, int myPart, const double* xyz) {
+                  int leafImages, TileSym& out, int nParts, int myPart) {
     const int T = TC_T;
     out = TileSym();
     int nCamCols = 0;
     for (int i = 0; i < nImg; ++i) nCamCols += nEO[i];
     if (mode < 0) mode = (nCamCols >= 24 * T) ? 2 : 0;      // small systems: one dense front
-    if (const char* e = getenv("DBAT_ORDER")) {
-        if (!strcmp(e, "natural")) mode = 0; else if (!strcmp(e, "rcm")) mode = 1; else if (!strcmp(e, "nd")) mode = 2;
-    }
-    if (const char* e = getenv("DBAT_ND_LEAF")) leafImages = std::max(8, atoi(e));
     // the tree can only be cut where it was dissected; parts = largest power of two <= nParts
     int cutDepth = 0;
     if (mode == 2) while ((2 << cutDepth) <= nParts) ++cutDepth;
-    if (getenv("DBAT_REPLICATED_CHOL")) cutDepth = 0;
     out.nParts = 1 << cutDepth;
     out.myPart = myPart < out.nParts ? myPart : -2;           // a rank beyond the parts owns nothing
     out.order_mode = mode;
@@ -248,9 +188,6 @@ int tile_symbolic(int nImg, const int64_t* adjPtr, const int32_t* adj, const int
     } else {
         Orderer o(g, leafImages);
         o.cutDepth = cutDepth;
-        // measured (config 4 and an 8000-station block): the level-set separators below give 25-50 % fewer tile
-        // products than coordinate bisection, so the geometric cut is opt-in
-        o.xyz = getenv("DBAT_ND_GEO") ? xyz : nullptr;
         std::vector<int> all(nImg);
         std::iota(all.begin(), all.end(), 0);
         for (int v : all) o.mark[v] = 0;
@@ -430,7 +367,7 @@ int tile_symbolic(int nImg, const int64_t* adjPtr, const int32_t* adj, const int
     // released through an auxiliary flag, then the task proper with the last terms.  Every link sorts into the list
     // right after the last column it reads, so the early links run long before the tile's turn and the link on the
     // critical path is short.
-    const int TC_CHUNK = getenv("DBAT_TC_CHUNK") ? std::max(2, atoi(getenv("DBAT_TC_CHUNK"))) : 10;
+    static_assert(TC_CHUNK >= 2, "a partial-sum chain link needs at least two terms");
     int nAux = 0;
     auto emit_chain = [&](const Tmp& t, bool alwaysFromTile, std::vector<Tmp>& list) {
         const int slot = out.tix[(size_t)t.I * nT + t.J];
@@ -522,12 +459,6 @@ int tile_symbolic(int nImg, const int64_t* adjPtr, const int32_t* adj, const int
 // NULL, imgS (nImg), tix (nT*nT, needs a second call once nT is known), taskIJ (2*nTasks), termPtr (nTasks+1),
 // termAB (2*nTerms), level (nT).
 static TileSym g_last_sym;
-static std::vector<double> g_xyz;
-// station coordinates (3 x nImg, column-major) for the next dbat_tile_symbolic call; nImg = 0 clears them
-extern "C" int dbat_tile_symbolic_coords(int64_t nImg, const double* xyz) {
-    g_xyz.assign(xyz ? xyz : nullptr, xyz ? xyz + 3 * nImg : nullptr);
-    return DBAT_OK;
-}
 extern "C" int dbat_tile_symbolic(int64_t nImg, int64_t nOP, int64_t nObs, const int64_t* obs_img,
                                   const int64_t* obs_op, const int64_t* nEO, int64_t nIO, int64_t mode,
                                   int64_t leafImages, int64_t* counts) {
@@ -548,8 +479,7 @@ extern "C" int dbat_tile_symbolic(int64_t nImg, int64_t nOP, int64_t nObs, const
     std::vector<int> ne((size_t)nImg);
     for (int64_t i = 0; i < nImg; ++i) ne[(size_t)i] = (int)nEO[i];
     const int nParts = counts[14] > 0 ? (int)counts[14] : 1, myPart = (int)counts[15];
-    int rc = tile_symbolic((int)nImg, ap.data(), ad.data(), ne.data(), (int)nIO, (int)mode, (int)leafImages, g_last_sym, nParts, myPart,
-                           (int64_t)g_xyz.size() == 3 * nImg ? g_xyz.data() : nullptr);
+    int rc = tile_symbolic((int)nImg, ap.data(), ad.data(), ne.data(), (int)nIO, (int)mode, (int)leafImages, g_last_sym, nParts, myPart);
     if (rc) return rc;
     const TileSym& s = g_last_sym;
     counts[0] = s.nT; counts[1] = s.ld; counts[2] = s.nS; counts[3] = s.nSlots; counts[4] = s.nSlotsS;

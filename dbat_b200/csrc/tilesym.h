@@ -54,11 +54,10 @@ struct TileSym {
 // adjacency of the co-visibility graph in CSR form (no self loops needed); nEO[i] = number of estimated
 // EO elements of image i (0..6); nIO = number of estimated shared IO columns.
 // mode: 0 natural, 1 rcm, 2 nested dissection, -1 automatic.
-// xyz: optional 3 x nImg station coordinates (column-major) - the dissection then cuts geometrically.
 // nParts / myPart: distributed factorisation - the elimination tree is cut into nParts (a power of two) subtrees,
 // part g factors the columns of subtree g, everybody the separators above the cut (nParts = 1: everything local).
 int tile_symbolic(int nImg, const int64_t* adjPtr, const int32_t* adj, const int* nEO, int nIO, int mode,
-                  int leafImages, TileSym& out, int nParts = 1, int myPart = 0, const double* xyz = nullptr);
+                  int leafImages, TileSym& out, int nParts = 1, int myPart = 0);
 
 // co-visibility graph from (0-based) point-major image lists
 void covis_graph(int nImg, int nOP, const int* pt_start, const int* img_pm, std::vector<int64_t>& adjPtr,

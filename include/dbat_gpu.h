@@ -174,16 +174,6 @@ typedef struct dbat_cov_hit_list {
 int dbat_cov_stats(dbat_handle *h, double s0, double thres, double *std_x, dbat_cov_hit_list *io,
                    dbat_cov_hit_list *eo, dbat_cov_hit_list *op);
 
-/* Elimination order of the images for a banded factorisation of the reduced camera system (host only, no
- * device needed): reverse Cuthill-McKee on the co-visibility graph - images i, j are adjacent when they
- * observe a common object point, which is exactly when S has a non-zero 6x6 block (i, j).  obs_img / obs_op
- * are 1-based as in dbat_problem_desc; perm (nImg, 1-based) lists the images in elimination order and
- * *bandwidth (may be NULL) is the largest distance, in images, between two adjacent images under it.  The
- * reference has no counterpart on its solver path (it factors the camera block densely, bundle_cov.m:97);
- * its ordering experiments are private/blkcolperm.m and test/postcov/reorder_test.m. */
-int dbat_camera_order(int64_t nImg, int64_t nOP, int64_t nObs, const int64_t *obs_img,
-                      const int64_t *obs_op, int64_t *perm, int64_t *bandwidth);
-
 /* Structure of the reduced camera system of a problem: info (16) = {nT (64 x 64 tile rows), ld, nS (camera-side
  * unknowns), nSlots (stored tiles incl. fill), nSlotsS (tiles of S itself), nTasks, nTerms (tile products per
  * factorisation), depth (longest dependency chain in tile columns), order mode, segments, grid of the factorisation,
@@ -210,9 +200,6 @@ int dbat_tile_symbolic_get(int64_t *imgS, int64_t *tix, int64_t *taskIJ, int64_t
  * {nTasks1 (tasks of phase 1), nTopS, nTop (slots of the top tile columns), parts actually used, nOwnS}.
  * dbat_tile_symbolic_get2: taskMode (nTasks; 1 = partial sum), colOwner (nT; -1 = top), ownSBegin (parts + 1). */
 int dbat_tile_symbolic_get2(int64_t *taskMode, int64_t *colOwner, int64_t *ownSBegin);
-/* Station coordinates (3 x nImg) for the next dbat_tile_symbolic call: the dissection then bisects geometrically
- * (dbat_create takes them from EOval); nImg = 0 / NULL clears them. */
-int dbat_tile_symbolic_coords(int64_t nImg, const double *xyz);
 
 /* The sparse tile solver on its own (unit tests / profiling): x = A^-1 b for a symmetric positive definite
  * column-major n x n matrix whose 6-column blocks play the role of images (coupled where A has a non-zero),

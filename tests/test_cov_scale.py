@@ -152,7 +152,7 @@ def elimination_order(s):
     """Images in the order the device's reduced system holds them (the host symbolic analysis dbat_create runs)."""
     nImg, nOP = s.EO.val.shape[1], s.OP.val.shape[1]
     nEO = s.bundle.est.EO[:6].sum(axis=0).astype(np.int64)
-    sym = dlib.tile_symbolic(s.IP.img, s.IP.op, nImg, nOP, nEO, len(s.bundle.serial.IO.dest), xyz=s.EO.val[0:3])
+    sym = dlib.tile_symbolic(s.IP.img, s.IP.op, nImg, nOP, nEO, len(s.bundle.serial.IO.dest))
     has = nEO > 0
     return np.flatnonzero(has)[np.argsort(sym['imgS'][has], kind='stable')], sym
 

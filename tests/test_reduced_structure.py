@@ -1,8 +1,9 @@
-"""Structure of the reduced camera system (groundwork for SURVEY §8(f) N4; tools/reduced_sparsity.py).
+"""Structure of the reduced camera system S that the symbolic analysis (csrc/tilesym.cu) relies on, checked with
+the host tools of tools/reduced_sparsity.py.
 
-Executable form of the design note in DESIGN.md §9: the block pattern of S is the co-visibility graph of the
-images; with the images in reverse Cuthill-McKee order and the shared IO block last, the Cholesky factor stays
-inside the band of that pattern; in x order (IO first, what the device path uses today) it fills completely."""
+The block pattern of S is the co-visibility graph of the images, the graph the symbolic analysis orders.  With the
+images in a bandwidth-reducing order and the shared IO block last, the Cholesky factor stays inside the band of that
+pattern; with the IO block first it fills completely, which is why the symbolic analysis places it last."""
 import os
 import sys
 
@@ -65,61 +66,3 @@ def test_band_of_the_reduced_system_survives_only_with_the_io_block_last():
     # (3) x order (IO first, today's layout of S): the arrowhead fills the whole factor
     L0 = np.linalg.cholesky(S)
     assert np.count_nonzero(np.abs(L0) > 1e-13) > 0.98 * nC * (nC + 1) / 2
-
-
-def test_banded_tile_cholesky_prototype_equals_the_dense_factor():
-    """tools/band_cholesky_proto.py: the tile loop restricted to band + border tiles gives the dense factor
-    on a band-plus-border SPD matrix, with the predicted number of tile operations."""
-    from band_cholesky_proto import band_tile_cholesky, dense_counts
-    rng = np.random.default_rng(1)
-    NB, nb, bt, nborder = 8, 12, 3, 2
-    n = NB * nb
-    ne = nb - nborder
-    M = rng.standard_normal((n, n))
-    keep = np.zeros((nb, nb), bool)
-    for i in range(nb):
-        for j in range(nb):
-            keep[i, j] = abs(i - j) <= bt or i >= ne or j >= ne
-    M = M * np.kron(keep, np.ones((NB, NB)))
-    A = M @ M.T                                            # band 2*bt in tiles ... so use it as the pattern source
-    A = A * np.kron(keep, np.ones((NB, NB))) + n * np.eye(n)   # SPD, band bt + dense border
-    L, cnt = band_tile_cholesky(A, NB, bt, nborder)
-    np.testing.assert_allclose(L, np.linalg.cholesky(A), rtol=1e-10, atol=1e-12)
-    assert cnt['gemm_tiles'] < dense_counts(nb)['gemm_tiles'] and cnt['potrf'] == nb
-    # one tile less of band is not enough: the factor is then wrong
-    Lbad, _ = band_tile_cholesky(A, NB, bt - 1, nborder)
-    assert np.abs(Lbad - np.linalg.cholesky(A)).max() > 1e-6
-
-
-def test_library_camera_order_is_a_valid_rcm_order():
-    """`dbat_camera_order` (host code in libdbatgpu.so, no device needed): a permutation whose bandwidth on
-    the co-visibility graph is reported correctly, is far below the natural one for a shuffled block and
-    comparable to SciPy's reverse Cuthill-McKee; isolated images and empty input are handled."""
-    from dbat_b200 import _lib
-    from dbat_b200.synth import make_scene
-    from reduced_sparsity import covisibility
-    s, _ = make_scene(196, 6000, rays=8, seed=5, build_indices=False)
-    nImg, nOP = s.EO.val.shape[1], s.OP.val.shape[1]
-    rng = np.random.default_rng(0)
-    shuffle = rng.permutation(nImg)                               # destroy the generator's strip order
-    img, op = shuffle[np.asarray(s.IP.img)], np.asarray(s.IP.op)
-    perm, bw = _lib.camera_order(img, op, nImg, nOP)
-    assert sorted(perm) == list(range(nImg))
-    G = covisibility(img, op, nImg).tocoo()
-    pos = np.empty(nImg, int)
-    pos[perm] = np.arange(nImg)
-    assert bw == np.abs(pos[G.row] - pos[G.col]).max()
-    natural = np.abs(G.row - G.col).max()
-    ref = np.asarray(reverse_cuthill_mckee(G.tocsr(), symmetric_mode=True))
-    rpos = np.empty(nImg, int)
-    rpos[ref] = np.arange(nImg)
-    scipy_bw = np.abs(rpos[G.row] - rpos[G.col]).max()
-    assert bw < 0.5 * natural and bw <= 1.3 * scipy_bw
-    # two images that see nothing in common with the rest, and no observations at all
-    perm2, bw2 = _lib.camera_order(np.array([0, 1, 0, 1]), np.array([0, 0, 1, 1]), 4, 2)
-    assert sorted(perm2) == [0, 1, 2, 3] and bw2 == 1
-    perm3, bw3 = _lib.camera_order(np.zeros(0, int), np.zeros(0, int), 3, 0)
-    assert sorted(perm3) == [0, 1, 2] and bw3 == 0
-    import pytest
-    with pytest.raises(_lib.DbatError):
-        _lib.camera_order(np.array([5]), np.array([0]), 3, 1)
