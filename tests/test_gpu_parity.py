@@ -495,69 +495,6 @@ def test_full_size_step_against_the_oracle():
     P.close()
 
 
-def _banded_arrow_spd(n, bw, border, rng, blocks=None):
-    """SPD test matrix with the structure of a reduced camera system: a band (or the given list of coupled
-    6-column block pairs), `border` dense rows at the end, diagonally dominant."""
-    A = np.zeros((n, n))
-    if blocks is None:
-        for c in range(n):
-            lo = max(0, c - bw)
-            A[c, lo:c] = rng.standard_normal(c - lo)
-    else:
-        for a, b in blocks:
-            ra, rb = slice(6 * a, min(n, 6 * a + 6)), slice(6 * b, min(n, 6 * b + 6))
-            A[ra, rb] = rng.standard_normal((ra.stop - ra.start, rb.stop - rb.start))
-        A = np.tril(A, -1)
-    if border:
-        A[n - border:, :] = rng.standard_normal((border, n))
-    A = np.tril(A, -1)
-    A = A + A.T
-    A += np.diag(np.abs(A).sum(axis=1) + 1.0 + rng.uniform(0, 1, n))
-    return A
-
-
-@pytest.mark.parametrize('n,bw,border,mode', [(50, 50, 0, 0), (423, 423, 0, -1), (700, 90, 9, 0), (2500, 200, 9, 1),
-                                              (2500, 200, 9, 2), (6002, 600, 9, 2)])
-def test_tile_cholesky_solver(n, bw, border, mode):
-    """The sparse tile Cholesky on its own (ordering + symbolic analysis + persistent data-flow kernel +
-    backward substitution) against LAPACK on matrices shaped like reduced camera systems."""
-    from dbat_b200 import _lib
-    rng = np.random.default_rng(n + mode)
-    A = _banded_arrow_spd(n, bw, border, rng)
-    b = rng.standard_normal(n)
-    x, st = _lib.tile_chol_solve(A, b, mode=mode, leaf=40)
-    assert st['rc'] == 0
-    ref = np.linalg.solve(A, b)
-    np.testing.assert_allclose(x, ref, rtol=1e-10, atol=1e-13 * np.abs(ref).max())
-    piv = np.diag(np.linalg.cholesky(A))
-    assert st['min_pivot'] <= piv.max() and st['max_pivot'] >= piv.min()      # bounds of the true pivots (ordering differs)
-    x2, st2 = _lib.tile_chol_solve(A, b, mode=mode, leaf=40, repeat=3)         # epochs: the flags are reused
-    np.testing.assert_array_equal(x2, x)
-    _, st3 = _lib.tile_chol_solve(A - 2 * np.diag(np.diag(A)), b, mode=mode)
-    assert st3['rc'] == _lib.E_NOTSPD
-
-
-def test_tile_cholesky_dissected_grid():
-    """Co-visibility of a 2-D block of images (every image coupled to its neighbours within two grid steps):
-    nested dissection gives independent subtrees; the factorisation must not care about the order."""
-    from dbat_b200 import _lib
-    g = 24
-    idx = np.arange(g * g).reshape(g, g)
-    blocks = [(int(idx[i, j]), int(idx[k, l])) for i in range(g) for j in range(g)
-              for k in range(max(0, i - 2), min(g, i + 3)) for l in range(max(0, j - 2), min(g, j + 3)) if idx[k, l] < idx[i, j]]
-    n = 6 * g * g
-    rng = np.random.default_rng(4)
-    A = _banded_arrow_spd(n, 0, 0, rng, blocks=blocks)
-    b = rng.standard_normal(n)
-    ref = np.linalg.solve(A, b)
-    depth = {}
-    for mode in (0, 1, 2):
-        x, st = _lib.tile_chol_solve(A, b, mode=mode, leaf=40)
-        np.testing.assert_allclose(x, ref, rtol=1e-10, atol=1e-13 * np.abs(ref).max())
-        depth[mode] = st['depth']
-    assert depth[2] < depth[1]
-
-
 @pytest.mark.parametrize('model,sigma0', [(-1, 1.62168), (1, 1.68901), (2, 1.68901), (3, 1.6148),
                                           (4, 1.61247), (5, 1.6148)])
 def test_camcal_all_models_golden_sigma0(model, sigma0):

@@ -7,7 +7,7 @@ os.environ['DBAT_TCHOL_PROF'] = os.path.join(ROOT, 'gpurun_out', 'tcprof.csv')
 import __graft_entry__ as g
 g.build()
 from dbat_b200 import _lib
-from test_gpu_parity import _banded_arrow_spd
+from test_tile_cholesky import _banded_arrow_spd
 n, bw, border, mode = 2500, 200, 9, 1
 rng = np.random.default_rng(n)
 A = _banded_arrow_spd(n, bw, border, rng)

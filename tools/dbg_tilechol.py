@@ -6,7 +6,7 @@ import numpy as np
 import __graft_entry__ as g
 g.build()
 from dbat_b200 import _lib
-from test_gpu_parity import _banded_arrow_spd
+from test_tile_cholesky import _banded_arrow_spd
 def alarm(*a): 
     print('TIMEOUT', flush=True); os._exit(3)
 signal.signal(signal.SIGALRM, alarm)
