@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'libdbatgpu.so')
-SOURCES = ['eval.cu', 'schur.cu', 'schur_win.cu', 'chol.cu', 'tilechol.cu', 'tilesym.cu', 'plan.cu', 'general_io.cu', 'covstats.cu', 'api.cu',
+SOURCES = ['eval.cu', 'schur.cu', 'schur_win.cu', 'schur_wide.cu', 'chol.cu', 'tilechol.cu', 'tilesym.cu', 'plan.cu', 'general_io.cu', 'covstats.cu', 'api.cu',
            'startval.cu']
 EXTRA = os.environ.get('DBAT_NVCC_EXTRA', '').split()
 NVCC_FLAGS = EXTRA + ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',

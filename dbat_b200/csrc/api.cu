@@ -227,7 +227,7 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail_create(nullptr, DBAT_E_CUDA, "no CUDA device available (libdbatgpu has no CPU fallback)");
     dbat_handle* h = new dbat_handle();
-    // points with more than grpMaxM rays go to k_schur_atomic; DBAT_GRP_MAXM=k lowers it (tests of the per-point path)
+    // points with more than grpMaxM rays go to the wide-point Schur path; DBAT_GRP_MAXM=k lowers it (tests of that path)
     int grpMaxM = DBAT_GRP_MAXM;
     if (const char* e = getenv("DBAT_GRP_MAXM")) grpMaxM = std::max(1, std::min(DBAT_GRP_MAXM, atoi(e)));
 
@@ -254,6 +254,7 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     P.evalCompact = plan_eval_compact(pl, d->nK, d->nP) ? 1 : 0;
     P.nPsb = up.nPsb; P.nPsbig = up.nPsbig;
     P.nCand = up.nCand; P.nBig = up.nBig; P.grpMaxRays = up.grpMaxRays; P.nClu = up.nClu; P.nRedBlk = up.nRedBlk;
+    P.nWObs = up.nWObs; P.nWPair = up.nWPair;
     if (cudaStreamCreate(&h->st) != cudaSuccess || cudaStreamCreateWithFlags(&h->st2, cudaStreamNonBlocking) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->evFork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&h->evJoin, cudaEventDisableTiming) != cudaSuccess ||
@@ -303,6 +304,11 @@ extern "C" int dbat_create(const dbat_problem_desc* d, dbat_handle** out) {
     UP(P.pt_pm, up.pt_pm);
     UP(P.psb_pt, up.psb_pt); UP(P.psbig, up.psbig);
     UP(P.grp_pt, up.grp_pt); UP(P.big_pt, up.big_pt);
+    UP(P.wide_o, up.wide_o); UP(P.wimg_ptr, up.wimg_ptr); UP(P.wimg_w, up.wimg_w); UP(P.wimg_pt, up.wimg_pt);
+    UP(P.wpair, up.wpair);
+    AL(P.wide_Z, (size_t)up.nWObs * 18); AL(P.wide_Zsh, (size_t)up.nBig * 48);
+    AL(P.wide_ssPart, (size_t)(up.nBig + DBAT_WIDE_SSPART - 1) / DBAT_WIDE_SSPART * 256);
+    AL(P.wide_shAcc, DBAT_NSLOT * (DBAT_NSLOT + 1));
     AL(P.vinv, (size_t)std::max(1, nOP) * 8);
     UP(P.clu_order, up.clu_order);
     UP(P.win_hdr, up.win_hdr); UP(P.clu_grp, up.clu_grp); UP(P.clu_img_off, up.clu_img_off); UP(P.clu_img, up.clu_img);

@@ -94,8 +94,20 @@ struct DevProblem {
     // points whose image lists have a union of at most 12 images (schur_win.cu)
     const int* grp_pt;     // point ids, grouped
     int grpMaxRays;        // largest union among the groups (sizes the window kernel's operand)
-    const int* big_pt;     // points with more than DBAT_GRP_MAXM rays (k_schur_atomic)
+    const int* big_pt;     // the wide points: estimated points with more than DBAT_GRP_MAXM rays, ascending id
     int nBig;
+    // wide-point Schur (schur_wide.cu): their observations numbered point by point ("wide observations"), the per-image
+    // lists of them, the camera-pair blocks they touch and the staged factors Z_o = M_j W_o', [Wsh_j g_j]' M_j'
+    const int* wide_o;     // nWObs: point-major observation of every wide observation
+    const int* wimg_ptr;   // nImg+1: wide observations of every image ...
+    const int* wimg_w;     // ... their numbers, ascending point
+    const int* wimg_pt;    // ... their wide points (index into big_pt)
+    const int* wpair;      // nWPair x (image A, image B), rank A >= rank B
+    int nWObs, nWPair;
+    double* wide_Z;        // nWObs x 18: Z_o[k][a], k = point coordinate, a = EO element
+    double* wide_Zsh;      // nBig x 48: [k][s], s = shared IO slot 0..13, 14 = gradient, 15 = zero
+    double* wide_ssPart;   // per DBAT_WIDE_SSPART wide points: their 16 x 16 shared x shared table
+    double* wide_shAcc;    // NSLOT x (NSLOT+1): the sum of the partial tables (k_schur_ss_apply's shAcc)
     double* vinv;          // nOP x 8: (V_j + lambda I)^-1 (6 entries) for dbat_cov (launch_point_vinv)
     // window Schur (schur_win.cu): clusters of consecutive groups accumulate their camera x camera blocks in
     // shared memory; every cluster leaves ONE image of its window in a staging buffer and a second kernel sums the
@@ -117,4 +129,5 @@ struct DevProblem {
     const long long* redi_off;   // staging offset of entry (shared row 0, EO element 0) of the contribution
     double* win_ssPart;    // per 256 clusters: partial sums of the 16 x 16 shared x shared tables
 };
-#define DBAT_GRP_MAXM 20   // grouped path up to 20 rays per point (= WIN_MAXW); more rays: k_schur_atomic
+#define DBAT_GRP_MAXM 20   // grouped path up to 20 rays per point (= WIN_MAXW); more rays: schur_wide.cu
+#define DBAT_WIDE_SSPART 16   // wide points per partial shared x shared table

@@ -44,6 +44,8 @@ void launch_mul(const double* a, const double* b, double* out, int n, cudaStream
 
 // schur_win.cu (Schur reduction: window accumulation per point cluster + fixed-order sums, no atomics)
 void launch_schur_win(const DevProblem& P, double lambda, const double* shAcc, cudaStream_t st);
+// schur_wide.cu (Schur reduction of the points with more than DBAT_GRP_MAXM rays: per-image lists + fixed-order sums)
+void launch_schur_wide(const DevProblem& P, double lambda, cudaStream_t st);
 
 // general_io.cu (general IO block structure)
 void launch_point_side_gen(const DevProblem& P, cudaStream_t st);

@@ -343,7 +343,36 @@ void plan_schur_windows(ProblemPlan& p, PlanUpload& u, const TileSym& sym, int g
     if (!cand.empty()) close_group(cand.size());
     const bool noCand = cand.empty();
     if (noCand) { cand.push_back(0); gstart.assign(1, 0); gimg_off.assign(1, 0); gimg.push_back(0); }
-    if (big.empty()) big.push_back(0); else u.nBig = (int)big.size();
+    // ---- wide points (schur_wide.cu): their observations numbered point by point (big ascends in point id), per
+    //      image the list of its wide observations in that order, and the camera-pair blocks they touch.  Linear in
+    //      the wide observations plus one entry per pair block: no per-point pair lists.
+    u.nBig = (int)big.size();
+    u.wimg_ptr.assign(nImg + 1, 0);
+    for (int j : big)
+        for (int o = ps[j]; o < ps[j + 1]; ++o) { u.wide_o.push_back(o); u.wimg_ptr[img_pm[o] + 1]++; }
+    u.nWObs = (int)u.wide_o.size();
+    for (int i = 0; i < nImg; ++i) u.wimg_ptr[i + 1] += u.wimg_ptr[i];
+    u.wimg_w.resize(u.nWObs); u.wimg_pt.resize(u.nWObs);
+    {
+        std::vector<int> fill(u.wimg_ptr.begin(), u.wimg_ptr.end() - 1);
+        int w = 0;
+        for (int jb = 0; jb < u.nBig; ++jb)
+            for (int o = ps[big[jb]]; o < ps[big[jb] + 1]; ++o, ++w) {
+                const int q = fill[img_pm[o]]++;
+                u.wimg_w[q] = w; u.wimg_pt[q] = jb;
+            }
+        std::vector<int> mark(nImg, -1);
+        for (int a = 0; a < nImg; ++a)
+            for (int q = u.wimg_ptr[a]; q < u.wimg_ptr[a + 1]; ++q) {
+                const int j = big[u.wimg_pt[q]];
+                for (int o = ps[j]; o < ps[j + 1]; ++o) {
+                    const int b = img_pm[o];
+                    if (imgRank[b] <= imgRank[a] && mark[b] != a) { mark[b] = a; u.wpair.push_back(a); u.wpair.push_back(b); }
+                }
+            }
+        u.nWPair = (int)u.wpair.size() / 2;
+    }
+    if (big.empty()) big.push_back(0);
     const int nGrp = (int)gstart.size() - 1;
     // ---- window Schur (schur_win.cu): group headers, clusters of consecutive groups whose unions span at most
     //      WIN_MAXW images, and the fixed-order reduction index of the cluster images

@@ -69,6 +69,12 @@ struct PlanUpload {
     std::vector<int> red_ptr, red_imgA, red_imgB, redi_ptr;
     std::vector<long long> red_off, redi_off;
     int nClu = 0, nRedBlk = 0;
+    // wide-point index (schur_wide.cu): the observations of the points in big_pt, numbered point by point
+    std::vector<int> wide_o;          // point-major observation of every wide observation
+    std::vector<int> wimg_ptr;        // nImg + 1: the wide observations of every image ...
+    std::vector<int> wimg_w, wimg_pt; // ... (wide observation, wide point), ascending point
+    std::vector<int> wpair;           // (image A, image B) of every camera-pair block wide points touch, rank A >= rank B
+    int nWObs = 0, nWPair = 0;
 };
 
 // S index maps of the camera-side columns for one tiling of the reduced system
@@ -90,7 +96,7 @@ int plan_cameras(const dbat_problem_desc* d, ProblemPlan& p, const PlanUpload& u
 // runs of whole points for the point-side assembly and the list of long points
 void plan_point_blocks(const ProblemPlan& p, PlanUpload& u);
 // window Schur index for the elimination order of sym: groups, clusters, headers, reduction CSR, cluster order;
-// estimated points with more than grpMaxM rays go to k_schur_atomic instead
+// estimated points with more than grpMaxM rays (the wide points) get the index of schur_wide.cu instead
 void plan_schur_windows(ProblemPlan& p, PlanUpload& u, const TileSym& sym, int grpMaxM);
 // sets p.x2s and returns the other S index maps
 ReducedMaps plan_reduced_maps(ProblemPlan& p, const TileSym& sym);

@@ -145,95 +145,6 @@ void launch_build_S(const DevProblem& P, const double* camDiag, const double* ca
     count_launch();
 }
 
-// Schur update of the points with more than DBAT_GRP_MAXM rays, which the window kernels (schur_win.cu) do not take:
-// one warp per point, lane = (pair, EO row), 6x6 pair blocks scattered with FP64 red.global.add (6 consecutive rows
-// per lane group -> coalesced sectors).  The shared x shared table and its rhs column go to shAcc.  The sum ORDER into
-// an entry of S is not fixed, so a project with such points is not bit-reproducible from run to run.
-__global__ void __launch_bounds__(256) k_schur_atomic(DevProblem P, double lambda, double* __restrict__ shAcc,
-                                                      const int* __restrict__ list, int nList) {
-    const int lane = threadIdx.x & 31;
-    const int warpGlobal = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int nWarps = (gridDim.x * blockDim.x) >> 5;
-    // shared x shared accumulators: entries e = lane + 32*k of the NSLOT x (NSLOT+1) table
-    constexpr int NE = DBAT_NSLOT * (DBAT_NSLOT + 1);
-    constexpr int NEL = (NE + 31) / 32;
-    double accSh[NEL];
-#pragma unroll
-    for (int k = 0; k < NEL; ++k) accSh[k] = 0.0;
-
-    for (int jj = warpGlobal; jj < nList; jj += nWarps) {
-        const int j = list[jj];
-        const double* rec = P.pt + (size_t)j * DBAT_PT_STRIDE;
-        const int* opc = P.op_col + 3 * (size_t)j;
-        if (opc[0] < 0 && opc[1] < 0 && opc[2] < 0) continue;
-        double Vi[6];
-        point_inverse(rec, opc, lambda, Vi);
-        const double gj[3] = {rec[6], rec[7], rec[8]};
-        double Vg[3];
-        symv3(Vi, gj, Vg);
-        const int o0 = P.pt_start[j], k = P.pt_start[j + 1] - o0;
-        // local x local pair blocks: item = (pair, a)
-        const int nItems = k * (k + 1) / 2 * 6;
-        for (int it = lane; it < nItems; it += 32) {
-            const int pr = it / 6, a = it - pr * 6;
-            int o = (int)((sqrt(8.0 * pr + 1.0) - 1.0) * 0.5);
-            while ((o + 1) * (o + 2) / 2 <= pr) ++o;
-            while (o * (o + 1) / 2 > pr) --o;
-            const int o2 = pr - o * (o + 1) / 2;            // o2 <= o  => image(o2) <= image(o)
-            const int row = P.eo_s[6 * (size_t)P.img_pm[o0 + o] + a];
-            if (row < 0) continue;
-            const double* Wa = P.W + (size_t)(o0 + o) * DBAT_W_STRIDE + 3 * a;
-            const double wa[3] = {Wa[0], Wa[1], Wa[2]};
-            double ya[3];
-            symv3(Vi, wa, ya);
-            const int* ec2 = P.eo_s + 6 * (size_t)P.img_pm[o0 + o2];
-            const double* Wb = P.W + (size_t)(o0 + o2) * DBAT_W_STRIDE;
-#pragma unroll
-            for (int b = 0; b < 6; ++b) {
-                const int col = ec2[b];
-                if (col < 0 || (o2 == o && col > row)) continue;     // same image: lower triangle only
-                const double v = ya[0] * Wb[3 * b] + ya[1] * Wb[3 * b + 1] + ya[2] * Wb[3 * b + 2];
-                atomicAdd(tc_at(P.T, max(row, col), min(row, col)), -v);
-            }
-            if (o2 == 0) {                                   // once per (o, a): rhs and shared x local
-                atomicAdd(&P.rhs[row], ya[0] * gj[0] + ya[1] * gj[1] + ya[2] * gj[2]);
-#pragma unroll
-                for (int s = 0; s < DBAT_NSLOT; ++s) {
-                    const int srow = P.sh_s[s];
-                    if (srow < 0) continue;
-                    const double* ws = rec + DBAT_PT_WSH + 3 * s;
-                    atomicAdd(tc_at(P.T, srow, row), -(ya[0] * ws[0] + ya[1] * ws[1] + ya[2] * ws[2]));
-                }
-            }
-        }
-        // shared x shared (+ rhs): accumulate in registers, flushed once per warp
-#pragma unroll
-        for (int kk = 0; kk < NEL; ++kk) {
-            const int e = lane + 32 * kk;
-            if (e < NE) {
-                const int a = e / (DBAT_NSLOT + 1), b = e - a * (DBAT_NSLOT + 1);
-                const double* wa = rec + DBAT_PT_WSH + 3 * a;
-                if (b < DBAT_NSLOT) {
-                    if (b <= a) {
-                        const double* wb = rec + DBAT_PT_WSH + 3 * b;
-                        const double w3[3] = {wb[0], wb[1], wb[2]};
-                        double y[3];
-                        symv3(Vi, w3, y);
-                        accSh[kk] += wa[0] * y[0] + wa[1] * y[1] + wa[2] * y[2];
-                    }
-                } else {
-                    accSh[kk] += wa[0] * Vg[0] + wa[1] * Vg[1] + wa[2] * Vg[2];
-                }
-            }
-        }
-    }
-#pragma unroll
-    for (int kk = 0; kk < NEL; ++kk) {
-        const int e = lane + 32 * kk;
-        if (e < NE) atomicAdd(&shAcc[e], accSh[kk]);
-    }
-}
-
 // (V_j + lambda I)^-1 of every point into P.vinv (the point blocks of the covariance, dbat_cov)
 __global__ void k_point_vinv(DevProblem P, double lambda) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
@@ -247,19 +158,16 @@ __global__ void k_point_vinv(DevProblem P, double lambda) {
 void launch_point_vinv(const DevProblem& P, double lambda, cudaStream_t st) {
     if (P.nOP > 0) { k_point_vinv<<<(P.nOP + 255) / 256, 256, 0, st>>>(P, lambda); count_launch(); }
 }
-static thread_local double* g_shAcc = nullptr;       // per device (one host thread drives one device)
 void launch_schur(const DevProblem& P, double lambda, cudaStream_t st) {
     if (P.nOP <= 0) return;
     if (P.ioGeneral) { launch_schur_gen(P, lambda, st); return; }
-    // window accumulation + fixed-order reduction (schur_win.cu); only points with more than DBAT_GRP_MAXM rays
-    // (none at BASELINE configs 4 / 5) go through the per-point kernel and its atomics
+    // the wide points (more than DBAT_GRP_MAXM rays; none at BASELINE configs 4 / 5) first (schur_wide.cu), then the
+    // window accumulation + fixed-order reduction of all others (schur_win.cu), which adds the wide points' shared x
+    // shared table; every step of both is in a fixed order
     const double* shAcc = nullptr;
     if (P.nBig > 0) {
-        if (!g_shAcc) cudaMalloc(&g_shAcc, sizeof(double) * DBAT_NSLOT * (DBAT_NSLOT + 1));
-        cudaMemsetAsync(g_shAcc, 0, sizeof(double) * DBAT_NSLOT * (DBAT_NSLOT + 1), st);
-        k_schur_atomic<<<std::min((P.nBig + 7) / 8, 148 * 8), 256, 0, st>>>(P, lambda, g_shAcc, P.big_pt, P.nBig);
-        count_launch();
-        shAcc = g_shAcc;
+        launch_schur_wide(P, lambda, st);
+        shAcc = P.wide_shAcc;
     }
     launch_schur_win(P, lambda, shAcc, st);
 }

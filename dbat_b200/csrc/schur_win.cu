@@ -20,7 +20,7 @@
 //                   tile of S.  Same for the shared-IO x EO rows (per image) and the shared x shared table.
 //
 // S is touched once per entry, and the result is bit-reproducible.  Points with more than DBAT_GRP_MAXM rays are not
-// grouped: k_schur_atomic (schur.cu) adds them with FP64 atomics before these kernels run.
+// grouped: schur_wide.cu adds them, also in a fixed order, before these kernels run.
 #include <algorithm>
 #include <cstdio>
 #include <vector>

@@ -139,6 +139,11 @@ int dbat_eval(dbat_handle *h, const double *x, double *r, int weighted);
 int dbat_jacobian_nnz(dbat_handle *h, int weighted, int64_t *nnz);
 int dbat_jacobian_csc(dbat_handle *h, int weighted, int64_t *Jc, int64_t *Ir, double *vals);
 
+/* Reproducibility of dbat_normal_step, dbat_solve, dbat_cov and dbat_cov_stats: with one IO block shared by all
+ * images every sum runs in an order fixed at dbat_create, whatever the number of rays of the points, so two calls on
+ * the same input on the same device return bit-identical results, from one handle or from two.  A general IO block
+ * structure (several cameras, image-variant IO parameters) assembles and reduces with FP64 atomics; its results may
+ * differ in the last bits from run to run. */
 void dbat_default_opts(int method, dbat_opts *opts);
 int  dbat_solve(dbat_handle *h, int method, const dbat_opts *opts, const double *x0,
                 dbat_result *res);
@@ -180,7 +185,7 @@ int dbat_cov_stats(dbat_handle *h, double s0, double thres, double *std_x, dbat_
  * grid of the backward solve, then which point-side paths the problem takes:
  *   [12] points with more than 128 observations (one-thread-per-point assembly and back-substitution, or one block
  *        per point in several passes with general IO),
- *   [13] estimated points with more than 20 observations (per-point Schur kernel with FP64 atomics),
+ *   [13] estimated points with more than 20 observations (Schur update from per-image lists, schur_wide.cu),
  *   [14] largest union of image lists of one window Schur group (above 12 the wider window instantiation runs),
  *   [15] most points in one window Schur group}. */
 int dbat_reduced_info(const dbat_handle *h, int64_t *info);
